@@ -2,7 +2,7 @@
 """Benchmark of the self-play search hot path (BASELINE.json metric:
 MCTS simulations/sec and self-play moves/sec, Hex 11x11).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--dump-outputs DIR]
 
 One *step* = one lockstep move of every resident game: evaluate_root +
 81 x (select, evaluate, expand/backup) + move commit = 810 root-to-leaf
@@ -65,7 +65,13 @@ def parse_args():
     ap.add_argument('--c5-games', type=int, default=512)
     ap.add_argument('--c5-sims', type=int, default=4000)
     ap.add_argument('--c4-rounds', type=int, default=64, help='tournament rounds per GPU')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help="write what the last timed end-to-end step returned (rank 0's chosen "
+                         'moves and the replay rows of the games it finished) as DIR/<name>.npy; '
+                         'git ignores bench_outputs/')
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error('--steps must be at least 1')
     SEARCH['simulations'] = args.sims
     return args
 
@@ -434,16 +440,19 @@ def run_ours(args):
                          (time.perf_counter() - c3) * 1e3), file=sys.stderr)
             rows_out += len(rows)
             down += chosen_host.numel() * 4 + rows.nbytes + 8
-        return rows_out, up, down, ev
+        return rows_out, up, down, ev, rows
 
     # one untimed pass of the same loop: the first pipelined iteration pays one-off set-up
     # (30 ms of stream time between its two moves, measured) that a long run never sees again
     e2e_loop(2)
     barrier()
     t0 = time.perf_counter()
-    rows_out, h2d, d2h, move_ev = e2e_loop(steps)
+    rows_out, h2d, d2h, move_ev, last_rows = e2e_loop(steps)
     barrier()
     e2e_s = time.perf_counter() - t0
+    if args.dump_outputs and rank == 0:
+        # chosen_host holds the last step's (move, move_id, result, ply): harvest_end waited for it
+        dump_outputs(args.dump_outputs, chosen_host.numpy(), last_rows, args.board)
     if world > 1:
         t = torch.tensor([e2e_s], device=dev)
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -557,13 +566,12 @@ def run_ours(args):
             sp2.preroll(args.preroll)
             for _ in range(2):
                 sp2.step_move()
-        k2 = max(steps, 8)
-        ms2, d2 = timed_steps(sp2, k2, barrier, world, dev)
-        tree_only = {'value': world * G * per_move * k2 / (ms2 * 1e-3), 'unit': UNIT,
-                     'evaluator': 'device stub (mode 2)', 'ms_per_step': ms2 / k2,
-                     'moves_per_sec': world * G * k2 / (ms2 * 1e-3),
+        ms2, d2 = timed_steps(sp2, steps, barrier, world, dev)
+        tree_only = {'value': world * G * per_move * steps / (ms2 * 1e-3), 'unit': UNIT,
+                     'evaluator': 'device stub (mode 2)', 'ms_per_step': ms2 / steps,
+                     'moves_per_sec': world * G * steps / (ms2 * 1e-3),
                      'mean_depth': d2['sum_depth'] / max(1, d2['simulations']),
-                     'games_finished_per_step': d2['games'] / k2}
+                     'games_finished_per_step': d2['games'] / steps}
         del sp2
         torch.cuda.empty_cache()
 
@@ -642,6 +650,36 @@ def run_ours(args):
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, chosen, rows, board):
+    """What one end-to-end step hands its caller, as float64 / float32 .npy
+    files: per game slot the chosen move, its ordinal among the legal moves,
+    the result after it and the new ply (chosen_*.npy); per replay row of the
+    games that finished in the step, the header fields (replay_<field>.npy),
+    the board before the move (replay_board.npy) and the root's visit counts
+    (replay_visits.npy).  Rows are sorted by (game id, ply); if they exceed
+    the size limit a fixed seeded sample of them is written."""
+    from azalea_b200.engine import decode_replay_rows
+    os.makedirs(out_dir, exist_ok=True)
+    out = {f'chosen_{f}': chosen[:, i].astype(np.float64)
+           for i, f in enumerate(('move', 'move_id', 'result', 'ply'))}
+    head, boards, visits = decode_replay_rows(rows, board)
+    fields = [f for f in head.dtype.names if f != 'reserved']
+    row_bytes = 8 * len(fields) + 4 * boards[0].size + 4 * visits.shape[1] if len(rows) else 1
+    cap = (DUMP_BYTES - sum(a.nbytes for a in out.values())) // row_bytes
+    keep = np.arange(len(rows))
+    if len(rows) > cap:
+        keep = np.sort(np.random.RandomState(0).choice(len(rows), cap, replace=False))
+    for f in fields:
+        out[f'replay_{f}'] = head[f][keep].astype(np.float64)
+    out['replay_board'] = boards[keep].astype(np.float32)
+    out['replay_visits'] = visits[keep].astype(np.float32)
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def guarded(fn):
@@ -758,7 +796,7 @@ def bench_config5(args, rank, world, dev, barrier, hbm_peak, bf16_peak):
     per_move = sp.sims_per_move
     for _ in range(3):
         sp.step_move()
-    steps = 2
+    steps = args.steps
     ms, d = timed_steps(sp, steps, barrier, world, dev)
     # per-launch shares from one eager move
     eng, stream = sp.eng, torch.cuda.current_stream()

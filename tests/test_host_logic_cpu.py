@@ -89,6 +89,40 @@ def test_decode_replay_rows_layout():
     assert (visits[1] == vis).all()
 
 
+def test_bench_dump_outputs_dtypes_and_size_cap(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: float32 / float64 files only; above the size
+    limit a fixed seeded sample of the replay rows is written, the same
+    sample for the same rows."""
+    import bench
+    from azalea_b200.engine import ROW_HEADER, replay_row_bytes
+    n, nn, R = 5, 25, 60
+    rows = np.zeros((R, replay_row_bytes(n)), dtype=np.uint8)
+    h = rows[:, :48].view(ROW_HEADER).reshape(-1)
+    h['game_id'] = np.arange(R) // 10 + (1 << 40)
+    h['ply'] = np.arange(R) % 10
+    rows[:, 48:48 + nn] = np.arange(nn) % 3
+    rows[:, 48 + 32:48 + 32 + 4 * nn] = (np.arange(R * nn, dtype='<f4') % 7).reshape(R, nn).view(np.uint8)
+    chosen = np.arange(32 * 4, dtype=np.int32).reshape(32, 4)
+
+    def dump(d):
+        bench.dump_outputs(str(d), chosen, rows, n)
+        out = {f[:-4]: np.load(d / f) for f in os.listdir(d)}
+        assert all(a.dtype in (np.float32, np.float64) for a in out.values())
+        return out
+
+    full = dump(tmp_path / 'full')
+    assert (full['chosen_move_id'] == chosen[:, 1]).all()
+    assert (full['replay_game_id'] == h['game_id']).all() and full['replay_visits'].shape == (R, nn)
+    assert (full['replay_board'][3].ravel() == np.arange(nn) % 3).all()
+    per_row = 8 * 10 + 4 * nn * 2
+    monkeypatch.setattr(bench, 'DUMP_BYTES', full['chosen_ply'].nbytes * 4 + 17 * per_row)
+    a, b = dump(tmp_path / 'a'), dump(tmp_path / 'b')
+    assert sum(x.nbytes for x in a.values()) <= bench.DUMP_BYTES
+    assert len(a['replay_ply']) == 17 and all((a[k] == b[k]).all() for k in a)
+    idx = (a['replay_game_id'] - (1 << 40)) * 10 + a['replay_ply']
+    assert (np.diff(idx) > 0).all() and (a['replay_visits'] == full['replay_visits'][idx.astype(int)]).all()
+
+
 def _gather_worker(rank, world, port, q):
     import torch.distributed as dist
     sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
