@@ -16,6 +16,7 @@ HEADER_PATH = os.path.join(os.path.dirname(_HERE), 'include', 'azalea_b200.h')
 AZ_OK = 0
 AZ_ST_POOL_FULL, AZ_ST_TREE_FULL, AZ_ST_ILLEGAL, AZ_ST_DISABLED = 1, 2, 4, 8
 AZ_LEAF_TERMINAL_KNOWN, AZ_LEAF_TERMINAL_NEW = 1, 2
+AZ_LEAF_REFLECTED_BIT = 9       # leaf_info[..][1]: the leaf's network row is rotated
 AZ_PRIOR_PROBS, AZ_PRIOR_LOGITS = 0, 1
 AZ_CFG_SOFT_POOL_FULL, AZ_CFG_PACK_LEAVES = 1, 2
 AZ_ABI_VERSION = 3
@@ -25,7 +26,8 @@ AZ_ABI_VERSION = 3
 COUNTER_NAMES = ('simulations', 'sum_children', 'sum_depth', 'unique_leaves',
                  'expanded_children', 'plies', 'games', 'replay_rows',
                  'replay_dropped', 'games_failed', 'compacted_nodes',
-                 'nn_rows', 'pool_skipped_expansions', 'terminal_leaves')
+                 'nn_rows', 'pool_skipped_expansions', 'terminal_leaves',
+                 'reflected_rows')
 ROW_HEADER_BYTES = 48
 
 
@@ -104,10 +106,12 @@ def lib():
     L.az_tree_move.argtypes = [eng, i32p, vp]
     L.az_mcts_root_uniform.argtypes = [eng, vp]
     L.az_engine_set_window.argtypes = [eng, C.c_int, C.c_int]
+    L.az_engine_set_reflect.argtypes = [eng, C.c_int]
     L.az_status.argtypes = [eng, i32p, vp]
     L.az_stub_eval.argtypes = [eng, C.c_int, vp]
     L.az_replay_collate.argtypes = [vp, C.c_int, vp, C.c_int, C.c_int, i32p, i32p,
                                     f32p, f32p, vp, vp, i32p, vp]
+    L.az_batch_reflect.argtypes = [i32p, i32p, f32p, vp, C.c_int, C.c_int, C.c_int, C.c_int, vp]
     L.az_nn_stem.argtypes = [vp, C.c_int, C.c_int, C.c_int64, vp, f32p, vp, C.c_int,
                              C.c_int, vp]
     L.az_nn_heads.argtypes = [vp, C.c_int64, f32p, f32p, vp, C.c_int64, C.c_int, C.c_int, C.c_int, vp]

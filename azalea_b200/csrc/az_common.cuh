@@ -45,6 +45,7 @@ struct az_engine {
     int device;
     int G, n, nn, NW, B, C;
     int g0, g1;             // game window [g0, g1) the per-game kernels cover (az_engine_set_window)
+    int reflect;            // 1: network rows in a random orientation (az_engine_set_reflect)
     int cell_stride;        // bytes per leaf board row (nn rounded up to 16)
     int path_stride;        // uint32 per descent path
     int row_bytes;          // replay row
@@ -187,6 +188,14 @@ __device__ __forceinline__ int az_flip_tile(int t, int n, uint32_t magic)
     int r = (int)(((uint32_t)t * magic) >> 16), c = t - r * n;
     return (n - 1 - c) * n + (n - 1 - r);
 }
+
+// Philox counter domains of the orientation coins (word w; the root noise uses 0xD1C10000)
+#define AZ_REFLECT_DOMAIN 0x5EF1EC70u
+#define AZ_REFLECT_ROOT_DOMAIN 0x5EF1EC71u
+#define AZ_LEAF_REFLECTED (1 << AZ_LEAF_REFLECTED_BIT)
+
+// Hex's one rule-preserving symmetry, the 180-degree rotation (i, j) -> (n-1-i, n-1-j)
+__device__ __forceinline__ int az_rot_tile(int t, int nn) { return nn - 1 - t; }
 
 __device__ __forceinline__ uint32_t az_orderable(float x)
 {

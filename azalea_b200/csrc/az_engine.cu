@@ -683,6 +683,43 @@ __global__ void k_replay_collate(const uint8_t *rows, int row_bytes, const int64
     }
 }
 
+// ---------------------------------------------------------- batch reflect
+
+// random_reflect of a collated training batch (the reference's hex.py:124-134
+// hook): rows with a coin are turned by 180 degrees, tile t -> n*n-1-t, in
+// place.  One warp per row; every element is swapped with its mirror by one
+// lane, so the rotation is its own inverse.
+__global__ void k_batch_reflect(int32_t *board, int32_t *moves, float *probs, const uint8_t *coins,
+                                int count, int nn, int width, int ld)
+{
+    const int lane = az_lane();
+    const int i = blockIdx.x * AZ_WARPS_PER_CTA + (threadIdx.x >> 5);
+    if (i >= count || !coins[i]) return;
+    int32_t *b = board + (size_t)i * nn;
+    for (int t = lane; t < nn / 2; t += 32) {
+        const int32_t c = b[t];
+        b[t] = b[nn - 1 - t];
+        b[nn - 1 - t] = c;
+    }
+    int32_t *m = moves + (size_t)i * ld;
+    float *p = probs + (size_t)i * ld;
+    // the legal moves are ascending and zero padded: k = non-zero entries
+    int k = 0;
+    for (int j0 = 0; j0 < width; j0 += 32) {
+        const int j = j0 + lane;
+        k += __popc(__ballot_sync(AZ_FULL, j < width && m[j] != 0));
+    }
+    for (int j = lane; j < (k + 1) / 2; j += 32) {
+        const int jr = k - 1 - j;
+        const int32_t a = m[j], z = m[jr];
+        const float pa = p[j], pz = p[jr];
+        m[j] = nn + 1 - z;
+        m[jr] = nn + 1 - a;
+        p[j] = pz;
+        p[jr] = pa;
+    }
+}
+
 // =================================================================== C ABI
 
 static size_t az_align(size_t x) { return (x + 255) & ~(size_t)255; }
@@ -971,6 +1008,13 @@ int az_engine_set_window(az_engine *e, int first_game, int num_games)
     return AZ_OK;
 }
 
+int az_engine_set_reflect(az_engine *e, int on)
+{
+    if (!e) return AZ_E_INVALID;
+    e->reflect = on != 0;
+    return AZ_OK;
+}
+
 int az_mcts_root_uniform(az_engine *e, void *stream)
 {
     if (!e) return AZ_E_INVALID;
@@ -1018,6 +1062,20 @@ int az_replay_collate(const uint8_t *rows_dev, int row_bytes, const int64_t *ind
                        (cudaStream_t)stream>>>(rows_dev, row_bytes, index_dev, count, board_size, cs,
                                                board_dev, moves_dev, probs_dev, reward_dev, color_dev,
                                                result_dev, num_moves_dev);
+    return az_check(cudaGetLastError());
+}
+
+int az_batch_reflect(int32_t *board_dev, int32_t *moves_dev, float *probs_dev,
+                     const uint8_t *coins_dev, int count, int board_size, int width, int ld,
+                     void *stream)
+{
+    if (!board_dev || !moves_dev || !probs_dev || !coins_dev || board_size < 2 || board_size > 19 ||
+        count < 0 || width < 0 || width > board_size * board_size || ld < width)
+        return AZ_E_INVALID;
+    if (count == 0) return AZ_OK;
+    k_batch_reflect<<<(count + AZ_WARPS_PER_CTA - 1) / AZ_WARPS_PER_CTA, AZ_WARPS_PER_CTA * 32, 0,
+                      (cudaStream_t)stream>>>(board_dev, moves_dev, probs_dev, coins_dev, count,
+                                              board_size * board_size, width, ld);
     return az_check(cudaGetLastError());
 }
 

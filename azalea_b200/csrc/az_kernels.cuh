@@ -51,12 +51,13 @@ struct az_expand_args {
 
 // Network-view board cells (mcts.py:176-181, hex.py:72-87): cell v of the
 // view is tile v of the board (colour 0 to move) or the colour-swapped
-// anti-diagonal mirror (colour 1 to move).  Each lane packs 4 cells into
-// one 32-bit store; the two masks are staged in shared memory so that every
-// lane can test arbitrary tiles.
+// anti-diagonal mirror (colour 1 to move); `rot` turns that view by 180
+// degrees (az_engine_set_reflect): cell v reads tile rot(flip?(v)).  Each lane
+// packs 4 cells into one 32-bit store; the two masks are staged in shared
+// memory so that every lane can test arbitrary tiles.
 __device__ __forceinline__ void az_emit_board(const az_engine &e, uint32_t *smask,
                                               uint32_t x, uint32_t o, int flip,
-                                              int8_t *dst)
+                                              int rot, int8_t *dst)
 {
     const int lane = az_lane();
     __syncwarp();
@@ -70,7 +71,8 @@ __device__ __forceinline__ void az_emit_board(const az_engine &e, uint32_t *smas
             int v = v0 + q;
             uint32_t cell = 0;
             if (v < e.nn) {
-                int t = flip ? az_flip_tile(v, e.n, e.div_magic) : v;
+                const int vr = rot ? az_rot_tile(v, e.nn) : v;
+                int t = flip ? az_flip_tile(vr, e.n, e.div_magic) : vr;
                 uint32_t bx = (smask[t >> 5] >> (t & 31)) & 1u;
                 uint32_t bo = (smask[32 + (t >> 5)] >> (t & 31)) & 1u;
                 // colour swap under flip: X(1) <-> O(2)  (hex.py:84)
@@ -81,6 +83,19 @@ __device__ __forceinline__ void az_emit_board(const az_engine &e, uint32_t *smas
         if (v0 < e.cell_stride)
             *reinterpret_cast<uint32_t *>(dst + v0) = packed;
     }
+}
+
+// One orientation coin per network row (az_engine_set_reflect) for descent b of
+// the launch, from the game's Philox key and counter (descent, ply): the same
+// for any window, stream count, graph or world size.  Everything is re-read
+// from meta here so that nothing stays live across k_select's descent loop.
+__device__ __forceinline__ int az_reflect_coin(const az_engine &e, const int32_t *meta, int b,
+                                               uint32_t domain)
+{
+    const uint2 key = make_uint2((uint32_t)e.cfg.seed ^ (uint32_t)meta[M_GID_LO],
+                                 (uint32_t)(e.cfg.seed >> 32) ^ (uint32_t)meta[M_GID_HI]);
+    const uint4 c = make_uint4((uint32_t)(meta[M_SIM] + b), 0u, (uint32_t)meta[M_PLY], domain);
+    return (int)(az_philox7(c, key).x & 1u);
 }
 
 // ------------------------------------------------------------- root noise
@@ -259,9 +274,13 @@ k_select(az_engine e, az_select_args a)
             return;
         }
         int k = az_count_bits(~(rx | ro) & valid);
+        const int coin = e.reflect ? az_reflect_coin(e, meta, 0, AZ_REFLECT_ROOT_DOMAIN) : 0;
         if (lane < e.NW) { lmask[lane] = rx; lmask[e.NW + lane] = ro; }
-        az_emit_board(e, smask, rx, ro, rcolor == 2, lboard);
-        if (lane == 0) info[0] = make_int4(0, (rcolor - 1) << 8, k, 0);
+        az_emit_board(e, smask, rx, ro, rcolor == 2, coin, lboard);
+        if (lane == 0) {
+            info[0] = make_int4(0, ((rcolor - 1) << 8) | (coin << AZ_LEAF_REFLECTED_BIT), k, 0);
+            if (coin) e.counters[(size_t)g * AZ_CNT_PER_GAME + AZ_CNT_REFLECTED_ROWS] += 1;
+        }
         return;
     }
     if (rootlink == AZ_UNEVAL || (rootlink & AZ_LINK_KMASK) == 0u) {
@@ -281,8 +300,10 @@ k_select(az_engine e, az_select_args a)
     const int sim0 = meta[M_SIM];
     const int ply = meta[M_PLY];
     int my_leaf = -1, my_depth = 0;         // lane b remembers descent b: depth | needs the network << 16 | flip << 17
+                                            // | rotated << 18
     const bool pack = (e.cfg.flags & AZ_CFG_PACK_LEAVES) != 0;
-    uint32_t sum_k = 0, sum_d = 0, uniq = 0, nn_rows = 0, term = 0;   // per launch: small
+    // per launch: small.  nn_rows counts rotated rows (az_engine_set_reflect) in its high half
+    uint32_t sum_k = 0, sum_d = 0, uniq = 0, nn_rows = 0, term = 0;
     const int k0 = (int)(rootlink & AZ_LINK_KMASK), fc0 = (int)(rootlink >> AZ_LINK_KBITS);
     uint32_t touched = 0;                   // bit s: this lane's root child lane + 32 s took a virtual loss
     if (AZ_STAGE_ROOT) {
@@ -405,7 +426,7 @@ k_select(az_engine e, az_select_args a)
             continue;
         }
         uniq++;
-        int flags = 0, kk = 0;
+        int flags = 0, kk = 0, coin = 0;
         if (link != AZ_UNEVAL) {
             flags = AZ_LEAF_TERMINAL_KNOWN;
             term++;
@@ -416,17 +437,19 @@ k_select(az_engine e, az_select_args a)
                 term++;
             } else {
                 kk = az_count_bits(~(x | o) & valid);
+                if (e.reflect) coin = az_reflect_coin(e, meta, b, AZ_REFLECT_DOMAIN);
                 // packed leaves: the board is written once the batch's rows have been reserved
-                if (!pack) az_emit_board(e, smask, x, o, color == 2, lboard + (size_t)b * e.cell_stride);
-                else if (lane == b) my_depth |= (1 << 16) | ((color == 2) << 17);
-                nn_rows++;
+                if (!pack) az_emit_board(e, smask, x, o, color == 2, coin, lboard + (size_t)b * e.cell_stride);
+                else if (lane == b) my_depth |= (1 << 16) | ((color == 2) << 17) | (coin << 18);
+                nn_rows += 1u + ((uint32_t)coin << 16);
             }
             if (lane < e.NW) {
                 lmask[(size_t)b * 2 * e.NW + lane] = x;
                 lmask[(size_t)b * 2 * e.NW + e.NW + lane] = o;
             }
         }
-        if (lane == 0) info[b] = make_int4(node, flags | ((color - 1) << 8), kk, depth);
+        if (lane == 0) info[b] = make_int4(node, flags | ((color - 1) << 8) | (coin << AZ_LEAF_REFLECTED_BIT),
+                                           kk, depth);
     }
     __syncwarp();
     if (pack) {
@@ -444,7 +467,7 @@ k_select(az_engine e, az_select_args a)
             const int r = row < cap ? row : cap - 1;
             const uint32_t lx = lane < e.NW ? lmask[(size_t)b * 2 * e.NW + lane] : 0u;
             const uint32_t lo = lane < e.NW ? lmask[(size_t)b * 2 * e.NW + e.NW + lane] : 0u;
-            az_emit_board(e, smask, lx, lo, (meta_b >> 17) & 1,
+            az_emit_board(e, smask, lx, lo, (meta_b >> 17) & 1, (meta_b >> 18) & 1,
                           e.leaf_board + ((size_t)e.g0 * e.B + r) * e.cell_stride);
             if (lane == 0) info[b].w = (meta_b & 0xffff) | (r << 10);
         }
@@ -482,8 +505,9 @@ k_select(az_engine e, az_select_args a)
         cnt[AZ_CNT_SUM_CHILDREN] += sum_k;
         cnt[AZ_CNT_SUM_DEPTH] += sum_d;
         cnt[AZ_CNT_UNIQUE_LEAVES] += uniq;
-        cnt[AZ_CNT_NN_ROWS] += nn_rows;
+        cnt[AZ_CNT_NN_ROWS] += nn_rows & 0xffffu;
         cnt[AZ_CNT_TERMINAL_LEAVES] += term;
+        if (nn_rows >> 16) cnt[AZ_CNT_REFLECTED_ROWS] += nn_rows >> 16;
     }
 }
 
@@ -517,6 +541,7 @@ k_expand_backup(az_engine e, az_expand_args a)
         const int4 inf = info[b];
         if (inf.x < 0) continue;
         const int node = inf.x, flags = inf.y & 0xff, lcolor = (inf.y >> 8) & 1;
+        const int lrot = (inf.y >> AZ_LEAF_REFLECTED_BIT) & 1;
         const int k = inf.z, depth = pack ? (inf.w & 1023) : inf.w;
         const size_t row = pack ? (size_t)e.g0 * e.B + (size_t)(inf.w >> 10) : (size_t)g * e.B + b;
         // evaluate_batch, mcts.py:192-200: terminal positions are worth -1
@@ -547,7 +572,10 @@ k_expand_backup(az_engine e, az_expand_args a)
                     // policy head tail (network.py:146-151) + mcts.py:210:
                     // gather the legal tiles' logits, log-softmax, exp.
                     // Lane owns tiles 32*s + lane; the ordinal of an empty
-                    // tile is the number of empty tiles before it.
+                    // tile is the number of empty tiles before it.  A row the
+                    // network saw rotated holds the logit of view tile u at
+                    // n*n-1-u; the lane still owns the true tile, so the
+                    // reductions below run in the same order either way.
                     const uint32_t occ = lane < e.NW
                         ? (lmask[(size_t)b * 2 * e.NW + lane] | lmask[(size_t)b * 2 * e.NW + e.NW + lane]) : ~0u;
                     const uint32_t emp = ~occ & valid;
@@ -561,7 +589,8 @@ k_expand_backup(az_engine e, az_expand_args a)
                         if ((es >> lane) & 1u) {
                             int t = 32 * s + lane;
                             ord[s] = base + __popc(es & ((1u << lane) - 1u));
-                            lg[s] = prow[lcolor ? az_flip_tile(t, e.n, e.div_magic) : t];
+                            const int u = lcolor ? az_flip_tile(t, e.n, e.div_magic) : t;
+                            lg[s] = prow[lrot ? az_rot_tile(u, e.nn) : u];
                             mx = fmaxf(mx, lg[s]);
                         }
                         base += __popc(es);

@@ -94,6 +94,7 @@ class Engine:
             if replay_rows else None
         self.cell_stride = self.leaf_board.shape[-1]
         self._spans = {}
+        self.reflect = False
 
     def span(self, first, last):
         """One contiguous uint8 view of the device block covering the buffers
@@ -216,6 +217,14 @@ class Engine:
         (0, 0: all games).  Read at launch time: see az_engine_set_window."""
         check(self.lib.az_engine_set_window(self._h, int(first_game), int(num_games)))
         self.window = (int(first_game), int(num_games) or self.num_games)
+
+    def set_reflect(self, on=True):
+        """Random orientation of the network rows (az_engine_set_reflect):
+        each leaf that goes to the evaluator is written rotated by 180 degrees
+        with probability 1/2, and the logits of such a row are read back
+        rotated.  Read at launch time: set it before capturing a graph."""
+        check(self.lib.az_engine_set_reflect(self._h, int(bool(on))))
+        self.reflect = bool(on)
 
     def root_uniform(self):
         """One visit on every child of every expanded root: the RandomPolicy

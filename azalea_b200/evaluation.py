@@ -57,7 +57,8 @@ def _policy_key(policy):
     return (policy.simulations, policy.search_batch_size,
             float(policy.exploration_coef), float(policy.exploration_temperature),
             int(policy.exploration_depth), sampling, float(noise),
-            float(policy.exploration_noise_alpha)) + kind
+            float(policy.exploration_noise_alpha),
+            bool(getattr(policy, 'random_reflect', False))) + kind
 
 
 class _Seat:
@@ -137,6 +138,8 @@ class _Seat:
         for key, by_net in self.index.items():
             games = torch.cat(list(by_net.values()))
             self._pause_all_but(games)
+            # the orientation of this group's network rows (az_engine_set_reflect)
+            eng.set_reflect(key[0] != 'random' and key[8])
             if key[0] == 'random':
                 # RandomPolicy.choose_action (random_policy.py:25-41) in terms of the
                 # tree: one visit on every child of the expanded root, then the

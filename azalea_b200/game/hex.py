@@ -118,6 +118,22 @@ class HexGame:
         return board, np.where(moves > 0, flipped, 0).astype(moves.dtype)
 
     @staticmethod
+    def rotate_board_moves(board: np.ndarray, moves: np.ndarray) \
+            -> Tuple[np.ndarray, np.ndarray]:
+        """Hex's rule-preserving symmetry, the 180-degree rotation
+        (i, j) -> (n-1-i, n-1-j), of a batch of boards [B, n, n] and their
+        ascending, zero-padded moves [B, K]: the board is reversed on both
+        axes, the k non-zero moves m of a row become n*n+1-m and are reversed
+        so that they stay ascending.  Its own inverse."""
+        assert isinstance(board, np.ndarray) and isinstance(moves, np.ndarray)
+        assert board.ndim == 3 and moves.ndim == 2 and len(board) == len(moves)
+        nn = board.shape[-1] * board.shape[-2]
+        out = np.zeros_like(moves)
+        for i, k in enumerate(np.count_nonzero(moves, axis=1)):
+            out[i, :k] = nn + 1 - moves[i, k - 1::-1] if k else 0
+        return np.ascontiguousarray(board[:, ::-1, ::-1]), out
+
+    @staticmethod
     def random_reflect(board, moves=None, rng=None):
         """hex.py:124-134: a no-op in the reference (consumes no RNG)."""
         if moves is not None:

@@ -44,6 +44,7 @@ class Player:
             exploration_temperature=policy.exploration_temperature,
             move_sampling=settings.get('move_sampling', True),
             move_exploration=settings.get('move_exploration', True),
+            random_reflect=getattr(policy, 'random_reflect', False),
             seed=seed, **kwargs)
         self.running = True
 

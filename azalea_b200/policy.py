@@ -6,6 +6,13 @@ with the reference's config keys, ``state_dict`` / ``load_state_dict`` /
 ``load`` with the reference's checkpoint format (the shipped
 ``hex11-20180712-3362.policy.pth`` loads), and the host ``RandomState`` that
 draws the move, so seeded deterministic play reproduces the reference's.
+
+``random_reflect`` (config key, default off) shows every position the network
+evaluates in a random one of Hex's two rule-preserving orientations (the
+180-degree rotation), in the search and in training.  It is saved with the
+policy; checkpoints without the key load with it off.  In
+``choose_action`` the orientation coins come from the policy's
+``RandomState``, so with it on the sampled moves differ from a run with it off.
 """
 from typing import Any, Dict, Optional, Tuple
 
@@ -42,6 +49,7 @@ class Policy:
         }
         self.rng = np.random.RandomState()
         self.seed()
+        self.random_reflect = False
 
     def initialize(self, config):
         """Initialize policy for training (policy.py:36-63)."""
@@ -64,6 +72,7 @@ class Policy:
         self.exploration_noise_alpha = config['exploration_noise_alpha']
         self.exploration_noise_scale = config['exploration_noise_scale']
         self.exploration_temperature = config['exploration_temperature']
+        self.random_reflect = bool(config.get('random_reflect', False))
         if 'seed' in config:
             self.seed(config['seed'])
 
@@ -99,6 +108,7 @@ class Policy:
         self.net.load_state_dict(state['net'])
         for key in self.SEARCH_KEYS:
             setattr(self, key, state[key])
+        self.random_reflect = bool(state.get('random_reflect', False))
         if 'rng' in state:
             self.rng.__setstate__(state['rng'])
 
@@ -108,6 +118,7 @@ class Policy:
                  'rng': self.rng.__getstate__()}
         for key in self.NET_KEYS + self.SEARCH_KEYS:
             state[key] = getattr(self, key)
+        state['random_reflect'] = self.random_reflect
         return state
 
     def choose_action(self, game) -> Tuple[int, Dict[str, Any]]:
@@ -131,6 +142,7 @@ class Policy:
             batch_size=self.search_batch_size,
             exploration_coef=self.exploration_coef,
             exploration_noise_alpha=self.exploration_noise_alpha,
+            random_reflect=self.random_reflect,
             rng=self.rng)
         move_id = np.argmax(self.rng.multinomial(1, probs))
         legal_moves = game.state.legal_moves

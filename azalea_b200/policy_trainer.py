@@ -20,7 +20,11 @@ Deviations from the reference, all on purpose:
   ``num_dataloader_workers`` are ignored, ``num_selfplay_games`` (default
   1024) sets how many games are resident on the GPU;
 * ``game`` may be ``'hex'`` or a dotted class path;
-* tensorboard monitoring is out of scope: scalars go to ``logging``.
+* tensorboard monitoring is out of scope: scalars go to ``logging``;
+* ``random_reflect`` (default off) is honoured: each minibatch sample is
+  rotated by 180 degrees with probability 1/2 (``DeviceReplayBuffer.sample``,
+  coins from the seeded device generator), and the self-play search shows the
+  network its leaves in random orientations (the policy's setting).
 """
 import logging
 import os
@@ -251,6 +255,7 @@ def train(policy, config, rundir, *,
         player = DistributedSelfPlay(player, policy.net)
     sampler = torch.Generator(device=device)
     sampler.manual_seed(seed)
+    reflect = bool(config.get('random_reflect', False))
 
     log_interval = config.get('log_interval', 0)
     ckpt_interval = config.get('model_checkpoint_interval', 0)
@@ -258,7 +263,7 @@ def train(policy, config, rundir, *,
     start_time = time.time()
     history = []
     for step in range(total_steps):
-        batch = replaybuf.sample(batch_size, generator=sampler)
+        batch = replaybuf.sample(batch_size, generator=sampler, reflect=reflect)
         batch = game_class.random_reflect(batch)
         output, loss_ = supervised_step(policy.net, batch, train=True,
                                         optimizer=optimizer, device=device)

@@ -76,17 +76,24 @@ class DeviceReplayBuffer:
         self.fresh_counter = state['fresh_counter']
 
     def sample(self, batch_size: int, generator: Optional[torch.Generator] = None,
-               trim: bool = True) -> Dict[str, torch.Tensor]:
+               trim: bool = True, reflect: bool = False) -> Dict[str, torch.Tensor]:
         """A uniformly sampled minibatch as the reference's collated dict:
         ``board`` int32 [B,n,n], ``legal_moves`` int32 [B,K], ``moves_prob``
         f32 [B,K], ``reward`` f32 [B], ``color``/``result`` int64 [B].  With
         ``trim`` K is the longest legal-move list in the batch (prep.pad,
-        one host sync); otherwise K = n*n."""
+        one host sync); otherwise K = n*n.  With ``reflect`` each sample is
+        rotated by 180 degrees with probability 1/2 (``reflect_batch``; the
+        coins come from ``generator`` after the row indices)."""
         if self.size == 0:
             raise RuntimeError('replay buffer is empty')
         idx = torch.randint(0, self.size, (batch_size,), device=self.device,
                             generator=generator, dtype=torch.int64)
-        return self.collate(idx, trim=trim)
+        batch = self.collate(idx, trim=trim)
+        if reflect:
+            coins = torch.randint(0, 2, (batch_size,), device=self.device,
+                                  generator=generator, dtype=torch.uint8)
+            reflect_batch(batch, coins)
+        return batch
 
     def collate(self, idx: torch.Tensor, trim: bool = True):
         B, nn, dev = idx.numel(), self.nn, self.device
@@ -108,3 +115,22 @@ class DeviceReplayBuffer:
             moves, probs = moves[:, :K], probs[:, :K]
         return dict(color=color, legal_moves=moves, result=result, board=board,
                     moves_prob=probs, reward=reward)
+
+
+def reflect_batch(batch: Dict[str, torch.Tensor], coins: torch.Tensor) -> None:
+    """Hex's 180-degree rotation of the collated samples whose coin (uint8 [B],
+    device) is non-zero, in place (az_batch_reflect): ``board`` is reversed on
+    both axes, the k legal moves m become n*n+1-m and, like their
+    ``moves_prob``, are reversed so that they stay ascending; padding stays
+    zero.  Its own inverse for the same coins."""
+    board, moves, probs = batch['board'], batch['legal_moves'], batch['moves_prob']
+    B, n = board.shape[0], board.shape[-1]
+    assert board.dtype == torch.int32 and board.is_contiguous()
+    assert moves.dtype == torch.int32 and probs.dtype == torch.float32
+    assert moves.shape == probs.shape and moves.stride() == probs.stride() and moves.stride(1) == 1
+    coins = coins.to(board.device, torch.uint8).contiguous()
+    assert coins.numel() == B
+    p = lambda t: C.c_void_p(t.data_ptr())
+    stream = C.c_void_p(torch.cuda.current_stream(board.device).cuda_stream)
+    _cabi.check(_cabi.lib().az_batch_reflect(
+        p(board), p(moves), p(probs), p(coins), B, n, moves.shape[1], moves.stride(0), stream))

@@ -21,7 +21,7 @@ from numpy.random import RandomState
 
 from . import _cabi
 from .engine import Engine
-from .game.hex import default_device
+from .game.hex import HexGame, default_device
 
 # search_tree.py:17-18
 MAX_NODES = 10000000
@@ -130,9 +130,14 @@ class SearchTree:
                exploration_noise_scale: float = 1.0,
                exploration_noise_alpha: float = 1.0,
                batch_size: int = 10,
-               rng: Optional[RandomState] = None) \
+               rng: Optional[RandomState] = None,
+               random_reflect: bool = False) \
             -> Tuple[np.ndarray, float, Dict[str, Any]]:
         """Plan next moves with batched MCTS (search_tree.py:73-113).
+
+        ``random_reflect``: every position handed to ``network.run`` is
+        rotated by 180 degrees with probability 1/2 (one ``rng`` draw per
+        position, so the later move draws differ from a run without it).
 
         :return: next move probabilities, game value, debug metrics
         """
@@ -156,7 +161,7 @@ class SearchTree:
             metrics = self._sample_paths(
                 eng, game, network, num_simulations, batch_size,
                 exploration_coef, exploration_noise_scale,
-                exploration_noise_alpha, rng)
+                exploration_noise_alpha, rng, random_reflect)
 
         visits, _, _, root_n, root_w = self.root_stats()
         move_probs = as_distribution(visits, temperature)
@@ -169,19 +174,19 @@ class SearchTree:
 
     # ------------------------------------------------------ mcts.py glue --
     def _sample_paths(self, eng, game, net, num_simulations, batch_size,
-                      coef, noise_scale, noise_alpha, rng):
+                      coef, noise_scale, noise_alpha, rng, reflect=False):
         """mcts.sample_paths (mcts.py:258-293) around the device kernels."""
         num_batches = num_simulations // batch_size + 1
         search_value = 0
         if not self.root_is_evaluated():
             # evaluate_root, mcts.py:18-27 (value discarded)
             eng.select_root()
-            self._evaluate(eng, game, net, rng)
+            self._evaluate(eng, game, net, rng, reflect)
             eng.expand_root()
             self._raise_if_full()
         for _ in range(num_batches):
             eng.select(batch_size, coef, noise_scale, noise_alpha)
-            values = self._evaluate(eng, game, net, rng)
+            values = self._evaluate(eng, game, net, rng, reflect)
             eng.expand_backup()
             search_value += np.sum(values)
         self._raise_if_full()
@@ -213,7 +218,7 @@ class SearchTree:
             self._hb = hb
         return hb
 
-    def _evaluate(self, eng, game, net, rng):
+    def _evaluate(self, eng, game, net, rng, reflect=False):
         """mcts.evaluate_batch (mcts.py:155-217) for the leaves the select
         kernel just produced.  Returns the values in leaf-list order
         (terminal rows included).  One device-to-host copy + sync and one
@@ -244,8 +249,14 @@ class SearchTree:
                 'result': np.zeros(len(live), dtype=np.int64),
                 'board': boards.reshape(-1, n, n).astype(np.int32),
             }
-            # random_reflect is a no-op and takes no random numbers
-            # (hex.py:124-134)
+            # the reference's random_reflect is a no-op and takes no random
+            # numbers (hex.py:124-134); with `reflect` a coin per position
+            # rotates it, and its priors (by move ordinal) are turned back below
+            coins = rng.randint(2, size=len(live)).astype(bool) if reflect else None
+            if coins is not None and coins.any():
+                batch['board'][coins], batch['legal_moves'][coins] = \
+                    HexGame.rotate_board_moves(batch['board'][coins],
+                                               batch['legal_moves'][coins])
             tbatch = {}
             for k in batch:
                 tbatch[k] = torch.from_numpy(batch[k])
@@ -257,6 +268,10 @@ class SearchTree:
             assert (prior >= 0.0).all(), 'negative prior prob'
             assert (np.abs(prior.sum(1) - 1.0) < 1e-4).all(), \
                 'prior probs normalized incorrectly'
+            if coins is not None:
+                for i in np.flatnonzero(coins):
+                    k = int(info[live[i], 2])
+                    prior[i, :k] = prior[i, k - 1::-1].copy()
             values[~term] = nonterm_value
             hb['value'][live] = nonterm_value
             hb['prior'][live, :prior.shape[1]] = prior

@@ -68,7 +68,8 @@ class LockstepSelfPlay:
                  move_sampling=True, move_exploration=True, seed=0,
                  device=None, rank=0, world_size=1, nodes_per_game=None,
                  replay_rows=None, collect_replay=True, cuda_graph=True,
-                 max_plies=300, random_play=False, streams=None, pack_leaves=None):
+                 max_plies=300, random_play=False, streams=None, pack_leaves=None,
+                 random_reflect=False):
         # random_play: RandomPolicy self-play (random_policy.py:25-41) -- no
         # search, uniform move choice and uniform moves_prob at every ply;
         # how the reference fills the replay buffer before training
@@ -116,6 +117,12 @@ class LockstepSelfPlay:
                           seed=seed, first_game_id=rank * self.G,
                           game_id_stride=world_size * self.G, device=device,
                           soft_pool_full=True, pack_leaves=self.pack_leaves)
+        # random_reflect: every leaf the network evaluates is shown in a random one of
+        # Hex's two rule-preserving orientations (az_engine_set_reflect); part of the
+        # captured graph, so it is fixed for the life of this object
+        self.random_reflect = bool(random_reflect) and not self.random_play
+        if self.random_reflect:
+            self.eng.set_reflect(True)
         self.device = self.eng.device
         self.chosen = torch.zeros(self.G, 4, dtype=torch.int32,
                                   device=self.device)

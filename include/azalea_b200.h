@@ -59,6 +59,8 @@ enum {
     AZ_LEAF_TERMINAL_KNOWN = 1, /* re-visited terminal node, mcts.py:236-237 */
     AZ_LEAF_TERMINAL_NEW = 2    /* first visit found the game over */
 };
+/* leaf_info[..][1] bit 9: the leaf's network row is rotated (az_engine_set_reflect) */
+#define AZ_LEAF_REFLECTED_BIT 9
 
 typedef struct az_config {
     int32_t num_games;       /* G: games resident on this GPU */
@@ -103,7 +105,7 @@ typedef struct az_engine az_engine;
 /* buffers the caller may view inside its device block */
 enum {
     AZ_BUF_LEAF_BOARD = 0,  /* int8  [G][max_batch][cell_stride]  network-view cells 0/1/2 */
-    AZ_BUF_LEAF_INFO = 1,   /* int32 [G][max_batch][4] node(-1 = none), flags|colour<<8, num_moves, depth
+    AZ_BUF_LEAF_INFO = 1,   /* int32 [G][max_batch][4] node(-1 = none), flags|colour<<8|rotated<<9, num_moves, depth
                                (AZ_CFG_PACK_LEAVES: depth | row << 10) */
     AZ_BUF_VALUE = 2,       /* f32   [G][max_batch]           evaluator output */
     AZ_BUF_PRIOR = 3,       /* f32   [G][max_batch][n*n]      evaluator output (priors or logits) */
@@ -133,7 +135,8 @@ enum {
     AZ_CNT_COMPACTED_NODES = 10,
     AZ_CNT_NN_ROWS = 11,      /* non-terminal unique leaves (rows the network must evaluate) */
     AZ_CNT_POOL_SKIPPED = 12, /* expansions skipped because the pool half was full (AZ_CFG_SOFT_POOL_FULL) */
-    AZ_CNT_TERMINAL_LEAVES = 13 /* unique leaves that were terminal positions (value -1, mcts.py:192-195) */
+    AZ_CNT_TERMINAL_LEAVES = 13, /* unique leaves that were terminal positions (value -1, mcts.py:192-195) */
+    AZ_CNT_REFLECTED_ROWS = 14  /* network rows written rotated (az_engine_set_reflect) */
 };
 
 typedef struct az_buffer_desc {
@@ -171,6 +174,22 @@ int az_replay_row_bytes(const az_engine *e);
  * streams: the tree kernels of one half run under the evaluator of the other
  * (selfplay.LockstepSelfPlay(streams=2)). */
 int az_engine_set_window(az_engine *e, int first_game, int num_games);
+
+/* Random orientation of the network rows (the reference's random_reflect
+ * hook, mcts.py:179-186), off by default.  Hex has one symmetry that keeps
+ * the rules: the 180-degree rotation tile t -> n*n-1-t.  With on != 0,
+ * az_mcts_select and az_mcts_select_root draw one coin per leaf that goes to
+ * the network from the game's Philox stream (counter: descent, ply) and, when
+ * it is set, write the leaf's AZ_BUF_LEAF_BOARD row rotated and set
+ * AZ_LEAF_REFLECTED in leaf_info[..][1]; the AZ_PRIOR_LOGITS path of
+ * az_mcts_expand_backup / az_mcts_expand_root reads the logit of tile t of a
+ * rotated row at n*n-1-t.  Coins do not depend on windows, streams or the
+ * world size.  AZ_PRIOR_PROBS priors (by move ordinal), az_stub_eval and
+ * az_leaf_moves refer to the true board and ignore the orientation: a host
+ * evaluator leaves this off and rotates its own batch.  Read at launch time
+ * like the window (set it before capturing a graph).  Off: every buffer is
+ * byte for byte what it is without this call. */
+int az_engine_set_reflect(az_engine *e, int on);
 
 /* HexGame.reset + Policy.reset for the games whose mask byte is non-zero
  * (NULL = all), hex.py:47-49, policy.py:72-76, search_tree.py:59-71. */
@@ -273,6 +292,17 @@ int az_replay_collate(const uint8_t *rows_dev, int row_bytes,
                       int32_t *board_dev, int32_t *moves_dev, float *probs_dev,
                       float *reward_dev, int64_t *color_dev, int64_t *result_dev,
                       int32_t *num_moves_dev, void *stream);
+
+/* random_reflect for training samples: rotates the rows i of a collated batch
+ * whose coins_dev[i] (uint8) is non-zero by 180 degrees, in place.  board
+ * int32[count][n*n]; legal_moves int32 and moves_prob f32 rows of `ld`
+ * elements, of which the first `width` hold the ascending, zero-padded moves
+ * and their probabilities: the k non-zero moves m become n*n+1-m and, like
+ * their probabilities, are reversed, so the list stays ascending; padding
+ * stays zero.  Applying it twice with the same coins is the identity. */
+int az_batch_reflect(int32_t *board_dev, int32_t *moves_dev, float *probs_dev,
+                     const uint8_t *coins_dev, int count, int board_size, int width,
+                     int ld, void *stream);
 
 /* ------------------------------------------------------- evaluator glue */
 
