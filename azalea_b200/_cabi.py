@@ -27,7 +27,7 @@ COUNTER_NAMES = ('simulations', 'sum_children', 'sum_depth', 'unique_leaves',
                  'expanded_children', 'plies', 'games', 'replay_rows',
                  'replay_dropped', 'games_failed', 'compacted_nodes',
                  'nn_rows', 'pool_skipped_expansions', 'terminal_leaves',
-                 'reflected_rows')
+                 'reflected_rows', 'fast_plies')
 ROW_HEADER_BYTES = 48
 
 
@@ -107,6 +107,7 @@ def lib():
     L.az_mcts_root_uniform.argtypes = [eng, vp]
     L.az_engine_set_window.argtypes = [eng, C.c_int, C.c_int]
     L.az_engine_set_reflect.argtypes = [eng, C.c_int]
+    L.az_engine_set_playout_cap.argtypes = [eng, C.c_float, C.c_int]
     L.az_status.argtypes = [eng, i32p, vp]
     L.az_stub_eval.argtypes = [eng, C.c_int, vp]
     L.az_replay_collate.argtypes = [vp, C.c_int, vp, C.c_int, C.c_int, i32p, i32p,

@@ -37,7 +37,8 @@ enum {
     M_GID_LO = 10,  // global game id (Philox stream)
     M_GID_HI = 11,
     M_DRAW = 12,    // game hit max_plies without a winner (play_game.py:59-61)
-    M_LAST = 13     // last tile played (-1 none)
+    M_LAST = 13,    // last tile played (-1 none)
+    M_PLY_SIM0 = 14 // M_SIM when this move's search began (az_engine_set_playout_cap)
 };
 
 struct az_engine {
@@ -46,6 +47,8 @@ struct az_engine {
     int G, n, nn, NW, B, C;
     int g0, g1;             // game window [g0, g1) the per-game kernels cover (az_engine_set_window)
     int reflect;            // 1: network rows in a random orientation (az_engine_set_reflect)
+    int fast_descents;      // > 0: playout cap on, new descents of a fast ply (az_engine_set_playout_cap)
+    unsigned long long full_thresh;     // a ply is a full search iff its coin < full_thresh
     int cell_stride;        // bytes per leaf board row (nn rounded up to 16)
     int path_stride;        // uint32 per descent path
     int row_bytes;          // replay row
@@ -227,6 +230,22 @@ __device__ __forceinline__ uint4 az_philox7(uint4 c, uint2 k)
         k.x += 0x9E3779B9u; k.y += 0xBB67AE85u;
     }
     return c;
+}
+
+// Philox counter domain of the playout cap's full-search coin (word w)
+#define AZ_FULL_SEARCH_DOMAIN 0xCA9F5EA7u
+
+// Playout cap (az_engine_set_playout_cap): does the current ply of this game get the full
+// search?  One coin per (seed, global game id, ply), so the answer does not depend on windows,
+// streams, graphs or the world size.  Everything is re-read from meta so that nothing stays
+// live across k_select's descent loop.
+__device__ __forceinline__ bool az_full_search(const az_engine &e, const int32_t *meta)
+{
+    if (e.fast_descents == 0) return true;
+    const uint2 key = make_uint2((uint32_t)e.cfg.seed ^ (uint32_t)meta[M_GID_LO],
+                                 (uint32_t)(e.cfg.seed >> 32) ^ (uint32_t)meta[M_GID_HI]);
+    const uint4 c = make_uint4((uint32_t)meta[M_PLY], 0u, 0u, AZ_FULL_SEARCH_DOMAIN);
+    return (unsigned long long)az_philox(c, key).x < e.full_thresh;
 }
 
 __device__ __forceinline__ float az_u01(uint32_t r)     // (0,1)

@@ -521,6 +521,8 @@ k_play_commit(az_engine e, az_play_params p, int32_t *chosen)
     const uint32_t o = lane < e.NW ? e.board[((size_t)g * 2 + 1) * e.NW + lane] : 0u;
     const int tile = az_kth_empty(~(x | o) & valid, move_id, e.NW);
     const int color = meta[M_COLOR];
+    // playout cap: this ply had the fast search; its row stays out of the replay output
+    const bool fast = !az_full_search(e, meta);
 
     // replay row before the move (play_game.py:90-96)
     if (p.collect_replay && ply < e.hist_rows) {
@@ -537,7 +539,7 @@ k_play_commit(az_engine e, az_play_params p, int32_t *chosen)
             h.move = tile + 1;
             h.move_id = move_id;
             h.game_len = 0;
-            h.reserved = 0;
+            h.reserved = fast ? 1 : 0;      // history rows only: flushed rows keep 0
             *reinterpret_cast<az_row_header *>(row) = h;
         }
         int8_t *cells = reinterpret_cast<int8_t *>(row + sizeof(az_row_header));
@@ -568,6 +570,7 @@ k_play_commit(az_engine e, az_play_params p, int32_t *chosen)
     }
     if (lane == 0) {
         cnt[AZ_CNT_PLIES] += 1;
+        if (fast) cnt[AZ_CNT_FAST_PLIES] += 1;
         if (chosen) reinterpret_cast<int4 *>(chosen)[g] = make_int4(tile + 1, move_id, result, nply);
     }
     if (!over) return;
@@ -575,7 +578,16 @@ k_play_commit(az_engine e, az_play_params p, int32_t *chosen)
     // play_game.py:63-67: reward = result - 2 for the first player's rows,
     // negated on the second player's
     if (p.collect_replay) {
-        const int rows = min(nply, e.hist_rows);
+        const int plies = min(nply, e.hist_rows);
+        const uint8_t *src = e.hist + (size_t)g * e.hist_rows * e.row_bytes;
+        // playout cap: only the rows of full-search plies (reserved bit 0 clear) are flushed
+        int rows = plies;
+        if (e.fast_descents) {
+            int kept = 0;
+            for (int r = lane; r < plies; r += 32)
+                kept += !(reinterpret_cast<const az_row_header *>(src + (size_t)r * e.row_bytes)->reserved & 1);
+            rows = __reduce_add_sync(AZ_FULL, kept);
+        }
         // reserve `rows` output rows; the cursor only ever advances by reservations that fit,
         // so concurrent finishers can never be handed space beyond the capacity
         unsigned long long base = ~0ull;
@@ -590,16 +602,28 @@ k_play_commit(az_engine e, az_play_params p, int32_t *chosen)
         }
         base = __shfl_sync(AZ_FULL, base, 0);
         if (base != ~0ull) {
-            const uint8_t *src = e.hist + (size_t)g * e.hist_rows * e.row_bytes;
             uint8_t *dst = e.replay + (size_t)base * e.row_bytes;
-            const size_t n16 = (size_t)rows * e.row_bytes / 16;
-            for (size_t i = lane; i < n16; i += 32)
-                reinterpret_cast<uint4 *>(dst)[i] = reinterpret_cast<const uint4 *>(src)[i];
+            if (rows == plies) {
+                const size_t n16 = (size_t)rows * e.row_bytes / 16;
+                for (size_t i = lane; i < n16; i += 32)
+                    reinterpret_cast<uint4 *>(dst)[i] = reinterpret_cast<const uint4 *>(src)[i];
+            } else {
+                // the kept rows, compacted in ply order
+                const int n16 = e.row_bytes / 16;
+                uint8_t *d = dst;
+                for (int r = 0; r < plies; r++) {
+                    const uint8_t *s = src + (size_t)r * e.row_bytes;
+                    if (reinterpret_cast<const az_row_header *>(s)->reserved & 1) continue;
+                    for (int i = lane; i < n16; i += 32)
+                        reinterpret_cast<uint4 *>(d)[i] = reinterpret_cast<const uint4 *>(s)[i];
+                    d += e.row_bytes;
+                }
+            }
             __syncwarp();
             for (int r = lane; r < rows; r += 32) {
                 az_row_header *h = reinterpret_cast<az_row_header *>(dst + (size_t)r * e.row_bytes);
                 float rw = (float)(result - 2);
-                h->reward = (r & 1) ? -rw : rw;
+                h->reward = (h->ply & 1) ? -rw : rw;    // the row's own ply (rows may be skipped)
                 h->result = result;
                 h->game_len = nply;
             }
@@ -1012,6 +1036,21 @@ int az_engine_set_reflect(az_engine *e, int on)
 {
     if (!e) return AZ_E_INVALID;
     e->reflect = on != 0;
+    return AZ_OK;
+}
+
+int az_engine_set_playout_cap(az_engine *e, float full_search_prob, int fast_descents)
+{
+    if (!e || !(full_search_prob >= 0.0f)) return AZ_E_INVALID;     // (NaN fails the test)
+    if (full_search_prob >= 1.0f) {
+        e->fast_descents = 0;
+        e->full_thresh = 0;
+        return AZ_OK;
+    }
+    if (fast_descents < 1) return AZ_E_INVALID;
+    e->fast_descents = fast_descents;
+    // coin < p * 2^32 for an integer coin is coin < ceil(p * 2^32); exact in double
+    e->full_thresh = (unsigned long long)ceil((double)full_search_prob * 4294967296.0);
     return AZ_OK;
 }
 

@@ -257,6 +257,14 @@ k_select(az_engine e, az_select_args a)
         if (lane < e.B) info[lane] = make_int4(-1, 0, 0, 0);
         return;
     }
+    // playout cap: a fast ply's search ends once it has made fast_descents new descents (the
+    // unsigned difference: M_SIM is a running counter of the slot)
+    if (!a.root_mode && e.fast_descents &&
+        (uint32_t)(meta[M_SIM] - meta[M_PLY_SIM0]) >= (uint32_t)e.fast_descents &&
+        !az_full_search(e, meta)) {
+        if (lane < e.B) info[lane] = make_int4(-1, 0, 0, 0);
+        return;
+    }
     uint4 *nodes = e.nodes + ((size_t)g * 2 + meta[M_HALF]) * e.C;
     const uint32_t valid = az_valid_word(lane, e.nn);
     const uint32_t rx = lane < e.NW ? e.board[((size_t)g * 2 + 0) * e.NW + lane] : 0u;
@@ -267,6 +275,9 @@ k_select(az_engine e, az_select_args a)
     int8_t *lboard = e.leaf_board + (size_t)g * e.B * e.cell_stride;
 
     if (a.root_mode) {
+        // every lockstep move starts here: the playout cap counts this move's new descents from
+        // this point, tree reuse or not
+        if (e.fast_descents && lane == 0) meta[M_PLY_SIM0] = meta[M_SIM];
         // evaluate_root (mcts.py:18-24): the root position itself is the leaf
         if (lane < e.B && lane > 0) info[lane] = make_int4(-1, 0, 0, 0);
         if (rootlink != AZ_UNEVAL) {
@@ -335,9 +346,11 @@ k_select(az_engine e, az_select_args a)
             const int sum_n = __reduce_add_sync(AZ_FULL, ni);
             const float sq = __fsqrt_rn((float)sum_n);
             const bool sq_zero = sum_n == 0;
-            // (drawn after the record loads have been issued: the generator hides their latency)
+            // (drawn after the record loads have been issued: the generator hides their latency;
+            // a fast ply of the playout cap draws and mixes none, warp-uniformly)
             float noise[MAXS];
-            if (NOISE && depth == 0)
+            const bool mix = NOISE && depth == 0 && az_full_search(e, meta);
+            if (mix)
                 az_dirichlet_noise<MAXS>(lane, k, (float)a.noise_alpha, (uint32_t)(sim0 + b),
                                          (uint32_t)ply, key, noise);
             uint32_t bestkey = 0;
@@ -353,7 +366,7 @@ k_select(az_engine e, az_select_args a)
                 const int j = lane + 32 * s;
                 const float nv = __uint_as_float(rec[s].x), tv = __uint_as_float(rec[s].y);
                 float pr = __uint_as_float(rec[s].z);
-                if (NOISE && depth == 0)    // mcts.py:128-131, mixed in float64
+                if (mix)                    // mcts.py:128-131, mixed in float64
                     pr = (float)((1.0 - a.noise_scale) * (double)pr +
                                  a.noise_scale * (double)noise[s]);
                 const float cp = __fmul_rn(a.coef, pr);

@@ -226,6 +226,17 @@ class Engine:
         check(self.lib.az_engine_set_reflect(self._h, int(bool(on))))
         self.reflect = bool(on)
 
+    def set_playout_cap(self, full_search_prob=1.0, fast_descents=0):
+        """Playout cap randomization (az_engine_set_playout_cap): each ply of
+        each game is a full search with probability ``full_search_prob``
+        (one coin per game id and ply); otherwise ``select`` stops after
+        ``fast_descents`` new descents this move, with no root noise, and the
+        ply's replay row is not flushed.  ``full_search_prob >= 1`` is off.
+        Every move must begin with ``select_root``.  Read at launch time: set
+        it before capturing a graph."""
+        check(self.lib.az_engine_set_playout_cap(self._h, float(full_search_prob),
+                                                 int(fast_descents)))
+
     def root_uniform(self):
         """One visit on every child of every expanded root: the RandomPolicy
         seat (random_policy.py:25-41) in terms of the tree."""
@@ -330,6 +341,10 @@ def decode_replay_rows(rows, board_size):
     int32 ply, color, num_moves, f32 reward, int32 result, f32 temperature,
     int32 move, move_id, game_len, reserved; then int8 board[cell_stride]
     (absolute view, before the move), then f32 visits[n*n] by move ordinal.
+    With the playout cap on (``Engine.set_playout_cap``) the rows of fast
+    plies never reach the output: a game's rows may skip plies, while
+    ``game_len`` and ``result`` are still the whole game's and ``reward``
+    follows the row's own ply.
     """
     rows = np.ascontiguousarray(rows)
     n, nn = board_size, board_size * board_size

@@ -52,17 +52,21 @@ class Player:
         """Play self-play games until ``size`` positions are available."""
         examples = ReplayDataFrame()
         metrics: Metrics = defaultdict(int)
+        fast0 = self.sp.counters()['fast_plies']
         while len(examples) < size:
             self.sp.step_move()
             if self.sp.eng.replay_count() == 0:
                 continue
             rows = self.sp.harvest()
             h, _, _ = decode_replay_rows(rows, self.board_size)
-            last = np.flatnonzero(np.r_[h['ply'][1:] == 0, True])
+            # rows come sorted by (game id, ply); a game's first or last ply may have no row
+            # (playout cap), so games are told apart by id and measured by game_len
+            last = np.flatnonzero(np.r_[h['game_id'][1:] != h['game_id'][:-1], True])
             metrics['games'] += len(last)
-            metrics['moves_per_game'] += float(np.sum(h['ply'][last] + 1))
+            metrics['moves_per_game'] += float(np.sum(h['game_len'][last]))
             metrics['reward'] += float(np.sum(h['reward'][last]))
             examples.append(rows_to_dataframe(rows, self.board_size))
+        metrics['fast_plies'] = self.sp.counters()['fast_plies'] - fast0
         self._report(metrics)
         return examples, metrics
 
@@ -85,7 +89,7 @@ class Player:
         eng = self.sp.eng
         chunks, total = [], 0
         metrics: Metrics = defaultdict(int)
-        games0 = self.sp.counters()['games']
+        cnt0 = self.sp.counters()
         while total < size:
             self.sp.step_move()
             count = min(eng.replay_count(), eng.replay.shape[0])
@@ -93,7 +97,9 @@ class Player:
                 chunks.append(eng.replay[:count].clone())
                 eng.replay_clear()
                 total += count
-        metrics['games'] = self.sp.counters()['games'] - games0
+        cnt = self.sp.counters()
+        metrics['games'] = cnt['games'] - cnt0['games']
+        metrics['fast_plies'] = cnt['fast_plies'] - cnt0['fast_plies']
         metrics['moves_per_game'] = float(total)
         self._report(metrics)
         return torch.cat(chunks), metrics

@@ -24,7 +24,12 @@ Deviations from the reference, all on purpose:
 * ``random_reflect`` (default off) is honoured: each minibatch sample is
   rotated by 180 degrees with probability 1/2 (``DeviceReplayBuffer.sample``,
   coins from the seeded device generator), and the self-play search shows the
-  network its leaves in random orientations (the policy's setting).
+  network its leaves in random orientations (the policy's setting);
+* ``full_search_prob`` (default 1.0, off) and ``fast_simulations`` turn on
+  playout cap randomization (Wu 2019) in the self-play refills: a ply gets the
+  full search with probability ``full_search_prob`` and otherwise a fast one of
+  ``fast_simulations`` without root noise, and only full-search plies become
+  training rows, so a refill finishes more games per GPU-second.
 """
 import logging
 import os
@@ -198,6 +203,10 @@ def train(policy, config, rundir, *,
     batch_size = config['batch_size']
     num_games = int(config.get('num_selfplay_games', 1024))
 
+    # playout cap randomization: a self-play setting, not part of the policy (not checkpointed)
+    cap = dict(full_search_prob=float(config.get('full_search_prob', 1.0)),
+               fast_simulations=config.get('fast_simulations'))
+
     game_class = _game_class(config['game'])
     game_factory = partial(game_class, board_size=config['board_size'])
 
@@ -213,7 +222,7 @@ def train(policy, config, rundir, *,
         agent = AzaleaAgent(game_factory, policy=policy, device=str(device))
         worker = DistributedSelfPlay(
             _TrainingPlayer(Player(None, [agent], num_games=num_games, seed=seed & 0x7fffffff,
-                                   device=device, rank=rank, world_size=world), policy.net),
+                                   device=device, rank=rank, world_size=world, **cap), policy.net),
             policy.net)
         served = worker.serve()
         logging.info(f'rank {rank}: served {served} replay refills')
@@ -250,7 +259,7 @@ def train(policy, config, rundir, *,
     # instantiate game and wrap it together with policy
     agent = AzaleaAgent(game_factory, policy=policy, device=str(device))
     player = _TrainingPlayer(Player(None, [agent], num_games=num_games, seed=seed & 0x7fffffff,
-                                    device=device, rank=rank, world_size=world), policy.net)
+                                    device=device, rank=rank, world_size=world, **cap), policy.net)
     if dist:
         player = DistributedSelfPlay(player, policy.net)
     sampler = torch.Generator(device=device)

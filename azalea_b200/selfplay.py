@@ -52,6 +52,30 @@ def default_nodes_per_game(num_games, num_tiles, sims_per_move, device=None,
     return int(min(want, (1 << 23) - 1))
 
 
+def playout_cap_descents(full_search_prob, fast_simulations, simulations, search_batch_size):
+    """New descents of a fast ply under playout cap randomization, 0 = off.
+
+    The reference's rule for a full search (mcts.py:268, ``num_batches =
+    sims // batch + 1``) applied to ``fast_simulations``.  Raises
+    ``ValueError`` unless ``full_search_prob`` is a number >= 0 and, when it
+    is below 1, ``fast_simulations`` gives fewer descents than a full search.
+    """
+    p = float(full_search_prob)
+    if not p >= 0.0:
+        raise ValueError(f'full_search_prob must be >= 0, got {full_search_prob!r}')
+    if p >= 1.0:
+        return 0
+    batch = int(search_batch_size)
+    full = (int(simulations) // batch + 1) * batch
+    if fast_simulations is None or int(fast_simulations) < 0:
+        raise ValueError('full_search_prob < 1 needs fast_simulations >= 0')
+    fast = (int(fast_simulations) // batch + 1) * batch
+    if fast >= full:
+        raise ValueError(f'fast_simulations={fast_simulations} gives {fast} descents per move, '
+                         f'not fewer than the {full} of a full search')
+    return fast
+
+
 class StubEvaluator:
     """Deterministic device stub (test / bench aid; modes as in
     oracle/azalea_oracle.h): 0 uniform, 1 dyadic, 2 rough."""
@@ -69,7 +93,7 @@ class LockstepSelfPlay:
                  device=None, rank=0, world_size=1, nodes_per_game=None,
                  replay_rows=None, collect_replay=True, cuda_graph=True,
                  max_plies=300, random_play=False, streams=None, pack_leaves=None,
-                 random_reflect=False):
+                 random_reflect=False, full_search_prob=1.0, fast_simulations=None):
         # random_play: RandomPolicy self-play (random_policy.py:25-41) -- no
         # search, uniform move choice and uniform moves_prob at every ply;
         # how the reference fills the replay buffer before training
@@ -87,6 +111,11 @@ class LockstepSelfPlay:
         # mcts.py:268: num_batches = sims // batch + 1
         self.num_batches = int(simulations) // self.batch + 1
         self.sims_per_move = self.num_batches * self.batch
+        # playout cap randomization (Wu 2019): a ply is a full search with probability
+        # full_search_prob, otherwise a fast one of fast_descents new descents without root
+        # noise whose replay row is dropped (az_engine_set_playout_cap); 0 = off
+        self.fast_descents = 0 if self.random_play else playout_cap_descents(
+            full_search_prob, fast_simulations, simulations, self.batch)
         self.coef = float(exploration_coef)
         self.depth = int(exploration_depth)
         self.temperature = float(exploration_temperature)
@@ -123,6 +152,8 @@ class LockstepSelfPlay:
         self.random_reflect = bool(random_reflect) and not self.random_play
         if self.random_reflect:
             self.eng.set_reflect(True)
+        if self.fast_descents:
+            self.eng.set_playout_cap(full_search_prob, self.fast_descents)
         self.device = self.eng.device
         self.chosen = torch.zeros(self.G, 4, dtype=torch.int32,
                                   device=self.device)

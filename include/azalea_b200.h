@@ -109,7 +109,8 @@ enum {
                                (AZ_CFG_PACK_LEAVES: depth | row << 10) */
     AZ_BUF_VALUE = 2,       /* f32   [G][max_batch]           evaluator output */
     AZ_BUF_PRIOR = 3,       /* f32   [G][max_batch][n*n]      evaluator output (priors or logits) */
-    AZ_BUF_META = 4,        /* int32 [G][16] */
+    AZ_BUF_META = 4,        /* int32 [G][16]; [14] = descent count when this move's search
+                               began (az_engine_set_playout_cap) */
     AZ_BUF_REPLAY = 5,      /* uint8 [replay_rows][replay_row_bytes] */
     AZ_BUF_COUNTERS = 6,    /* int64 [G][16] per-game counters (sum over games on the host) */
     AZ_BUF_LEAF_MOVES = 7,  /* int32 [G][max_batch][n*n] network-view legal moves, 0-padded */
@@ -136,7 +137,9 @@ enum {
     AZ_CNT_NN_ROWS = 11,      /* non-terminal unique leaves (rows the network must evaluate) */
     AZ_CNT_POOL_SKIPPED = 12, /* expansions skipped because the pool half was full (AZ_CFG_SOFT_POOL_FULL) */
     AZ_CNT_TERMINAL_LEAVES = 13, /* unique leaves that were terminal positions (value -1, mcts.py:192-195) */
-    AZ_CNT_REFLECTED_ROWS = 14  /* network rows written rotated (az_engine_set_reflect) */
+    AZ_CNT_REFLECTED_ROWS = 14, /* network rows written rotated (az_engine_set_reflect) */
+    AZ_CNT_FAST_PLIES = 15      /* committed moves of fast plies (az_engine_set_playout_cap);
+                                   their rows are not flushed to the replay output */
 };
 
 typedef struct az_buffer_desc {
@@ -190,6 +193,26 @@ int az_engine_set_window(az_engine *e, int first_game, int num_games);
  * like the window (set it before capturing a graph).  Off: every buffer is
  * byte for byte what it is without this call. */
 int az_engine_set_reflect(az_engine *e, int on);
+
+/* Playout cap randomization (Wu 2019, "Accelerating Self-Play Learning in
+ * Go"), off by default.  At each ply every game draws one coin from its
+ * Philox key (counter: ply), so the draw does not depend on windows, streams
+ * or the world size; with probability full_search_prob the ply gets the full
+ * search.  Otherwise it is a fast ply: az_mcts_select stops searching the
+ * game once it has made fast_descents new descents in this move (counted from
+ * az_mcts_select_root, which every move must begin with; visits reused from
+ * the previous move do not count, and the check is made per launch, so
+ * fast_descents should be a multiple of the batch size), a capped game emits
+ * no leaves, and the root draws and mixes no Dirichlet noise.  az_play_commit
+ * picks the move by the same rule on both kinds of ply, counts fast plies in
+ * AZ_CNT_FAST_PLIES and flushes only the rows of full plies to the replay
+ * output (game_len and result are still the whole game's).  The start of the
+ * move's search is kept in meta slot 14.  full_search_prob >= 1 turns it off;
+ * AZ_E_INVALID for a negative or NaN probability, or for fast_descents < 1
+ * with the cap on.  Read at launch time like the window (set it before
+ * capturing a graph).  Off: every buffer is byte for byte what it is without
+ * this call. */
+int az_engine_set_playout_cap(az_engine *e, float full_search_prob, int fast_descents);
 
 /* HexGame.reset + Policy.reset for the games whose mask byte is non-zero
  * (NULL = all), hex.py:47-49, policy.py:72-76, search_tree.py:59-71. */
