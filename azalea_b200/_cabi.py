@@ -129,8 +129,6 @@ def lib():
     L.az_nn_resblock.argtypes = [vp, vp, f32p, vp, C.c_int, C.c_int64, vp]
     L.az_nn_resblocks.argtypes = [vp, vp, f32p, vp, C.c_int, C.c_int64, C.c_int, vp]
     L.az_nn_resblocks_live.argtypes = L.az_nn_resblocks.argtypes[:-1] + [i32p, vp]
-    L.az_nn_resblocks_heads_live.argtypes = [vp, vp, f32p, vp, C.c_int, C.c_int64, C.c_int, f32p,
-                                             vp, C.c_int64, i32p, vp]
     L.az_nn_resblock_scratch_bytes.restype = C.c_size_t
     L.az_noise_sample.argtypes = [eng, C.c_float, C.c_int, C.c_int, f32p, vp]
     L.az_play_commit.argtypes = [eng, C.POINTER(AzPlayParams), i32p, vp]

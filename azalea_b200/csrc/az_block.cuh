@@ -52,6 +52,20 @@
 //    stores) was bit-exact and took 0.92 ms per block; its direct, per-row global accesses in
 //    C's epilogue (32 different lines per warp instruction) alone cost 0.19 ms each way.
 //
+// Alternatives measured and removed (all bit-exact; where the numbers are):
+//  * y from P to C through an L2-resident scratch ring in global memory (P bulk-stores the
+//    staging tile, C bulk-loads it; the link carries only arrives): 8.96e6 against 9.22e6
+//    simulations/s in the step (profiles/r02_fused_block.txt)
+//  * y sent by P's epilogue with st.async, registers -> C's ring: 0.65 against 0.59 ms per block;
+//    4 x STAS.128 per thread and slab keep P's epilogue busy 2600 cycles per slab (same file)
+//  * C's epilogue reading the residual from and writing its output to global memory directly,
+//    whole lines per eight lanes with an 8 x 8 shuffle transpose on each side: 0.63 against
+//    0.57 ms per block, ~400 instructions per thread and slab for the transposes (same file)
+//  * two storer threads per CTA (even / odd slabs): the kernel is bound elsewhere when the MMAs
+//    run, and the extra warp costs 1 % (same file)
+//  * the two 1x1 head convolutions fused into C's epilogue of the last pass: 3.3 % slower in the
+//    step than the separate heads kernel (profiles/r02_fused_heads_ab.txt)
+//
 // Everything else -- slab layout, pointer-shift taps, dy stacking into a TMEM accumulator
 // ring, ping-pong MMA issuers, two epilogue groups -- is az_tower.cuh's; see there.
 //
@@ -79,28 +93,12 @@
 
 #include "az_tower.cuh"
 
-#ifndef AZB_STORERS
-#define AZB_STORERS 1       // storer threads per CTA; 2 (probe): warps 20 / 21 take the even / odd slabs
-#endif
-#define AZB_THREADS (AZB_STORERS == 2 ? 704 : 672)
-// How y travels from P to C (all three are bit-exact; sustained-bench A/B on one box,
-// profiles/r02_fused_block.txt):
-//   0  staging tile + shared-to-shared bulk copy over the SM-to-SM link          9.22e6 sims/s
-//   2  (probe) through a small L2-resident scratch ring in global memory: P bulk-stores the
-//      staging tile, C bulk-loads it; the link carries only mbarrier arrives      8.96e6
-//   1  (probe) P's epilogue sends it with st.async, registers -> C's ring: 4 x STAS.128 per
-//      thread and slab keep P's epilogue busy 2600 cycles per slab                (0.65 ms burst)
-#ifndef AZB_HANDOVER
-#define AZB_HANDOVER 0
-#endif
-#define AZB_P_ASYNC (AZB_HANDOVER == 1)
-#define AZB_VIA_L2 (AZB_HANDOVER == 2)
-#define AZB_R 8             // scratch slots per cluster (16 KB each)
+#define AZB_THREADS 672     // 21 warps, see Roles
 #ifndef AZB_SX
-#define AZB_SX (AZB_P_ASYNC ? 8 : 4)    // P: input ring stages (x chunks, bulk loads)
+#define AZB_SX 4            // P: input ring stages (x chunks, bulk loads)
 #endif
 #ifndef AZB_TP
-#define AZB_TP 4            // P: staging tiles (bulk-copy variant only)
+#define AZB_TP 4            // P: staging tiles
 #endif
 #ifndef AZB_SY
 #define AZB_SY 4            // C: input ring stages (y slabs copied in by P)
@@ -112,26 +110,10 @@
 #define AZB_TC 2            // C: staging tiles
 #endif
 #define AZB_TMAX (AZB_TP > AZB_TC ? AZB_TP : AZB_TC)
-// How C reads the residual and writes its output:
-//   0  bulk-loaded residual ring + staging tile + bulk store (64 KB of shared-memory traffic per slab
-//      on top of the 136 KB of MMA operands and incoming y)
-//   1  (probe) straight from / to global memory by the epilogue threads, whole 128-byte lines per
-//      eight lanes, with an 8 x 8 register transpose (shuffles) between "lane = chunk" and "lane =
-//      row".  Bit-exact, no shared memory in C but operands and bias -- and slower: 0.628 ms per
-//      block against 0.572 (0.610 with six input stages): the two transposes are ~400 instructions
-//      per thread and slab, a group of four warps needs ~6000 cycles per slab, and the block ring
-//      waits for it (profiles/r02_fused_block.txt)
-#ifndef AZB_CDIRECT
-#define AZB_CDIRECT 0
-#endif
-#ifndef AZB_PROF
-#define AZB_PROF 0          // 1: probe build with per-role cycle accounting (tools/probe/block_time.py)
-#endif
 #define AZB_SMAX (AZB_SX > AZB_SY ? AZB_SX : AZB_SY)
-#define AZB_SMEM_P (AZT_WBYTES + AZB_SX * AZT_CHUNK_BYTES + (AZB_P_ASYNC ? 0 : AZB_TP) * AZT_OUT_BYTES)
-#define AZB_SMEM_C (AZT_WBYTES + AZB_SY * AZT_CHUNK_BYTES + (AZB_CDIRECT ? 0 : AZB_SR + AZB_TC) * AZT_OUT_BYTES)
+#define AZB_SMEM_P (AZT_WBYTES + AZB_SX * AZT_CHUNK_BYTES + AZB_TP * AZT_OUT_BYTES)
+#define AZB_SMEM_C (AZT_WBYTES + AZB_SY * AZT_CHUNK_BYTES + (AZB_SR + AZB_TC) * AZT_OUT_BYTES)
 #define AZB_SMEM_BYTES (AZB_SMEM_P > AZB_SMEM_C ? AZB_SMEM_P : AZB_SMEM_C)
-static_assert(AZB_SY <= AZB_R, "bar_y_free is sized for the scratch ring");
 static_assert(AZB_SX <= 8 && AZB_SY <= 8, "stage reuse is tracked through the 8 MMA-retired barriers");
 // Every ring that the two epilogue groups of a CTA share has an EVEN number of entries, so an
 // entry always belongs to the same group (slab parity).  A parity wait then cannot be two
@@ -139,43 +121,10 @@ static_assert(AZB_SX <= 8 && AZB_SY <= 8, "stage reuse is tracked through the 8 
 // that completed late let the other group pass the wait of the NEXT use of the stage -- wrong
 // residuals, and with the arrival counts mixed up, a hang or a launch failure when two
 // instances ran concurrently on two streams (tools/soak.py --streams 2).
-static_assert(AZB_TC % 2 == 0 && AZB_SR % 2 == 0 && (AZB_P_ASYNC || AZB_TP % 2 == 0),
+static_assert(AZB_TC % 2 == 0 && AZB_SR % 2 == 0 && AZB_TP % 2 == 0,
               "rings shared by the two epilogue groups must have an even number of entries");
-static_assert(!AZB_P_ASYNC || AZB_SY % 2 == 0, "st.async variant: a stage of C's ring belongs to one epilogue group of P");
 
 #define AZB_MAXPASS 8       // residual blocks one launch can chain (their biases sit in shared memory)
-
-// FUSED HEADS (az_nn_resblocks_heads_live): the network's two 1x1 head convolutions (+ BN + ReLU;
-// 64 -> 2 + 4 channels, network.py:75-76,82-83) read the tower's output and nothing else does,
-// so C's epilogue of the LAST pass computes them from the rows it has just rounded to bf16:
-// thread = row holds 32 of the 64 channels, 6 x 32 FMAs against weights in CONSTANT memory (an
-// operand fetch through the constant cache: the shared-memory port, which bounds this kernel,
-// is not touched), the two halves of a row meet through 3 KB of shared memory, and the six bf16
-// head activations of the cell go straight into the [board][n*n*6 (+ pad)] rows the merged FC
-// GEMM reads.  Saves the separate heads launch and its pass over the activations.
-#define AZB_HEADS 6
-#define AZB_HEAD_FLOATS (AZB_HEADS * AZT_C + 8)     // [6][64] weights, then 6 biases
-// ONE weight set at a fixed address, so that every weight is an immediate constant-bank operand of
-// its FMA (a register-indexed LDC per weight made the last pass 65 % slower).  The launcher copies the
-// caller's weights here in stream order before every launch: launches on one stream may alternate
-// networks; launches that run CONCURRENTLY on several streams must use the same network (the two
-// windows of LockstepSelfPlay do).
-__constant__ float azb_heads_c[AZB_HEAD_FLOATS];
-
-// channels HALF * 32 + CHUNK * 8 .. + 8 of a row (bf16 pairs in ow) against the six head filters
-template <int HALF, int CHUNK>
-__device__ __forceinline__ void azb_heads_acc(const uint32_t (&ow)[4], float (&hacc)[AZB_HEADS])
-{
-#pragma unroll
-    for (int q = 0; q < 4; q++) {
-        const float a0 = __uint_as_float(ow[q] << 16), a1 = __uint_as_float(ow[q] & 0xffff0000u);
-        constexpr int c0 = HALF * 32 + CHUNK * 8;
-#pragma unroll
-        for (int hh = 0; hh < AZB_HEADS; hh++)
-            hacc[hh] = __fmaf_rn(a1, azb_heads_c[hh * AZT_C + c0 + 2 * q + 1],
-                                 __fmaf_rn(a0, azb_heads_c[hh * AZT_C + c0 + 2 * q], hacc[hh]));
-    }
-}
 
 struct azb_params {
     uint8_t *x;             // activations, slab layout, pre-swizzled; updated in place
@@ -185,14 +134,7 @@ struct azb_params {
     int bpg;                // boards per group = 128 / (n+1)
     long long groups;       // board groups
     int passes;             // residual blocks to apply, one after the other (1 .. AZB_MAXPASS)
-    uint8_t *scratch;       // AZB_VIA_L2: [clusters][AZB_R][16 KB] hand-over ring in global memory
-    unsigned long long *prof;   // probe only: per-role wait cycles of cluster 0 ([rank][32]) or NULL
-    uint16_t *heads_out;    // fused heads: bf16 [boards][heads_stride] (6 per cell, cell-major), or NULL
-    long long heads_stride; // elements between two boards' rows
-    long long heads_boards; // rows of heads_out
     const int *live;        // packed leaves: device count of boards that are live in this batch (or NULL: all)
-    int debug;              // probe only (tools/probe/block_time.py): 2 = C skips its global stores,
-                            // 4 = C skips the residual loads, 8 = no MMAs
 };
 
 __device__ __forceinline__ uint32_t azb_cluster_rank()
@@ -231,14 +173,6 @@ __device__ __forceinline__ void azb_bulk_s2s(uint32_t dst_cluster, const void *s
         ::"r"(dst_cluster), "r"(azt_smem(src)), "r"(bytes), "r"(bar_cluster) : "memory");
 }
 
-// 16 bytes from registers into the other CTA's shared memory, asynchronously; the bytes are
-// counted (complete_tx) on a barrier of the destination CTA, so the sender needs no fence
-__device__ __forceinline__ void azb_st_async(uint32_t dst_cluster, const uint4 &v, uint32_t bar_cluster)
-{
-    asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.v4.b32 [%0], {%1, %2, %3, %4}, [%5];"
-                 ::"r"(dst_cluster), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w), "r"(bar_cluster) : "memory");
-}
-
 // Wait on an own barrier whose phase is completed from the other CTA (a relaxed remote arrive,
 // or the bytes of its bulk copy).  The plain CTA-scope wait is enough: these barriers carry
 // flow control only -- what they guard was read or written by the tensor core or the copy
@@ -261,61 +195,6 @@ __device__ __forceinline__ void azb_wait_stored(const volatile uint32_t *cnt, ui
 {
     while (*cnt < need) asm volatile("nanosleep.u32 64;");
 }
-
-// one 32-byte sector of a row: 16-byte chunks lo | hi
-__device__ __forceinline__ void azb_stg_sector(void *p, const uint4 &lo, const uint4 &hi)
-{
-    asm volatile("st.global.v4.b64 [%0], {%1, %2, %3, %4};"
-                 ::"l"(p), "l"((unsigned long long)lo.x | ((unsigned long long)lo.y << 32)),
-                   "l"((unsigned long long)lo.z | ((unsigned long long)lo.w << 32)),
-                   "l"((unsigned long long)hi.x | ((unsigned long long)hi.y << 32)),
-                   "l"((unsigned long long)hi.z | ((unsigned long long)hi.w << 32)) : "memory");
-}
-
-__device__ __forceinline__ uint4 azb_ldg16(const void *p)
-{
-    uint4 v;
-    asm volatile("ld.global.cg.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p) : "memory");
-    return v;
-}
-
-__device__ __forceinline__ void azb_stg16(void *p, const uint4 &v)
-{
-    asm volatile("st.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(p), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-
-// 8 x 8 transpose of 16-byte elements over the eight lanes of a lane group: element r[i] of lane
-// s (s = lane & 7) <-> element r[s] of lane i.  Three butterfly stages; its own inverse.
-template <int BIT>
-__device__ __forceinline__ void azb_transpose_stage(uint4 (&r)[8], const bool up)
-{
-#pragma unroll
-    for (int i = 0; i < 8; i++) {
-        if (i & BIT) continue;
-        const uint4 a = r[i], b = r[i | BIT];
-        uint4 snd = up ? a : b, rcv;
-        rcv.x = __shfl_xor_sync(0xffffffffu, snd.x, BIT);
-        rcv.y = __shfl_xor_sync(0xffffffffu, snd.y, BIT);
-        rcv.z = __shfl_xor_sync(0xffffffffu, snd.z, BIT);
-        rcv.w = __shfl_xor_sync(0xffffffffu, snd.w, BIT);
-        r[i] = up ? rcv : a;
-        r[i | BIT] = up ? b : rcv;
-    }
-}
-
-__device__ __forceinline__ void azb_transpose8(uint4 (&r)[8], const int lane)
-{
-    azb_transpose_stage<1>(r, (lane & 1) != 0);
-    azb_transpose_stage<2>(r, (lane & 2) != 0);
-    azb_transpose_stage<4>(r, (lane & 4) != 0);
-}
-
-// probe: accumulate the cycles spent in `stmt` into slot k of this CTA's profile row
-#define AZB_TIMED(k, stmt)                                                          \
-    do {                                                                            \
-        if (prof_on) { const long long t0_ = clock64(); stmt; prof_acc[k] += clock64() - t0_; } \
-        else { stmt; }                                                              \
-    } while (0)
 
 // A role's position in the chained sequence of slabs: t = pass * nslabs + j runs over all the
 // passes (rings, barrier phases and the TMEM ring continue across a pass boundary; nslabs is a
@@ -345,25 +224,12 @@ k_resblock(const azb_params p)
     __shared__ uint64_t bar_res_full[AZB_SR], bar_res_empty[AZB_SR];        // C: residual ring
     __shared__ uint64_t bar_mma_done[8];            // MMA(t) retired, by t & 7
     __shared__ uint64_t bar_blk_free[AZT_BLOCKS];   // ring block read, zeroed and free for its next output slab
-    __shared__ uint64_t bar_y_free[AZB_R];          // P: stage of C's ring / scratch slot consumed (arrived by C)
-    __shared__ uint64_t bar_y_ready[AZB_R];         // C (AZB_VIA_L2): scratch slot written (arrived by P)
+    __shared__ uint64_t bar_y_free[AZB_SY];         // P: stage of C's ring consumed (arrived by C)
     __shared__ uint32_t tmem_holder;
     __shared__ volatile uint32_t s_stored;          // output slabs (index t) whose store has completed
     __shared__ __align__(16) float s_bias[AZB_MAXPASS * AZT_C];     // this CTA's layer of every pass
-    __shared__ float s_hx[2][2][AZB_HEADS * 128];   // fused heads: partial sums of channels 0..31, [group][slab parity]
 
     const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-    const bool prof_on = AZB_PROF && p.prof != nullptr && (blockIdx.x >> 1) == 0 && lane == 0;
-    long long prof_acc[6] = {0, 0, 0, 0, 0, 0};
-    const long long prof_t0 = clock64();
-    // probe (debug & 16, tools/probe/cluster_times.py): when each CTA started and ended, and where
-    if ((p.debug & 16) && p.prof != nullptr && tid == 0) {
-        unsigned long long gt; uint32_t smid;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-        asm volatile("mov.u32 %0, %%smid;" : "=r"(smid));
-        p.prof[128 + 4 * blockIdx.x] = gt;
-        p.prof[128 + 4 * blockIdx.x + 2] = smid;
-    }
     if (tid == 0) {
         azt_mbar_init(&bar_w, 1);
         for (int i = 0; i < AZB_SMAX; i++) azt_mbar_init(&bar_in_full[i], 1);   // one bulk transfer per stage
@@ -377,12 +243,12 @@ k_resblock(const azb_params p)
         }
         for (int i = 0; i < 8; i++) azt_mbar_init(&bar_mma_done[i], 1);
         // one arrival per warp of the group that drained the block
-        for (int i = 0; i < AZT_BLOCKS; i++) azt_mbar_init(&bar_blk_free[i], AZB_CDIRECT && !isP ? 4 : 8);
-        for (int i = 0; i < AZB_R; i++) { azt_mbar_init(&bar_y_free[i], 1); azt_mbar_init(&bar_y_ready[i], 1); }
+        for (int i = 0; i < AZT_BLOCKS; i++) azt_mbar_init(&bar_blk_free[i], 8);
+        for (int i = 0; i < AZB_SY; i++) azt_mbar_init(&bar_y_free[i], 1);
         s_stored = 0;
         asm volatile("fence.mbarrier_init.release.cluster;");
         // C arms every stage of its input ring for the first slab P will copy into it
-        if (!isP && !AZB_VIA_L2)
+        if (!isP)
             for (int i = 0; i < AZB_SY; i++) azt_mbar_expect_tx(&bar_in_full[i], AZT_OUT_BYTES);
     }
     for (int i = tid; i < p.passes * AZT_C; i += AZB_THREADS)
@@ -435,55 +301,35 @@ k_resblock(const azb_params p)
     if (NT == 0) {
         // packed leaves: fewer live groups than clusters -- this one has nothing to do (both of its
         // CTAs agree); it still takes part in the two cluster barriers and frees its TMEM
-    } else if (warp >= 20) {
-        // ----------------------------------------------------------- storers --
+    } else if (warp == 20) {
+        // ------------------------------------------------------------ storer --
         // A bulk store takes ~1000 cycles to read its 16 KB tile, and bulk groups are per
         // thread: one storer thread that waits for each store's read before it hands the tile
         // back caps the pipeline AROUND the MMAs at ~1200 cycles per slab (measured with the MMAs
-        // switched off); two threads (AZB_STORERS 2: even / odd slabs) lift that to ~1000, but
-        // with the MMAs running the kernel is bound elsewhere and the extra warp costs 1 %.
-        const int sw_ = warp - 20;          // AZB_STORERS == 1: warp 20 takes every slab
-        if (isP && lane == 0 && AZB_VIA_L2) {
-            // P: finished y slab: staging tile -> slot t % AZB_R of the cluster's scratch ring
-            uint8_t *ring = p.scratch + (size_t)cid * AZB_R * AZT_OUT_BYTES;
-            for (int t = sw_; t < NT; t += AZB_STORERS) {
-                const int sb = t % AZB_TP, ss = t % AZB_R;
-                AZB_TIMED(0, azt_mbar_wait(&bar_out_done[sb], (t / AZB_TP) & 1));
-                if (t >= AZB_R) AZB_TIMED(1, azb_wait_cluster(&bar_y_free[ss], ((t / AZB_R) & 1) ^ 1));
-                azt_bulk_s2g(ring + (size_t)ss * AZT_OUT_BYTES, s_out + sb * AZT_OUT_BYTES, AZT_OUT_BYTES);
-                asm volatile("cp.async.bulk.commit_group;" ::: "memory");
-                // the tile is free as soon as the store has READ it ...
-                asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
-                azt_mbar_arrive(&bar_out_empty[sb]);
-                // ... and C may load the slab once the store has COMPLETED
-                asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");
-                azb_remote_arrive(azb_remote(&bar_y_ready[ss], 1));
-            }
-        } else if (isP && lane == 0 && !AZB_P_ASYNC && sw_ == 0) {
+        // switched off); with the MMAs running the kernel is bound elsewhere.
+        if (isP && lane == 0) {
             // P: finished y slab: staging tile -> rows 8..135 of stage st of C's input ring
             for (int t = 0; t < NT; t++) {
                 const int sb = t % AZB_TP, st = t % AZB_SY;
-                AZB_TIMED(0, azt_mbar_wait(&bar_out_done[sb], (t / AZB_TP) & 1));
-                if (t >= AZB_SY) AZB_TIMED(1, azb_wait_cluster(&bar_y_free[st], ((t / AZB_SY) & 1) ^ 1));
+                azt_mbar_wait(&bar_out_done[sb], (t / AZB_TP) & 1);
+                if (t >= AZB_SY) azb_wait_cluster(&bar_y_free[st], ((t / AZB_SY) & 1) ^ 1);
                 azb_bulk_s2s(azb_remote(s_in + st * AZT_CHUNK_BYTES + 8 * AZT_ROW, 1),
                              s_out + sb * AZT_OUT_BYTES, AZT_OUT_BYTES, azb_remote(&bar_in_full[st], 1));
             }
-        } else if (!isP && lane == 0 && !AZB_CDIRECT) {
+        } else if (lane == 0) {
             // C: finished output slab -> global memory, in place
-            azb_pos at = {sw_, sw_, 0};
-            at.advance(0, nslabs);
-            for (; at.t < NT; at.advance(AZB_STORERS, nslabs)) {
+            azb_pos at = {0, 0, 0};
+            for (; at.t < NT; at.advance(1, nslabs)) {
                 const int sb = at.t % AZB_TC;
-                AZB_TIMED(0, azt_mbar_wait(&bar_out_done[sb], (at.t / AZB_TC) & 1));
-                if (!(p.debug & 2))
-                    azt_bulk_s2g(p.x + (size_t)(AZT_HALO + (q0 + at.j) * 128) * AZT_ROW, s_out + sb * AZT_OUT_BYTES,
-                                 AZT_OUT_BYTES);
+                azt_mbar_wait(&bar_out_done[sb], (at.t / AZB_TC) & 1);
+                azt_bulk_s2g(p.x + (size_t)(AZT_HALO + (q0 + at.j) * 128) * AZT_ROW, s_out + sb * AZT_OUT_BYTES,
+                             AZT_OUT_BYTES);
                 asm volatile("cp.async.bulk.commit_group;" ::: "memory");
                 // hand the tile back as soon as the store has READ it (the write to global
                 // memory goes on): each epilogue group has one tile
                 asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
                 azt_mbar_arrive(&bar_out_empty[sb]);
-                if (p.passes > 1 && AZB_STORERS == 1) {
+                if (p.passes > 1) {
                     // chained blocks: the next pass loads these slabs again (P as its input, C as
                     // its residual) once their stores have COMPLETED.  All stores but this one
                     // have (the last slab of a pass: this one too); say so in both CTAs.
@@ -513,36 +359,17 @@ k_resblock(const azb_params p)
                 for (int tp = 0; tp < 9; tp++)
                     azt_bulk_g2s(s_w + tp * 8192, w + (size_t)(pass * 2) * AZT_WBYTES + tp * 8192, 8192, &bar_w);
             }
-        } else if (!isP && lane == 0 && AZB_VIA_L2) {
-            // C: y loader: scratch slot -> rows 8..135 of stage st of the input ring (an L2 hit), and,
-            // two slabs later, the slot back to P
-            const uint8_t *ring = p.scratch + (size_t)cid * AZB_R * AZT_OUT_BYTES;
-            for (int t = 0; t < NT + 2; t++) {
-                if (t < NT) {
-                    const int ss = t % AZB_R, st = t % AZB_SY;
-                    AZB_TIMED(0, azb_wait_cluster(&bar_y_ready[ss], (t / AZB_R) & 1));
-                    if (t >= AZB_SY) AZB_TIMED(1, azt_mbar_wait(&bar_mma_done[(t - AZB_SY) & 7], ((t - AZB_SY) >> 3) & 1));
-                    azt_mbar_expect_tx(&bar_in_full[st], AZT_OUT_BYTES);
-                    azt_bulk_g2s(s_in + st * AZT_CHUNK_BYTES + 8 * AZT_ROW, ring + (size_t)ss * AZT_OUT_BYTES,
-                                 AZT_OUT_BYTES, &bar_in_full[st]);
-                }
-                if (t >= 2 && t - 2 + AZB_R < NT) {
-                    const int k = t - 2;
-                    azt_mbar_wait(&bar_in_full[k % AZB_SY], (k / AZB_SY) & 1);
-                    azb_remote_arrive(azb_remote(&bar_y_free[k % AZB_R], 0));
-                }
-            }
         } else if (!isP && lane == 0) {
             for (int t = 0; t <= NT; t++) {
-                if (t < NT && !AZB_P_ASYNC) {
+                if (t < NT) {
                     // slab t has landed in C: P's staging tile that held it may be rewritten
-                    AZB_TIMED(0, azb_wait_cluster(&bar_in_full[t % AZB_SY], (t / AZB_SY) & 1));
+                    azb_wait_cluster(&bar_in_full[t % AZB_SY], (t / AZB_SY) & 1);
                     azb_remote_arrive(azb_remote(&bar_out_empty[t % AZB_TP], 0));
                 }
                 if (t >= 1 && t - 1 + AZB_SY < NT) {
                     // MMA2(t-1) has read its stage: arm it for its next slab, then let P copy that in
                     const int k = t - 1;
-                    AZB_TIMED(1, azt_mbar_wait(&bar_mma_done[k & 7], (k >> 3) & 1));
+                    azt_mbar_wait(&bar_mma_done[k & 7], (k >> 3) & 1);
                     azt_mbar_expect_tx(&bar_in_full[k % AZB_SY], AZT_OUT_BYTES);
                     azb_remote_arrive(azb_remote(&bar_y_free[k % AZB_SY], 0));
                 }
@@ -555,9 +382,9 @@ k_resblock(const azb_params p)
             for (; at.t < NT; at.advance(1, nslabs)) {
                 const int st = at.t % AZB_SX;
                 // the stage is free once the MMAs of the slab that used it last have retired
-                if (at.t >= AZB_SX) AZB_TIMED(0, azt_mbar_wait(&bar_mma_done[(at.t - AZB_SX) & 7], ((at.t - AZB_SX) >> 3) & 1));
+                if (at.t >= AZB_SX) azt_mbar_wait(&bar_mma_done[(at.t - AZB_SX) & 7], ((at.t - AZB_SX) >> 3) & 1);
                 // chained blocks: the slab is the previous pass's output
-                if (at.pass > 0) AZB_TIMED(1, azb_wait_stored(&s_stored, (uint32_t)(at.t - nslabs) + 1u));
+                if (at.pass > 0) azb_wait_stored(&s_stored, (uint32_t)(at.t - nslabs) + 1u);
                 // slab rows plus 8 rows on each side: global rows [128 q, 128 q + 144)
                 azt_mbar_expect_tx(&bar_in_full[st], AZT_CHUNK_BYTES);
                 azt_bulk_g2s(s_in + st * AZT_CHUNK_BYTES, p.x + (size_t)((q0 + at.j) * 128) * AZT_ROW,
@@ -565,17 +392,15 @@ k_resblock(const azb_params p)
             }
         } else if (lane == 0) {
             // C: the residual: the block's own input slab, again (L2: P has just read it)
-            if (!(p.debug & 4) && !AZB_CDIRECT) {
-                azb_pos at = {0, 0, 0};
-                for (; at.t < NT; at.advance(1, nslabs)) {
-                    const int sr = at.t % AZB_SR;
-                    AZB_TIMED(0, azt_mbar_wait(&bar_res_empty[sr], ((at.t / AZB_SR) & 1) ^ 1));
-                    // chained blocks: the slab is this CTA's own output of the previous pass
-                    if (at.pass > 0) azb_wait_stored(&s_stored, (uint32_t)(at.t - nslabs) + 1u);
-                    azt_mbar_expect_tx(&bar_res_full[sr], AZT_OUT_BYTES);
-                    azt_bulk_g2s(s_res + sr * AZT_OUT_BYTES, p.x + (size_t)(AZT_HALO + (q0 + at.j) * 128) * AZT_ROW,
-                                 AZT_OUT_BYTES, &bar_res_full[sr]);
-                }
+            azb_pos at = {0, 0, 0};
+            for (; at.t < NT; at.advance(1, nslabs)) {
+                const int sr = at.t % AZB_SR;
+                azt_mbar_wait(&bar_res_empty[sr], ((at.t / AZB_SR) & 1) ^ 1);
+                // chained blocks: the slab is this CTA's own output of the previous pass
+                if (at.pass > 0) azb_wait_stored(&s_stored, (uint32_t)(at.t - nslabs) + 1u);
+                azt_mbar_expect_tx(&bar_res_full[sr], AZT_OUT_BYTES);
+                azt_bulk_g2s(s_res + sr * AZT_OUT_BYTES, p.x + (size_t)(AZT_HALO + (q0 + at.j) * 128) * AZT_ROW,
+                             AZT_OUT_BYTES, &bar_res_full[sr]);
             }
         }
     } else if (warp >= 16) {
@@ -595,14 +420,12 @@ k_resblock(const azb_params p)
             const int top = t + 1 - dy0;
             // highest output slab entered by the slabs before this one
             const int entered = t == 0 ? -1 : (y == 0 ? t - 1 : t);
-            AZB_TIMED(0, azb_wait_cluster(&bar_in_full[st], (t / S) & 1));
+            azb_wait_cluster(&bar_in_full[st], (t / S) & 1);
             // this pass's weights (the other warp's MMAs of the last pass retire before they are replaced)
             while (wpass < at.pass) { wpass++; azt_mbar_wait(&bar_w, wpass & 1); }
-            // st.async variant: the slab was not written by the async proxy the tensor core reads through
-            if (AZB_P_ASYNC && !isP) asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
             // a block entered for a new output slab u: its previous tenant u-8 must have been retired
             for (int u = entered + 1; u <= top; u++)
-                if (u >= 8) AZB_TIMED(2, azt_mbar_wait(&bar_blk_free[AZB_RING(u)], ((u >> 3) - 1) & 1));
+                if (u >= 8) azt_mbar_wait(&bar_blk_free[AZB_RING(u)], ((u >> 3) - 1) & 1);
             const int blk = AZB_RING(top), nb = dy1 - dy0 + 1;
             const int first = nb < 8 - blk ? nb : 8 - blk, second = nb - first;     // split where the ring wraps
             const uint32_t d0 = tmem + blk * 64, i0 = AZT_IDESC(first), i1 = AZT_IDESC(second);
@@ -611,15 +434,11 @@ k_resblock(const azb_params p)
             const uint64_t db0 = db_base + (uint64_t)(dy0 * 64 * (AZT_ROW / 16));
             const uint64_t db1 = db0 + (uint64_t)(first * 64 * (AZT_ROW / 16));
             // take the turn: the other warp has issued slab t-1
-            const long long tt_ = prof_on ? clock64() : 0;
             if (w == 0) asm volatile("bar.sync 3, 64;" ::: "memory");
             else asm volatile("bar.sync 4, 64;" ::: "memory");
             asm volatile("tcgen05.fence::after_thread_sync;");
-            const long long ti_ = prof_on ? clock64() : 0;
-            if (prof_on) prof_acc[3] += ti_ - tt_;
             if (azt_elect()) {
-                if (p.debug & 8) {
-                } else if (second == 0) {
+                if (second == 0) {
 #pragma unroll
                     for (int dx = 0; dx < 3; dx++)
 #pragma unroll
@@ -648,77 +467,6 @@ k_resblock(const azb_params p)
                 if (w == 0) asm volatile("bar.arrive 4, 64;" ::: "memory");
                 else asm volatile("bar.arrive 3, 64;" ::: "memory");
             }
-            if (prof_on) prof_acc[4] += clock64() - ti_;
-        }
-    } else if (AZB_CDIRECT && !isP) {
-        // ------------------------------------------- epilogue of C, direct --
-        // (probe, single pass only.)  Four groups of four warps on output slabs t = group (mod 4); a
-        // warp owns ALL 64 channels of the 32 rows of its TMEM lane quadrant: thread = TMEM lane = row
-        // l.  The residual comes from and the result goes to global memory as whole lines: in access
-        // i of 8 the eight lanes of lane group G cover the 128 bytes of row 8 G + i (lane k the chunk
-        // at position k ^ i, which is LOGICAL chunk k of that row: the swizzle is in the address), and
-        // a register transpose turns "lane k holds chunk k of rows 8 G + 0..7" into "lane k holds
-        // chunks 0..7 of row 8 G + k" and back.  No shared memory but the bias.
-        const int grp = warp >> 2, wq = warp & 3;
-        const int l = wq * 32 + lane, G = lane >> 3, k = lane & 7;
-        const bool real = l < p.bpg * (n + 1) && (l % (n + 1)) != n;    // not a pad cell
-        const uint32_t keep = real ? 0xffffffffu : 0u;
-        for (int j = grp, y = grp % n; j < nslabs; j += 4, y = (y + 4) % n) {
-            uint8_t *rows8 = p.x + (size_t)(AZT_HALO + (q0 + j) * 128 + wq * 32 + 8 * G) * AZT_ROW;
-            uint4 R[8];
-            if (!(p.debug & 4)) {
-#pragma unroll
-                for (int i = 0; i < 8; i++) R[i] = azb_ldg16(rows8 + i * AZT_ROW + ((k ^ i) << 4));
-            } else {
-#pragma unroll
-                for (int i = 0; i < 8; i++) R[i] = make_uint4(0u, 0u, 0u, 0u);
-            }
-            // output slab j is complete once MMA(j+1) retired (MMA(j) for the last board row)
-            const int last = y + 1 < n ? j + 1 : j;
-            AZB_TIMED(1, azt_mbar_wait(&bar_mma_done[last & 7], (last >> 3) & 1));
-            asm volatile("tcgen05.fence::after_thread_sync;");
-            const long long tb_ = prof_on ? clock64() : 0;
-            azb_transpose8(R, lane);                    // -> R[c] = logical chunk c of this thread's row
-            const int blk = AZB_RING(j);
-            const uint32_t ta = tmem + ((uint32_t)(wq * 32) << 16) + (uint32_t)blk * 64u;
-#pragma unroll
-            for (int h = 0; h < 4; h++) {
-                uint32_t acc[16];
-                AZT_TMEM_LD16(acc, ta + h * 16);
-                asm volatile("tcgen05.wait::ld.sync.aligned;");
-                azt_tmem_zero16(ta + h * 16);       // retire: zero for the block's next output slab
-#pragma unroll
-                for (int g = 0; g < 2; g++) {
-                    const int c8 = h * 2 + g;                       // 8-channel chunk of the row
-                    const float4 b0 = *reinterpret_cast<const float4 *>(&s_bias[c8 * 8]);
-                    const float4 b1 = *reinterpret_cast<const float4 *>(&s_bias[c8 * 8 + 4]);
-                    float f[8];
-                    f[0] = __uint_as_float(acc[g * 8 + 0]) + b0.x; f[1] = __uint_as_float(acc[g * 8 + 1]) + b0.y;
-                    f[2] = __uint_as_float(acc[g * 8 + 2]) + b0.z; f[3] = __uint_as_float(acc[g * 8 + 3]) + b0.w;
-                    f[4] = __uint_as_float(acc[g * 8 + 4]) + b1.x; f[5] = __uint_as_float(acc[g * 8 + 5]) + b1.y;
-                    f[6] = __uint_as_float(acc[g * 8 + 6]) + b1.z; f[7] = __uint_as_float(acc[g * 8 + 7]) + b1.w;
-                    const uint32_t rw[4] = {R[c8].x, R[c8].y, R[c8].z, R[c8].w};
-                    uint32_t ow[4];
-#pragma unroll
-                    for (int q = 0; q < 4; q++) {
-                        f[2 * q] += __uint_as_float(rw[q] << 16);
-                        f[2 * q + 1] += __uint_as_float(rw[q] & 0xffff0000u);
-                        ow[q] = azt_relu_bf16x2(f[2 * q], f[2 * q + 1]) & keep;
-                    }
-                    R[c8] = make_uint4(ow[0], ow[1], ow[2], ow[3]);
-                }
-            }
-            // hand the ring block back
-            asm volatile("tcgen05.wait::st.sync.aligned;");
-            asm volatile("tcgen05.fence::before_thread_sync;");
-            __syncwarp();
-            if (lane == 0) azt_mbar_arrive(&bar_blk_free[blk]);
-            azb_transpose8(R, lane);                    // -> R[i] = logical chunk k of row 8 G + i
-            if (!(p.debug & 2)) {
-#pragma unroll
-                for (int i = 0; i < 8; i++) azb_stg16(rows8 + i * AZT_ROW + ((k ^ i) << 4), R[i]);
-            }
-            if (prof_on) prof_acc[3] += clock64() - tb_;
         }
     } else {
         // ----------------------------------------------------- epilogue --
@@ -730,21 +478,17 @@ k_resblock(const azb_params p)
         const bool real = l < p.bpg * (n + 1) && (l % (n + 1)) != n;    // not a pad cell
         const uint32_t keep = real ? 0xffffffffu : 0u;
         const int sw = l & 7;                                       // == R & 7 (8 + 128 q + l)
-        const bool do_heads = !isP && p.heads_out != nullptr;
-        const int hbl = l / (n + 1), hbx = l - hbl * (n + 1);       // this row's board of the group and column
         azb_pos at = {grp, grp, 0};
         at.advance(0, nslabs);
         for (int y = grp % n; at.t < NT; at.advance(2, nslabs), y = (y + 2) % n) {
             const int t = at.t, sb = t % T;
             const float *bias = s_bias + at.pass * AZT_C;
-            const bool hpass = do_heads && at.pass == p.passes - 1;
-            float hacc[AZB_HEADS] = {0.f, 0.f, 0.f, 0.f, 0.f, 0.f};
             uint4 *srow = reinterpret_cast<uint4 *>(s_out + sb * AZT_OUT_BYTES + l * AZT_ROW);
             uint4 rv[4];
-            if (!isP && !(p.debug & 4)) {
+            if (!isP) {
                 // this thread's row and channels of the residual slab, from the bulk-loaded ring
                 const int sr = t % AZB_SR;
-                AZB_TIMED(2, azt_mbar_wait(&bar_res_full[sr], (t / AZB_SR) & 1));
+                azt_mbar_wait(&bar_res_full[sr], (t / AZB_SR) & 1);
                 const uint4 *rrow = reinterpret_cast<const uint4 *>(s_res + sr * AZT_OUT_BYTES + l * AZT_ROW);
 #pragma unroll
                 for (int c = 0; c < 4; c++) rv[c] = rrow[(half * 4 + c) ^ sw];
@@ -761,23 +505,12 @@ k_resblock(const azb_params p)
                 __syncwarp();
                 if (lane == 0) azt_mbar_arrive(&bar_res_empty[sr]);
             }
-            uint32_t ybase = 0, ybar = 0;
-            if (AZB_P_ASYNC && isP) {
-                // row 8 + l of stage st of C's ring, once MMA2 has retired the slab that was there
-                const int st = t % AZB_SY;
-                if (lane == 0) AZB_TIMED(0, azb_wait_cluster(&bar_y_free[st], ((t / AZB_SY) & 1) ^ 1));
-                __syncwarp();
-                ybase = azb_remote(s_in + st * AZT_CHUNK_BYTES + (8 + l) * AZT_ROW, 1);
-                ybar = azb_remote(&bar_in_full[st], 1);
-            } else {
-                // the staging tile must have been drained by the copy / store that used it last
-                AZB_TIMED(0, azb_wait_cluster(&bar_out_empty[sb], ((t / T) & 1) ^ 1));
-            }
+            // the staging tile must have been drained by the copy / store that used it last
+            azb_wait_cluster(&bar_out_empty[sb], ((t / T) & 1) ^ 1);
             // output slab t is complete once MMA(t+1) retired (MMA(t) for the last board row)
             const int last = y + 1 < n ? t + 1 : t;
-            AZB_TIMED(1, azt_mbar_wait(&bar_mma_done[last & 7], (last >> 3) & 1));
+            azt_mbar_wait(&bar_mma_done[last & 7], (last >> 3) & 1);
             asm volatile("tcgen05.fence::after_thread_sync;");
-            const long long tb_ = prof_on ? clock64() : 0;
             const int blk = AZB_RING(t);
             const uint32_t ta = tmem + ((uint32_t)(wq * 32) << 16) + (uint32_t)blk * 64u + (uint32_t)half * 32u;
 #pragma unroll
@@ -786,7 +519,6 @@ k_resblock(const azb_params p)
                 AZT_TMEM_LD16(acc, ta + h * 16);
                 asm volatile("tcgen05.wait::ld.sync.aligned;");
                 azt_tmem_zero16(ta + h * 16);       // retire: zero for the block's next output slab
-                uint4 o[2];  // (two chunks of this pass)
 #pragma unroll
                 for (int g = 0; g < 2; g++) {
                     const int c8 = half * 4 + h * 2 + g;            // 8-channel chunk of the row
@@ -797,7 +529,7 @@ k_resblock(const azb_params p)
                     f[2] = __uint_as_float(acc[g * 8 + 2]) + b0.z; f[3] = __uint_as_float(acc[g * 8 + 3]) + b0.w;
                     f[4] = __uint_as_float(acc[g * 8 + 4]) + b1.x; f[5] = __uint_as_float(acc[g * 8 + 5]) + b1.y;
                     f[6] = __uint_as_float(acc[g * 8 + 6]) + b1.z; f[7] = __uint_as_float(acc[g * 8 + 7]) + b1.w;
-                    if (!isP && !(p.debug & 4)) {
+                    if (!isP) {
                         const uint4 r = rv[h * 2 + g];
                         const uint32_t rw[4] = {r.x, r.y, r.z, r.w};
 #pragma unroll
@@ -811,24 +543,8 @@ k_resblock(const azb_params p)
                     for (int q = 0; q < 4; q++) {
                         ow[q] = azt_relu_bf16x2(f[2 * q], f[2 * q + 1]) & keep;
                     }
-                    o[g] = make_uint4(ow[0], ow[1], ow[2], ow[3]);
-                    if (hpass) {
-                        // the head convolutions see the bf16 activations the tower stores
-                        if (half == 0) {
-                            if (h == 0 && g == 0) azb_heads_acc<0, 0>(ow, hacc);
-                            if (h == 0 && g == 1) azb_heads_acc<0, 1>(ow, hacc);
-                            if (h == 1 && g == 0) azb_heads_acc<0, 2>(ow, hacc);
-                            if (h == 1 && g == 1) azb_heads_acc<0, 3>(ow, hacc);
-                        } else {
-                            if (h == 0 && g == 0) azb_heads_acc<1, 0>(ow, hacc);
-                            if (h == 0 && g == 1) azb_heads_acc<1, 1>(ow, hacc);
-                            if (h == 1 && g == 0) azb_heads_acc<1, 2>(ow, hacc);
-                            if (h == 1 && g == 1) azb_heads_acc<1, 3>(ow, hacc);
-                        }
-                    }
-                    // chunk c8 of the row, at its swizzled place in the staging tile / in C's stage
-                    if (AZB_P_ASYNC && isP) azb_st_async(ybase + (uint32_t)((c8 ^ sw) << 4), o[g], ybar);
-                    else srow[c8 ^ sw] = o[g];
+                    // chunk c8 of the row, at its swizzled place in the staging tile
+                    srow[c8 ^ sw] = make_uint4(ow[0], ow[1], ow[2], ow[3]);
                 }
             }
             // hand the ring block back
@@ -836,63 +552,15 @@ k_resblock(const azb_params p)
             asm volatile("tcgen05.fence::before_thread_sync;");
             __syncwarp();
             if (lane == 0) azt_mbar_arrive(&bar_blk_free[blk]);
-            if (!(AZB_P_ASYNC && isP)) {
-                // staging tile complete: the storer sends it on (the copy engine, async proxy, reads it)
-                asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-                __syncwarp();
-                if (lane == 0) azt_mbar_arrive(&bar_out_done[sb]);
-            }
-            if (hpass) {
-                // the warps with channels 0..31 hand their partial sums to the warps with channels
-                // 32..63 of the same rows (named barrier 5 + group, all eight warps); two buffers by
-                // slab parity, so the readers of one slab and the writers of the next never meet
-                float *hx = s_hx[grp][(t >> 1) & 1];
-                if (half == 0) {
-#pragma unroll
-                    for (int hh = 0; hh < AZB_HEADS; hh++) hx[hh * 128 + l] = hacc[hh];
-                    // (both halves wait: an arrive-only producer two slabs ahead would complete the
-                    // barrier on its own)
-                    if (grp == 0) asm volatile("bar.sync 5, 256;" ::: "memory");
-                    else asm volatile("bar.sync 6, 256;" ::: "memory");
-                } else {
-                    if (grp == 0) asm volatile("bar.sync 5, 256;" ::: "memory");
-                    else asm volatile("bar.sync 6, 256;" ::: "memory");
-                    const long long board = (g0 + at.j / n) * p.bpg + hbl;
-                    float v[AZB_HEADS];
-#pragma unroll
-                    for (int hh = 0; hh < AZB_HEADS; hh++)
-                        v[hh] = fmaxf(hx[hh * 128 + l] + hacc[hh] + azb_heads_c[AZB_HEADS * AZT_C + hh], 0.f);
-                    if (real && board < p.heads_boards) {
-                        uint32_t *dst = reinterpret_cast<uint32_t *>(
-                            p.heads_out + board * p.heads_stride + (long long)(y * n + hbx) * AZB_HEADS);
-#pragma unroll
-                        for (int hh = 0; hh < AZB_HEADS; hh += 2) {
-                            __nv_bfloat162 pr = __floats2bfloat162_rn(v[hh], v[hh + 1]);
-                            dst[hh >> 1] = *reinterpret_cast<uint32_t *>(&pr);
-                        }
-                    }
-                }
-            }
-            if (prof_on) prof_acc[3] += clock64() - tb_;
+            // staging tile complete: the storer sends it on (the copy engine, async proxy, reads it)
+            asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+            __syncwarp();
+            if (lane == 0) azt_mbar_arrive(&bar_out_done[sb]);
         }
     }
 #undef AZB_RING
-    if (prof_on && (warp == 0 || warp == 8 || warp >= 16)) {
-        // rows: rank x {epilogue g0, epilogue g1, mma even, mma odd, loader, relay, storer even, storer odd}
-        const int role = warp == 0 ? 0 : warp == 8 ? 1 : warp - 14;
-        unsigned long long *row = p.prof + ((size_t)rank * 8 + role) * 8;
-        for (int k = 0; k < 6; k++) row[k] = (unsigned long long)prof_acc[k];
-        row[6] = (unsigned long long)(clock64() - prof_t0);
-        row[7] = (unsigned long long)NT;
-    }
     asm volatile("tcgen05.fence::before_thread_sync;");
     __syncthreads();
-    if ((p.debug & 16) && p.prof != nullptr && tid == 0) {
-        unsigned long long gt;
-        asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(gt));
-        p.prof[128 + 4 * blockIdx.x + 1] = gt;
-        p.prof[128 + 4 * blockIdx.x + 3] = (unsigned long long)NT;
-    }
     // neither CTA may leave while the other can still reach into its shared memory
     azb_cluster_sync();
     if (warp == 0)

@@ -1306,39 +1306,21 @@ int az_nn_resblock_clusters(void)
     return azb_max_clusters[az_current_device()];
 }
 
-static int azb_debug = 0;
-static unsigned long long *azb_prof = nullptr;
-/* probe hooks, not part of the ABI (tools/probe/block_time.py) */
-void azb_set_debug(int flags) { azb_debug = flags; }
-void azb_set_prof(unsigned long long *prof_dev) { azb_prof = prof_dev; }
-
 size_t az_nn_resblock_scratch_bytes(void)
 {
-    /* only the AZB_HANDOVER == 2 probe build passes the intermediate slabs through global memory */
-    return AZB_VIA_L2 ? (size_t)(az_sm_count(az_current_device()) / 2) * AZB_R * AZT_OUT_BYTES : 0;
+    /* the intermediate slabs travel through distributed shared memory, never global memory */
+    return 0;
 }
 
-struct azb_heads_arg {
-    void *out; int64_t stride;
-};
-
-static int azb_launch(void *x_dev, const void *w_dev, const float *bias_dev, void *scratch_dev,
-                      int board_size, int64_t num_boards, int passes, const int32_t *live_rows_dev,
-                      const azb_heads_arg *heads, void *stream)
+static int azb_launch(void *x_dev, const void *w_dev, const float *bias_dev, int board_size,
+                      int64_t num_boards, int passes, const int32_t *live_rows_dev, void *stream)
 {
     azb_params p = {};
     p.live = live_rows_dev;
-    if (heads) {
-        p.heads_out = (uint16_t *)heads->out; p.heads_stride = heads->stride;
-        p.heads_boards = num_boards;
-    }
     p.x = (uint8_t *)x_dev; p.w = (const uint8_t *)w_dev; p.bias = bias_dev;
     p.n = board_size; p.bpg = 128 / (board_size + 1);
     p.groups = (num_boards + p.bpg - 1) / p.bpg;
     p.passes = passes;
-    p.scratch = (uint8_t *)scratch_dev;
-    p.debug = azb_debug;
-    p.prof = azb_prof;
     // clusters of two CTAs (one per SM) that can be resident at once on this device
     int *max_clusters = azb_max_clusters;
     const int dev = az_current_device();
@@ -1382,45 +1364,19 @@ int az_nn_resblocks_live(void *x_dev, const void *w_dev, const float *bias_dev, 
                          int board_size, int64_t num_boards, int num_blocks, const int32_t *live_rows_dev,
                          void *stream)
 {
-    return az_nn_resblocks_heads_live(x_dev, w_dev, bias_dev, scratch_dev, board_size, num_boards, num_blocks,
-                                      nullptr, nullptr, 0, live_rows_dev, stream);
-}
-
-int az_nn_resblocks_heads_live(void *x_dev, const void *w_dev, const float *bias_dev, void *scratch_dev,
-                               int board_size, int64_t num_boards, int num_blocks, const float *heads_wb_dev,
-                               void *heads_out_dev, int64_t heads_board_stride, const int32_t *live_rows_dev,
-                               void *stream)
-{
-    azb_heads_arg heads = {};
-    if (heads_wb_dev || heads_out_dev) {
-        // the fused heads need the shipped epilogue and a last block to ride on
-        if (!heads_wb_dev || !heads_out_dev || AZB_CDIRECT || num_blocks < 1 ||
-            heads_board_stride < (int64_t)board_size * board_size * AZB_HEADS || (heads_board_stride & 1))
-            return AZ_E_INVALID;
-        heads.out = heads_out_dev; heads.stride = heads_board_stride;
-        // weights into constant memory, in stream order (a memcpy node under graph capture, so a
-        // replay picks up weights refreshed in place)
-        int rc = az_check(cudaMemcpyToSymbolAsync(azb_heads_c, heads_wb_dev, AZB_HEAD_FLOATS * sizeof(float), 0,
-                                                  cudaMemcpyDeviceToDevice, (cudaStream_t)stream));
-        if (rc != AZ_OK) return rc;
-    }
-    if (!x_dev || !w_dev || !bias_dev || (AZB_VIA_L2 && !scratch_dev) || board_size < 2 || board_size > 19 ||
-        num_boards < 0 || num_blocks < 0)
+    if (!x_dev || !w_dev || !bias_dev || board_size < 2 || board_size > 19 || num_boards < 0 || num_blocks < 0)
         return AZ_E_INVALID;
     if (num_boards == 0) return AZ_OK;
-    // the chained form needs the shipped hand-over (one storer thread, staged output)
-    const int chain = (AZB_CDIRECT || AZB_STORERS != 1 || AZB_HANDOVER != 0) ? 1 : AZB_MAXPASS;
-    for (int b = 0; b < num_blocks; b += chain) {
-        const int passes = num_blocks - b < chain ? num_blocks - b : chain;
+    for (int b = 0; b < num_blocks; b += AZB_MAXPASS) {
+        const int passes = num_blocks - b < AZB_MAXPASS ? num_blocks - b : AZB_MAXPASS;
         int rc = azb_launch(x_dev, (const uint8_t *)w_dev + (size_t)b * 2 * AZT_WBYTES, bias_dev + (size_t)b * 2 * AZT_C,
-                            scratch_dev, board_size, num_boards, passes, live_rows_dev,
-                            heads.out && b + passes == num_blocks ? &heads : nullptr, stream);
+                            board_size, num_boards, passes, live_rows_dev, stream);
         if (rc != AZ_OK) return rc;
     }
     return AZ_OK;
 }
 
-static_assert(AZB_SMEM_BYTES + 4096 + sizeof(float) * 2 * 2 * AZB_HEADS * 128 <= 232448, "k_resblock: dynamic + static shared memory per CTA");
+static_assert(AZB_SMEM_BYTES + 4096 <= 232448, "k_resblock: dynamic + static shared memory per CTA");
 
 int az_play_commit(az_engine *e, const az_play_params *p, int32_t *chosen_dev, void *stream)
 {

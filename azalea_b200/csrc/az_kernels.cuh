@@ -20,18 +20,6 @@
 
 #include "az_common.cuh"
 
-// Shared-memory staging of the root's children for the descents of a batch (the north star's
-// "hot tree levels").  Built, bit-exact (the whole GPU suite passes with it), measured, and a
-// loss: at the same capture point ncu shows 144.9 vs 136.9 us, 1901 vs 1857 warp instructions
-// per descent and 97 vs 93 MB of DRAM traffic per launch (profiles/r02_k_select_staged.txt vs
-// r02_k_select.txt), and in the running step the launch is 6.7 % slower (0.164 vs 0.154 ms,
-// tree-only 1.54e8 vs 1.61e8 simulations/s, A/B on one box).  The root level is re-read from L1
-// anyway (69 % L1 hit rate), so staging saves nothing and adds a serial prologue, a warp
-// barrier per descent and a write-back to a kernel bound by latency and issue.  Off by default.
-#ifndef AZ_STAGE_ROOT
-#define AZ_STAGE_ROOT 0
-#endif
-
 struct az_select_args {
     int batch;
     float coef;
@@ -238,18 +226,11 @@ __global__ void __launch_bounds__(AZ_WARPS_PER_CTA * 32, MAXS <= 4 ? AZ_SELECT_M
 k_select(az_engine e, az_select_args a)
 {
     __shared__ uint32_t smask_all[AZ_WARPS_PER_CTA][64];
-    // The game's hottest tree level, the root's children, staged in shared memory for the
-    // batch: every one of the `batch` descents starts by scoring all of them
-    // (search_tree.py:192-204 slices the same arrays once per descent), and the virtual
-    // losses of the batch (mcts.py:69-72) land on them first.  Read from the pool once,
-    // updated in place here, the touched records written back once.
-    __shared__ uint4 sroot_all[AZ_WARPS_PER_CTA][AZ_STAGE_ROOT ? MAXS * 32 : 1];
     const int lane = az_lane();
     const int wib = threadIdx.x >> 5;
     const int g = e.g0 + blockIdx.x * AZ_WARPS_PER_CTA + wib;
     if (g >= e.g1) return;
     uint32_t *smask = smask_all[wib];
-    uint4 *sroot = sroot_all[wib];
     int32_t *meta = e.meta + (size_t)g * AZ_META_INTS;
     int4 *info = e.leaf_info + (size_t)g * e.B;
     const int status = meta[M_STATUS];
@@ -315,16 +296,6 @@ k_select(az_engine e, az_select_args a)
     const bool pack = (e.cfg.flags & AZ_CFG_PACK_LEAVES) != 0;
     // per launch: small.  nn_rows counts rotated rows (az_engine_set_reflect) in its high half
     uint32_t sum_k = 0, sum_d = 0, uniq = 0, nn_rows = 0, term = 0;
-    const int k0 = (int)(rootlink & AZ_LINK_KMASK), fc0 = (int)(rootlink >> AZ_LINK_KBITS);
-    uint32_t touched = 0;                   // bit s: this lane's root child lane + 32 s took a virtual loss
-    if (AZ_STAGE_ROOT) {
-#pragma unroll
-        for (int s = 0; s < MAXS; s++) {
-            const int j = lane + 32 * s;
-            if (j < k0) sroot[j] = nodes[fc0 + j];
-        }
-        __syncwarp();
-    }
 
     for (int b = 0; b < a.batch; b++) {
         uint32_t x = rx, o = ro, link = rootlink;
@@ -338,7 +309,7 @@ k_select(az_engine e, az_select_args a)
 #pragma unroll
             for (int s = 0; s < MAXS; s++) {
                 int j = lane + 32 * s;
-                rec[s] = j < k ? (AZ_STAGE_ROOT && depth == 0 ? sroot[j] : nodes[fc + j]) : make_uint4(0, 0, 0, 0);
+                rec[s] = j < k ? nodes[fc + j] : make_uint4(0, 0, 0, 0);
                 ni += (int)__uint_as_float(rec[s].x);
             }
             // score_actions, mcts.py:119-136.  sum(N) is a sum of small
@@ -408,17 +379,9 @@ k_select(az_engine e, az_select_args a)
             node = fc + jstar;
             // virtual loss on the way down (mcts.py:69,79-92): N += 1, W += 1
             // on every node of the path except the root
-            if (lane == owner) {
-                float2 nw = make_float2(__fadd_rn(__uint_as_float(cn), 1.0f),
-                                        __fadd_rn(__uint_as_float(cw), 1.0f));
-                if (AZ_STAGE_ROOT && depth == 0) {
-                    *reinterpret_cast<float2 *>(&sroot[jstar]) = nw;
-                    touched |= 1u << slot;
-                } else {
-                    *reinterpret_cast<float2 *>(&nodes[node]) = nw;
-                }
-            }
-            if (AZ_STAGE_ROOT && depth == 0) __syncwarp();       // the next descent's lanes read the staged level
+            if (lane == owner)
+                *reinterpret_cast<float2 *>(&nodes[node]) =
+                    make_float2(__fadd_rn(__uint_as_float(cn), 1.0f), __fadd_rn(__uint_as_float(cw), 1.0f));
             // ForwardSearchIterator.step, search_tree.py:298-308
             tile = az_kth_empty(~(x | o) & valid, jstar, e.NW);
             if (lane == (tile >> 5)) {
@@ -491,25 +454,13 @@ k_select(az_engine e, az_select_args a)
         const int depth = __shfl_sync(AZ_FULL, my_depth, b);
         const uint32_t *path = pathg + (size_t)b * e.path_stride;
         for (int dd = lane; dd < depth; dd += 32) {
-            const int nd = (int)(path[dd] & AZ_MAX_NODE);
-            // level 0 of every path is a root child: staged
-            float2 *p = AZ_STAGE_ROOT && dd == 0 ? reinterpret_cast<float2 *>(&sroot[nd - fc0])
-                                : reinterpret_cast<float2 *>(&nodes[nd]);
+            float2 *p = reinterpret_cast<float2 *>(&nodes[path[dd] & AZ_MAX_NODE]);
             float2 nw = *p;
             nw.x = __fadd_rn(nw.x, -1.0f);
             nw.y = __fadd_rn(nw.y, -1.0f);
             *p = nw;
         }
         __syncwarp();
-    }
-    // the touched root children go back to the pool: N and W after apply + undo, i.e. with the
-    // fp32 rounding of (W + 1) - 1 the reference leaves behind (mcts.py:79-92)
-    if (AZ_STAGE_ROOT) {
-#pragma unroll
-        for (int s = 0; s < MAXS; s++)
-            if ((touched >> s) & 1u)
-                *reinterpret_cast<float2 *>(&nodes[fc0 + lane + 32 * s]) =
-                    *reinterpret_cast<const float2 *>(&sroot[lane + 32 * s]);
     }
     if (lane == 0) {
         meta[M_SIM] = sim0 + a.batch;

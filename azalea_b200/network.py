@@ -91,11 +91,6 @@ class HexNetwork(nn.Module):
         # (default) chains all blocks in one launch, 1 is one launch per block, 0 the
         # two az_nn_conv3x3 launches per block
         self.tower_fused = int(os.environ.get('AZALEA_B200_FUSED', '2'))
-        # 1 (probe): the head convolutions run in the chained tower's last epilogue
-        # (az_nn_resblocks_heads_live): correct, and 3 % SLOWER in the step than the separate
-        # heads kernel (DESIGN.md 3.5) -- the consumer CTA's epilogue is the tower's
-        # bottleneck; 0 (default): the separate heads kernel
-        self.fuse_heads = int(os.environ.get('AZALEA_B200_FUSE_HEADS', '0'))
         nnet = sum(p.nelement() for p in self.parameters())
         nenc = sum(p.nelement() for p in self.encoder.parameters())
         logging.info('Net params: %d  Embedding params: %d', nnet - nenc, nenc)
@@ -215,10 +210,6 @@ class HexNetwork(nn.Module):
         fast['heads'] = pack(torch.cat([wv, wp]), torch.cat([bv, bp]))
         fast['heads_w32'] = keep32(torch.cat([wv, wp]).flatten(1))
         fast['heads_b32'] = keep32(torch.cat([bv, bp]))
-        # weights, biases, pad: what the tower's fused head epilogue keeps in constant memory
-        fast['heads_wb'] = keep32(torch.cat([torch.cat([wv, wp]).flatten().float(),
-                                             torch.cat([bv, bp]).float(),
-                                             torch.zeros(2, device=wv.device)]))
         nv, npc = wv.shape[0], wp.shape[0]
         hw = self.board_size ** 2
         hc = nv + npc
@@ -365,7 +356,7 @@ class HexNetwork(nn.Module):
                     torch.zeros(rows, 64, dtype=torch.bfloat16, device=dev),
                     torch.zeros(N, wfc.shape[1], dtype=torch.bfloat16, device=dev),
                     torch.empty(N, wfc.shape[0], dtype=torch.bfloat16, device=dev),
-                    # hand-over ring of the fused residual block (csrc/az_block.cuh)
+                    # scratch argument of the fused residual block (unused: az_nn_resblock_scratch_bytes() is 0)
                     torch.zeros(max(16, L.az_nn_resblock_scratch_bytes()), dtype=torch.uint8, device=dev))
             f['tower_buf'][(npad, dev, stream_id)] = bufs
         x, y, flat, yfc, scratch = bufs
@@ -387,15 +378,7 @@ class HexNetwork(nn.Module):
             ev.append((e0, e1, kind, N))
 
         fused = f.get('tower_fused') if self.tower_fused else None
-        heads_done = False
-        if fused is not None and self.tower_fused >= 2 and self.fuse_heads and f['heads_wb'].numel() == 392:
-            # the whole tower chained in one launch, the head convolutions in its last epilogue
-            wall, ball = f['tower_chain']
-            timed(lambda: _cabi.check(L.az_nn_resblocks_heads_live(
-                p(x), p(wall), p(ball), p(scratch), n, npad, len(fused), p(f['heads_wb']),
-                p(flat), flat.shape[1], live, stream)), 'chain%d' % len(fused))
-            heads_done = True
-        elif fused is not None and self.tower_fused >= 2:
+        if fused is not None and self.tower_fused >= 2:
             # the whole tower chained in one launch (csrc/az_block.cuh), in place
             wall, ball = f['tower_chain']
             timed(lambda: _cabi.check(L.az_nn_resblocks_live(
@@ -414,9 +397,8 @@ class HexNetwork(nn.Module):
         # head activations with the board row padded to a multiple of 8 (zeros):
         # the merged FC GEMM then runs a current cuBLAS kernel (K = 726 falls
         # back to a legacy one, 0.15 ms instead of 0.03)
-        if not heads_done:
-            _cabi.check(L.az_nn_heads_live(p(x), N * nn2, p(f['heads_w32']), p(f['heads_b32']),
-                                           p(flat), flat.shape[1], 64, 6, n, live, stream))
+        _cabi.check(L.az_nn_heads_live(p(x), N * nn2, p(f['heads_w32']), p(f['heads_b32']),
+                                       p(flat), flat.shape[1], 64, 6, n, live, stream))
         torch.mm(flat, f['fc_pad_t'], out=yfc)
         k2 = f['nfc2']
         if value_out is None and want_value:

@@ -387,11 +387,9 @@ int az_nn_conv3x3(const void *x_dev, const void *w_dev, const float *bias_dev,
  * cluster of two CTAs, conv1 on one SM streaming its output slabs through
  * distributed shared memory into conv2 on the other).  x: slab layout as for
  * az_nn_conv3x3; w: the two layers' packed weights back to back
- * [2][3 kx][3 ky][64][64] bf16; bias f32 [2][64]; scratch: device memory of
- * az_nn_resblock_scratch_bytes() bytes -- 0 in the shipped build, where the
- * intermediate slabs travel through distributed shared memory, so NULL is
- * fine; a probe build (AZB_HANDOVER=2) passes them through this ring instead
- * (L2 resident; one per stream that launches concurrently).
+ * [2][3 kx][3 ky][64][64] bf16; bias f32 [2][64]; scratch: unused, may be
+ * NULL (the intermediate slabs travel through distributed shared memory;
+ * az_nn_resblock_scratch_bytes() returns 0).
  * Bit-identical to az_nn_conv3x3(x, w1, b1, NULL, y) followed by
  * az_nn_conv3x3(y, w2, b2, x, x). */
 size_t az_nn_resblock_scratch_bytes(void);
@@ -424,20 +422,6 @@ int az_nn_stem_live(const int8_t *cells_dev, int cell_stride, int board_size,
 int az_nn_resblocks_live(void *x_dev, const void *w_dev, const float *bias_dev,
                          void *scratch_dev, int board_size, int64_t num_boards,
                          int num_blocks, const int32_t *live_rows_dev, void *stream);
-/* az_nn_resblocks_live with the head convolutions fused into the last block
- * (csrc/az_block.cuh): the epilogue that rounds the tower's output to bf16
- * also applies the two 1x1 head convolutions + BN + ReLU (64 -> 6 channels)
- * and writes out bf16 [num_boards][heads_board_stride] (6 per cell,
- * cell-major: what az_nn_heads writes with out_board_stride), so az_nn_heads
- * and its pass over the activations are not needed.  heads_wb: f32 [6][64]
- * weights followed by 6 biases and 2 pad floats (392 floats, device); copied
- * into constant memory in stream order at every call.  Same sums as
- * az_nn_heads up to the order of the fp32 additions. */
-int az_nn_resblocks_heads_live(void *x_dev, const void *w_dev, const float *bias_dev,
-                               void *scratch_dev, int board_size, int64_t num_boards,
-                               int num_blocks, const float *heads_wb_dev,
-                               void *heads_out_dev, int64_t heads_board_stride,
-                               const int32_t *live_rows_dev, void *stream);
 int az_nn_heads_live(const void *x_dev, int64_t positions, const float *w_dev,
                      const float *b_dev, void *out_dev, int64_t out_board_stride,
                      int channels, int heads, int padded_board_size,

@@ -864,46 +864,6 @@ def test_evaluator_live_rows():
         assert (v[live:] == 7.0).all() and (lg[live:] == 7.0).all(), live
 
 
-@pytest.mark.parametrize('n,N', ((11, 4100), (5, 37), (19, 300), (7, 1)))
-def test_fused_heads_match_heads_kernel(n, N):
-    """az_nn_resblocks_heads_live: the head convolutions computed in the chained
-    tower's last epilogue equal the separate heads kernel on the same tower
-    output up to the order of the fp32 additions (<= 1 bf16 ulp on a few
-    entries), and the tower's own output is unchanged."""
-    import ctypes
-    from azalea_b200 import _cabi, tower_layout as tl
-    L = _cabi.lib()
-    P = lambda t: ctypes.c_void_p(t.data_ptr())
-    torch.manual_seed(n * 1000 + N)
-    K = 3
-    rows = L.az_nn_tower_rows(n, N)
-    act = (torch.rand(N, n, n, 64, device='cuda') * 0.5).to(torch.bfloat16)
-    w = torch.cat([tl.pack_conv_weights((torch.randn(64, 64, 3, 3, device='cuda') * 0.03).to(torch.bfloat16))
-                   for _ in range(2 * K)]).contiguous()
-    b = (torch.randn(2 * K * 64, device='cuda') * 0.05).contiguous()
-    hw = torch.randn(6, 64, device='cuda') * 0.2
-    hb = torch.randn(6, device='cuda') * 0.1
-    wb = torch.cat([hw.flatten(), hb, torch.zeros(2, device='cuda')]).contiguous()
-    stride = (n * n * 6 + 7) & ~7
-    st = ctypes.c_void_p(torch.cuda.current_stream().cuda_stream)
-    x0 = tl.to_slabs(act)
-    assert x0.shape[0] == rows
-    x1 = x0.clone()
-    want = torch.zeros(N, stride, dtype=torch.bfloat16, device='cuda')
-    got = torch.zeros(N, stride, dtype=torch.bfloat16, device='cuda')
-    assert L.az_nn_resblocks(P(x0), P(w), P(b), None, n, N, K, st) == 0
-    assert L.az_nn_heads(P(x0), N * n * n, P(hw), P(hb), P(want), stride, 64, 6, n, st) == 0
-    assert L.az_nn_resblocks_heads_live(P(x1), P(w), P(b), None, n, N, K, P(wb), P(got), stride, None, st) == 0
-    torch.cuda.synchronize()
-    assert torch.equal(x0, x1)
-    g, wv = got.float(), want.float()
-    assert (got[:, n * n * 6:] == 0).all()
-    diff = (g - wv).abs()
-    tol = 2.0 ** -7 * wv.abs().clamp(min=2.0 ** -6)      # one bf16 ulp
-    assert (diff <= tol).all(), float(diff.max())
-    assert (diff > 0).float().mean() < 0.02
-
-
 def test_pipelined_harvest_equals_harvest():
     """harvest_begin / harvest_end (count sync, copy to pinned memory and clear
     enqueued, the next move launched before the rows are waited for) return
