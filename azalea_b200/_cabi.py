@@ -22,7 +22,10 @@ AZ_CFG_SOFT_POOL_FULL, AZ_CFG_PACK_LEAVES = 1, 2
 AZ_ABI_VERSION = 3
 (AZ_BUF_LEAF_BOARD, AZ_BUF_LEAF_INFO, AZ_BUF_VALUE, AZ_BUF_PRIOR, AZ_BUF_META,
  AZ_BUF_REPLAY, AZ_BUF_COUNTERS, AZ_BUF_LEAF_MOVES, AZ_BUF_GLOBALS,
- AZ_BUF_LEAF_ROWS) = range(10)
+ AZ_BUF_LEAF_ROWS, AZ_BUF_RESIGN) = range(11)
+# AZ_BUF_RESIGN columns: lowest r of colours 1 / 2 (f32 bits), resigned games, calibration games,
+# false positives, then the 65-bin histogram of the winner's lowest r
+AZ_RS_MIN, AZ_RS_RESIGNED, AZ_RS_CALIB, AZ_RS_FALSE_POS, AZ_RS_HIST, AZ_RS_BINS = 0, 2, 3, 4, 5, 65
 COUNTER_NAMES = ('simulations', 'sum_children', 'sum_depth', 'unique_leaves',
                  'expanded_children', 'plies', 'games', 'replay_rows',
                  'replay_dropped', 'games_failed', 'compacted_nodes',
@@ -108,6 +111,7 @@ def lib():
     L.az_engine_set_window.argtypes = [eng, C.c_int, C.c_int]
     L.az_engine_set_reflect.argtypes = [eng, C.c_int]
     L.az_engine_set_playout_cap.argtypes = [eng, C.c_float, C.c_int]
+    L.az_engine_set_resign.argtypes = [eng, C.c_float, C.c_float]
     L.az_status.argtypes = [eng, i32p, vp]
     L.az_stub_eval.argtypes = [eng, C.c_int, vp]
     L.az_replay_collate.argtypes = [vp, C.c_int, vp, C.c_int, C.c_int, i32p, i32p,

@@ -21,6 +21,7 @@
 #define AZ_WARPS_PER_CTA 4
 #define AZ_META_INTS 16
 #define AZ_CNT_PER_GAME 16
+#define AZ_RESIGN_INTS 72           // AZ_BUF_RESIGN row: AZ_RS_* below, padded to 72
 
 // meta[g][*]
 enum {
@@ -41,6 +42,16 @@ enum {
     M_PLY_SIM0 = 14 // M_SIM when this move's search began (az_engine_set_playout_cap)
 };
 
+// resign[g][*] (AZ_BUF_RESIGN, az_engine_set_resign)
+enum {
+    AZ_RS_MIN = 0,          // [0], [1]: f32 bits of colour 1's / 2's lowest r in this game
+    AZ_RS_RESIGNED = 2,     // games of this slot that ended by resignation
+    AZ_RS_CALIB = 3,        // calibration games of this slot that ended with a winner
+    AZ_RS_FALSE_POS = 4,    // ... whose winner's lowest r was below the threshold
+    AZ_RS_HIST = 5,         // [5, 70): histogram of the winner's lowest r
+    AZ_RS_BINS = 65
+};
+
 struct az_engine {
     az_config cfg;
     int device;
@@ -49,6 +60,9 @@ struct az_engine {
     int reflect;            // 1: network rows in a random orientation (az_engine_set_reflect)
     int fast_descents;      // > 0: playout cap on, new descents of a fast ply (az_engine_set_playout_cap)
     unsigned long long full_thresh;     // a ply is a full search iff its coin < full_thresh
+    int resign_on;          // 1: resignation / calibration bookkeeping on (az_engine_set_resign)
+    float resign_thresh;    // the mover resigns iff r < resign_thresh
+    unsigned long long calib_thresh;    // a game is a calibration game iff its coin < calib_thresh
     int cell_stride;        // bytes per leaf board row (nn rounded up to 16)
     int path_stride;        // uint32 per descent path
     int row_bytes;          // replay row
@@ -70,6 +84,7 @@ struct az_engine {
     int32_t *leaf_rows;     // [G]: [g0] = live packed leaf rows of the window starting at g0
     uint8_t *hist;          // [G][hist_rows][row_bytes]
     uint8_t *replay;        // [replay_rows][row_bytes]
+    uint32_t *resign;       // [G][AZ_RESIGN_INTS]
     az_buffer_desc desc[AZ_BUF__COUNT];
     size_t total_bytes;
 };
@@ -246,6 +261,18 @@ __device__ __forceinline__ bool az_full_search(const az_engine &e, const int32_t
                                  (uint32_t)(e.cfg.seed >> 32) ^ (uint32_t)meta[M_GID_HI]);
     const uint4 c = make_uint4((uint32_t)meta[M_PLY], 0u, 0u, AZ_FULL_SEARCH_DOMAIN);
     return (unsigned long long)az_philox(c, key).x < e.full_thresh;
+}
+
+// Philox counter domain of the resignation calibration coin (word w)
+#define AZ_RESIGN_DOMAIN 0x2E51C0A1u
+
+// Resignation (az_engine_set_resign): is this game a calibration game, one that never resigns?
+// One coin per (seed, global game id), counter (0, 0, 0, domain).
+__device__ __forceinline__ bool az_calibration_game(const az_engine &e, const int32_t *meta)
+{
+    const uint2 key = make_uint2((uint32_t)e.cfg.seed ^ (uint32_t)meta[M_GID_LO],
+                                 (uint32_t)(e.cfg.seed >> 32) ^ (uint32_t)meta[M_GID_HI]);
+    return (unsigned long long)az_philox(make_uint4(0u, 0u, 0u, AZ_RESIGN_DOMAIN), key).x < e.calib_thresh;
 }
 
 __device__ __forceinline__ float az_u01(uint32_t r)     // (0,1)

@@ -81,6 +81,8 @@ __device__ __forceinline__ void az_game_reset(const az_engine &e, int g, int32_t
     }
     uint4 *nodes = e.nodes + ((size_t)g * 2 + meta[M_HALF]) * e.C;
     az_tree_reset(nodes, meta, lane);
+    // resignation: no value seen yet by either colour of the new game
+    if (lane < 2) e.resign[(size_t)g * AZ_RESIGN_INTS + AZ_RS_MIN + lane] = 0x7f800000u;    // +inf
     if (lane == 0) {
         meta[M_COLOR] = 1;
         meta[M_WINNER] = 0;
@@ -108,6 +110,7 @@ __global__ void k_reset(az_engine e, const uint8_t *mask, int init)
     if (init) {
         if (lane < AZ_META_INTS) meta[lane] = 0;
         if (lane < AZ_CNT_PER_GAME) e.counters[(size_t)g * AZ_CNT_PER_GAME + lane] = 0ull;
+        for (int i = lane; i < AZ_RESIGN_INTS; i += 32) e.resign[(size_t)g * AZ_RESIGN_INTS + i] = 0u;
         if (g == 0 && lane < 16) e.globals[lane] = 0ull;
         __syncwarp();
         if (lane == 0) {
@@ -405,6 +408,74 @@ __global__ void k_stub_eval(az_engine e, int mode)
 
 // ------------------------------------------------------------ lockstep play
 
+// A game of `nply` plies ended with `result`: flush its history rows to the replay output, count
+// it and (auto_reset) start the next game in the slot.
+__device__ __forceinline__ void az_finish_game(const az_engine &e, const az_play_params &p, int g,
+                                               int32_t *meta, unsigned long long *cnt, int lane,
+                                               int nply, int result)
+{
+    // play_game.py:63-67: reward = result - 2 for the first player's rows,
+    // negated on the second player's
+    if (p.collect_replay) {
+        const int plies = min(nply, e.hist_rows);
+        const uint8_t *src = e.hist + (size_t)g * e.hist_rows * e.row_bytes;
+        // playout cap: only the rows of full-search plies (reserved bit 0 clear) are flushed
+        int rows = plies;
+        if (e.fast_descents) {
+            int kept = 0;
+            for (int r = lane; r < plies; r += 32)
+                kept += !(reinterpret_cast<const az_row_header *>(src + (size_t)r * e.row_bytes)->reserved & 1);
+            rows = __reduce_add_sync(AZ_FULL, kept);
+        }
+        // reserve `rows` output rows; the cursor only ever advances by reservations that fit,
+        // so concurrent finishers can never be handed space beyond the capacity
+        unsigned long long base = ~0ull;
+        if (lane == 0) {
+            unsigned long long cur = *(volatile unsigned long long *)&e.globals[0];
+            for (;;) {
+                if (cur + (unsigned long long)rows > (unsigned long long)e.cfg.replay_rows) break;
+                const unsigned long long prev = atomicCAS(&e.globals[0], cur, cur + (unsigned long long)rows);
+                if (prev == cur) { base = cur; break; }
+                cur = prev;
+            }
+        }
+        base = __shfl_sync(AZ_FULL, base, 0);
+        if (base != ~0ull) {
+            uint8_t *dst = e.replay + (size_t)base * e.row_bytes;
+            if (rows == plies) {
+                const size_t n16 = (size_t)rows * e.row_bytes / 16;
+                for (size_t i = lane; i < n16; i += 32)
+                    reinterpret_cast<uint4 *>(dst)[i] = reinterpret_cast<const uint4 *>(src)[i];
+            } else {
+                // the kept rows, compacted in ply order
+                const int n16 = e.row_bytes / 16;
+                uint8_t *d = dst;
+                for (int r = 0; r < plies; r++) {
+                    const uint8_t *s = src + (size_t)r * e.row_bytes;
+                    if (reinterpret_cast<const az_row_header *>(s)->reserved & 1) continue;
+                    for (int i = lane; i < n16; i += 32)
+                        reinterpret_cast<uint4 *>(d)[i] = reinterpret_cast<const uint4 *>(s)[i];
+                    d += e.row_bytes;
+                }
+            }
+            __syncwarp();
+            for (int r = lane; r < rows; r += 32) {
+                az_row_header *h = reinterpret_cast<az_row_header *>(dst + (size_t)r * e.row_bytes);
+                float rw = (float)(result - 2);
+                h->reward = (h->ply & 1) ? -rw : rw;    // the row's own ply (rows may be skipped)
+                h->result = result;
+                h->game_len = nply;
+            }
+            if (lane == 0) cnt[AZ_CNT_REPLAY_ROWS] += rows;
+        } else if (lane == 0) {
+            cnt[AZ_CNT_REPLAY_DROPPED] += rows;
+        }
+    }
+    if (lane == 0) cnt[AZ_CNT_GAMES] += 1;
+    __syncwarp();
+    if (p.auto_reset) az_game_reset(e, g, meta, lane, true);
+}
+
 __global__ void __launch_bounds__(AZ_WARPS_PER_CTA * 32)
 k_play_commit(az_engine e, az_play_params p, int32_t *chosen)
 {
@@ -440,6 +511,47 @@ k_play_commit(az_engine e, az_play_params p, int32_t *chosen)
     }
     const int k = (int)(rootlink & AZ_LINK_KMASK), fc = (int)(rootlink >> AZ_LINK_KBITS);
     const int nslots = (k + 31) >> 5;
+    // resignation (az_engine_set_resign), after the search and before the move is drawn:
+    // r = max(Q_root, Q_best) for the player to move.  A node's W is from the view of the
+    // player to move there, so Q_best = -W/N of the most-visited child (lowest ordinal on ties).
+    if (e.resign_on) {
+        uint32_t nmax = 0u;                 // N >= 0: the float order is the bit order
+        for (int s = 0; s < nslots; s++) {
+            const int j = lane + 32 * s;
+            if (j < k) nmax = max(nmax, nodes[fc + j].x);
+        }
+        nmax = __reduce_max_sync(AZ_FULL, nmax);
+        const uint4 root = nodes[0];
+        float r = __fdiv_rn(__uint_as_float(root.y), __uint_as_float(root.x));
+        if (nmax != 0u) {
+            uint32_t best = (uint32_t)k;
+            for (int s = 0; s < nslots; s++) {
+                const int j = lane + 32 * s;
+                if (j < k && nodes[fc + j].x == nmax) best = min(best, (uint32_t)j);
+            }
+            const uint4 c = nodes[fc + __reduce_min_sync(AZ_FULL, best)];
+            r = fmaxf(r, -__fdiv_rn(__uint_as_float(c.y), __uint_as_float(c.x)));
+        }
+        const int color = meta[M_COLOR];
+        uint32_t *rs = e.resign + (size_t)g * AZ_RESIGN_INTS;
+        if (az_calibration_game(e, meta)) {
+            // never resigns: keep each colour's lowest r for the bookkeeping at the game's end
+            if (lane == 0)
+                rs[AZ_RS_MIN + color - 1] =
+                    __float_as_uint(fminf(__uint_as_float(rs[AZ_RS_MIN + color - 1]), r));
+        } else if (r < e.resign_thresh) {
+            // the mover resigns: no move, no row for this ply, the opponent wins
+            const int result = color == 1 ? 1 : 3;
+            if (lane == 0) {
+                meta[M_WINNER] = 3 - color;
+                rs[AZ_RS_RESIGNED] += 1;
+                if (chosen) reinterpret_cast<int4 *>(chosen)[g] = make_int4(0, -1, result, ply);
+            }
+            __syncwarp();
+            az_finish_game(e, p, g, meta, cnt, lane, ply, result);
+            return;
+        }
+    }
     // Policy.choose_action, policy.py:142-149
     float temp = 0.0f;
     if (p.move_sampling && ply < p.exploration_depth) temp = p.temperature;
@@ -572,69 +684,18 @@ k_play_commit(az_engine e, az_play_params p, int32_t *chosen)
         cnt[AZ_CNT_PLIES] += 1;
         if (fast) cnt[AZ_CNT_FAST_PLIES] += 1;
         if (chosen) reinterpret_cast<int4 *>(chosen)[g] = make_int4(tile + 1, move_id, result, nply);
+        // a calibration game ended with a winner: would the winner have resigned at some ply?
+        if (won > 0 && e.resign_on && az_calibration_game(e, meta)) {
+            uint32_t *rs = e.resign + (size_t)g * AZ_RESIGN_INTS;
+            const float m = __uint_as_float(rs[AZ_RS_MIN + won - 1]);
+            rs[AZ_RS_CALIB] += 1;
+            rs[AZ_RS_FALSE_POS] += m < e.resign_thresh ? 1u : 0u;
+            const int bin = (int)floorf(__fmul_rn(__fadd_rn(m, 1.0f), 64.0f));
+            rs[AZ_RS_HIST + min(AZ_RS_BINS - 1, max(0, bin))] += 1;
+        }
     }
     if (!over) return;
-
-    // play_game.py:63-67: reward = result - 2 for the first player's rows,
-    // negated on the second player's
-    if (p.collect_replay) {
-        const int plies = min(nply, e.hist_rows);
-        const uint8_t *src = e.hist + (size_t)g * e.hist_rows * e.row_bytes;
-        // playout cap: only the rows of full-search plies (reserved bit 0 clear) are flushed
-        int rows = plies;
-        if (e.fast_descents) {
-            int kept = 0;
-            for (int r = lane; r < plies; r += 32)
-                kept += !(reinterpret_cast<const az_row_header *>(src + (size_t)r * e.row_bytes)->reserved & 1);
-            rows = __reduce_add_sync(AZ_FULL, kept);
-        }
-        // reserve `rows` output rows; the cursor only ever advances by reservations that fit,
-        // so concurrent finishers can never be handed space beyond the capacity
-        unsigned long long base = ~0ull;
-        if (lane == 0) {
-            unsigned long long cur = *(volatile unsigned long long *)&e.globals[0];
-            for (;;) {
-                if (cur + (unsigned long long)rows > (unsigned long long)e.cfg.replay_rows) break;
-                const unsigned long long prev = atomicCAS(&e.globals[0], cur, cur + (unsigned long long)rows);
-                if (prev == cur) { base = cur; break; }
-                cur = prev;
-            }
-        }
-        base = __shfl_sync(AZ_FULL, base, 0);
-        if (base != ~0ull) {
-            uint8_t *dst = e.replay + (size_t)base * e.row_bytes;
-            if (rows == plies) {
-                const size_t n16 = (size_t)rows * e.row_bytes / 16;
-                for (size_t i = lane; i < n16; i += 32)
-                    reinterpret_cast<uint4 *>(dst)[i] = reinterpret_cast<const uint4 *>(src)[i];
-            } else {
-                // the kept rows, compacted in ply order
-                const int n16 = e.row_bytes / 16;
-                uint8_t *d = dst;
-                for (int r = 0; r < plies; r++) {
-                    const uint8_t *s = src + (size_t)r * e.row_bytes;
-                    if (reinterpret_cast<const az_row_header *>(s)->reserved & 1) continue;
-                    for (int i = lane; i < n16; i += 32)
-                        reinterpret_cast<uint4 *>(d)[i] = reinterpret_cast<const uint4 *>(s)[i];
-                    d += e.row_bytes;
-                }
-            }
-            __syncwarp();
-            for (int r = lane; r < rows; r += 32) {
-                az_row_header *h = reinterpret_cast<az_row_header *>(dst + (size_t)r * e.row_bytes);
-                float rw = (float)(result - 2);
-                h->reward = (h->ply & 1) ? -rw : rw;    // the row's own ply (rows may be skipped)
-                h->result = result;
-                h->game_len = nply;
-            }
-            if (lane == 0) cnt[AZ_CNT_REPLAY_ROWS] += rows;
-        } else if (lane == 0) {
-            cnt[AZ_CNT_REPLAY_DROPPED] += rows;
-        }
-    }
-    if (lane == 0) cnt[AZ_CNT_GAMES] += 1;
-    __syncwarp();
-    if (p.auto_reset) az_game_reset(e, g, meta, lane, true);
+    az_finish_game(e, p, g, meta, cnt, lane, nply, result);
 }
 
 __global__ void k_replay_clear(az_engine e)
@@ -789,6 +850,7 @@ static int az_layout(az_engine *e, const az_config *cfg)
     size_t o_lrows = off; off = az_align(off + (size_t)e->G * 4);
     size_t o_hist = off; off = az_align(off + (size_t)e->G * e->hist_rows * e->row_bytes);
     size_t o_replay = off; off = az_align(off + (size_t)e->cfg.replay_rows * e->row_bytes);
+    size_t o_resign = off; off = az_align(off + (size_t)e->G * AZ_RESIGN_INTS * 4);
     e->total_bytes = off;
     // offsets are stored as pointers relative to NULL until create() binds them
     e->nodes = (uint4 *)o_nodes;
@@ -806,6 +868,7 @@ static int az_layout(az_engine *e, const az_config *cfg)
     e->leaf_rows = (int32_t *)o_lrows;
     e->hist = (uint8_t *)o_hist;
     e->replay = (uint8_t *)o_replay;
+    e->resign = (uint32_t *)o_resign;
 #define AZ_DESC(which, off_, bytes_, elem_, nd_, s0, s1, s2, s3)                         \
     do {                                                                                 \
         az_buffer_desc *d = &e->desc[which];                                             \
@@ -822,6 +885,7 @@ static int az_layout(az_engine *e, const az_config *cfg)
     AZ_DESC(AZ_BUF_LEAF_MOVES, o_lmoves, (size_t)e->G * e->B * e->nn * 4, 4, 3, e->G, e->B, e->nn, 0);
     AZ_DESC(AZ_BUF_GLOBALS, o_glob, 16 * 8, 8, 1, 16, 0, 0, 0);
     AZ_DESC(AZ_BUF_LEAF_ROWS, o_lrows, (size_t)e->G * 4, 4, 1, e->G, 0, 0, 0);
+    AZ_DESC(AZ_BUF_RESIGN, o_resign, (size_t)e->G * AZ_RESIGN_INTS * 4, 4, 2, e->G, AZ_RESIGN_INTS, 0, 0);
 #undef AZ_DESC
     return AZ_OK;
 }
@@ -882,6 +946,7 @@ int az_engine_create(az_engine **out, const az_config *cfg, void *mem_dev, size_
     AZ_BIND(leaf_rows, int32_t *);
     AZ_BIND(hist, uint8_t *);
     AZ_BIND(replay, uint8_t *);
+    AZ_BIND(resign, uint32_t *);
 #undef AZ_BIND
     // scratch the evaluator reads even for unused slots must be defined
     rc = az_check(cudaMemsetAsync(e->leaf_board, 0, (size_t)e->G * e->B * e->cell_stride, 0));
@@ -1051,6 +1116,18 @@ int az_engine_set_playout_cap(az_engine *e, float full_search_prob, int fast_des
     e->fast_descents = fast_descents;
     // coin < p * 2^32 for an integer coin is coin < ceil(p * 2^32); exact in double
     e->full_thresh = (unsigned long long)ceil((double)full_search_prob * 4294967296.0);
+    return AZ_OK;
+}
+
+int az_engine_set_resign(az_engine *e, float threshold, float disable_prob)
+{
+    // (NaN fails every test)
+    if (!e || !(threshold <= 1.0f) || !(disable_prob >= 0.0f && disable_prob <= 1.0f))
+        return AZ_E_INVALID;
+    e->resign_on = threshold > -1.0f;
+    e->resign_thresh = e->resign_on ? threshold : 0.0f;
+    // coin < p * 2^32 for an integer coin is coin < ceil(p * 2^32); exact in double
+    e->calib_thresh = e->resign_on ? (unsigned long long)ceil((double)disable_prob * 4294967296.0) : 0ull;
     return AZ_OK;
 }
 

@@ -90,6 +90,8 @@ class Engine:
         self.globals = self._view(AZ_BUF_GLOBALS)
         # AZ_CFG_PACK_LEAVES: [g0] = live leaf rows of the window that starts at game g0
         self.leaf_rows = self._view(_cabi.AZ_BUF_LEAF_ROWS)
+        # per-slot resignation state and counts (az_engine_set_resign)
+        self.resign = self._view(_cabi.AZ_BUF_RESIGN)
         self.replay = self._view(AZ_BUF_REPLAY, torch.uint8) \
             if replay_rows else None
         self.cell_stride = self.leaf_board.shape[-1]
@@ -237,6 +239,30 @@ class Engine:
         check(self.lib.az_engine_set_playout_cap(self._h, float(full_search_prob),
                                                  int(fast_descents)))
 
+    def set_resign(self, threshold=None, disable_prob=0.1):
+        """Resignation with calibration games (az_engine_set_resign): after
+        the search, the player to move resigns when r = max(Q_root, Q_best)
+        is below ``threshold``, except in calibration games (probability
+        ``disable_prob``, one coin per game id), which never resign and
+        record how often the eventual winner's value fell below it
+        (``resign_stats``).  ``threshold=None`` (or <= -1) is off;
+        ``disable_prob=1`` only measures.  Read at launch time: set it before
+        capturing a graph."""
+        t = -1.0 if threshold is None else float(threshold)
+        check(self.lib.az_engine_set_resign(self._h, t, float(disable_prob)))
+
+    def resign_stats(self):
+        """Resignation counts summed over the slots (one D2H copy):
+        ``resigned_games``, ``calibration_games`` (calibration games that
+        ended with a winner), ``false_positives`` (those whose winner's lowest
+        r was below the threshold) and ``histogram`` (int64[65], the winner's
+        lowest r: bin i < 64 holds [-1 + i/64, -1 + (i+1)/64), bin 64 r >= 0)."""
+        tot = self.resign.to(torch.int64).sum(0).cpu().numpy()
+        return dict(resigned_games=int(tot[_cabi.AZ_RS_RESIGNED]),
+                    calibration_games=int(tot[_cabi.AZ_RS_CALIB]),
+                    false_positives=int(tot[_cabi.AZ_RS_FALSE_POS]),
+                    histogram=tot[_cabi.AZ_RS_HIST:_cabi.AZ_RS_HIST + _cabi.AZ_RS_BINS].copy())
+
     def root_uniform(self):
         """One visit on every child of every expanded root: the RandomPolicy
         seat (random_policy.py:25-41) in terms of the tree."""
@@ -344,7 +370,9 @@ def decode_replay_rows(rows, board_size):
     With the playout cap on (``Engine.set_playout_cap``) the rows of fast
     plies never reach the output: a game's rows may skip plies, while
     ``game_len`` and ``result`` are still the whole game's and ``reward``
-    follows the row's own ply.
+    follows the row's own ply.  A game that ended by resignation
+    (``Engine.set_resign``) has no row for its last ply, the one at which
+    the mover resigned: its rows are plies ``0 .. game_len - 1``.
     """
     rows = np.ascontiguousarray(rows)
     n, nn = board_size, board_size * board_size

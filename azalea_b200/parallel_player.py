@@ -18,8 +18,13 @@ from .selfplay import LockstepSelfPlay, rows_to_dataframe
 
 Metrics = Dict[str, float]
 
+# Player.read warns when more calibration games than this would have resigned the eventual winner
+RESIGN_MAX_FP_RATE = 0.05
+
 
 class Player:
+    resign = False      # resignation on (LockstepSelfPlay(resign_threshold=...))
+
     def __init__(self, pool, agents: Sequence, num_games: int = 4096,
                  seed: int = 0, **kwargs):
         self.agents = agents
@@ -46,6 +51,7 @@ class Player:
             move_exploration=settings.get('move_exploration', True),
             random_reflect=getattr(policy, 'random_reflect', False),
             seed=seed, **kwargs)
+        self.resign = self.sp.resign_threshold is not None
         self.running = True
 
     def read(self, size: int) -> Tuple[ReplayDataFrame, Metrics]:
@@ -53,6 +59,7 @@ class Player:
         examples = ReplayDataFrame()
         metrics: Metrics = defaultdict(int)
         fast0 = self.sp.counters()['fast_plies']
+        rs0 = self.sp.resign_stats() if self.resign else None
         while len(examples) < size:
             self.sp.step_move()
             if self.sp.eng.replay_count() == 0:
@@ -67,8 +74,24 @@ class Player:
             metrics['reward'] += float(np.sum(h['reward'][last]))
             examples.append(rows_to_dataframe(rows, self.board_size))
         metrics['fast_plies'] = self.sp.counters()['fast_plies'] - fast0
+        self._report_resign(metrics, rs0)
         self._report(metrics)
         return examples, metrics
+
+    def _report_resign(self, metrics, rs0) -> None:
+        """Resignation counts of this call; a warning when the calibration
+        games' false-positive rate (an upper bound on wrong resignations)
+        is above RESIGN_MAX_FP_RATE."""
+        if rs0 is None:
+            return
+        import logging
+        rs = self.sp.resign_stats()
+        metrics['resigned_games'] = rs['resigned_games'] - rs0['resigned_games']
+        calib = metrics['resign_calibration_games'] = rs['calibration_games'] - rs0['calibration_games']
+        fp = metrics['resign_false_positives'] = rs['false_positives'] - rs0['false_positives']
+        if calib and fp / calib > RESIGN_MAX_FP_RATE:
+            logging.warning('self-play: %d of %d calibration games (%.1f %%) would have resigned the '
+                            'eventual winner -- lower resign_threshold', fp, calib, 100.0 * fp / calib)
 
     def _report(self, metrics) -> None:
         """Games dropped on SearchTreeFull (parallel_player.py:71-76) and
@@ -90,6 +113,7 @@ class Player:
         chunks, total = [], 0
         metrics: Metrics = defaultdict(int)
         cnt0 = self.sp.counters()
+        rs0 = self.sp.resign_stats() if self.resign else None
         while total < size:
             self.sp.step_move()
             count = min(eng.replay_count(), eng.replay.shape[0])
@@ -101,6 +125,7 @@ class Player:
         metrics['games'] = cnt['games'] - cnt0['games']
         metrics['fast_plies'] = cnt['fast_plies'] - cnt0['fast_plies']
         metrics['moves_per_game'] = float(total)
+        self._report_resign(metrics, rs0)
         self._report(metrics)
         return torch.cat(chunks), metrics
 

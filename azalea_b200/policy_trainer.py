@@ -29,7 +29,12 @@ Deviations from the reference, all on purpose:
   playout cap randomization (Wu 2019) in the self-play refills: a ply gets the
   full search with probability ``full_search_prob`` and otherwise a fast one of
   ``fast_simulations`` without root noise, and only full-search plies become
-  training rows, so a refill finishes more games per GPU-second.
+  training rows, so a refill finishes more games per GPU-second;
+* ``resign_threshold`` (default None, off) and ``resign_disable_prob``
+  (default 0.1) turn on resignation (AlphaGo Zero) in the self-play refills:
+  the player to move resigns when its root value is below the threshold,
+  except in calibration games, which never resign and measure how often the
+  eventual winner would have; the refill metrics report both (rank 0's games).
 """
 import logging
 import os
@@ -204,8 +209,11 @@ def train(policy, config, rundir, *,
     num_games = int(config.get('num_selfplay_games', 1024))
 
     # playout cap randomization: a self-play setting, not part of the policy (not checkpointed)
+    # resignation (AlphaGo Zero) likewise: a data-generation setting, not checkpointed
     cap = dict(full_search_prob=float(config.get('full_search_prob', 1.0)),
-               fast_simulations=config.get('fast_simulations'))
+               fast_simulations=config.get('fast_simulations'),
+               resign_threshold=config.get('resign_threshold'),
+               resign_disable_prob=float(config.get('resign_disable_prob', 0.1)))
 
     game_class = _game_class(config['game'])
     game_factory = partial(game_class, board_size=config['board_size'])

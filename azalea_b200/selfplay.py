@@ -76,6 +76,46 @@ def playout_cap_descents(full_search_prob, fast_simulations, simulations, search
     return fast
 
 
+def resign_setting(threshold, disable_prob):
+    """Validated resignation setting: the threshold, or None when off.
+
+    ``threshold`` None or <= -1 is off.  Raises ``ValueError`` for a NaN
+    threshold or one above 1, and for ``disable_prob`` outside [0, 1].
+    """
+    p = float(disable_prob)
+    if not 0.0 <= p <= 1.0:
+        raise ValueError(f'resign_disable_prob must be in [0, 1], got {disable_prob!r}')
+    if threshold is None:
+        return None
+    t = float(threshold)
+    if not t <= 1.0:
+        raise ValueError(f'resign_threshold must be a number <= 1, got {threshold!r}')
+    return None if t <= -1.0 else t
+
+
+def resign_threshold_for(hist, calib_games, max_fp_rate):
+    """The highest resignation threshold whose estimated false-positive
+    rate is at most ``max_fp_rate``, from ``Engine.resign_stats()``.
+
+    Candidates are the histogram's bin edges ``-1 + j / 64``, j = 0..64; at
+    edge j the false positives are the calibration games whose winner's
+    lowest value fell in bins below j, so the estimate is exact for them.
+    It is an upper bound on the rate of wrong resignations (the loser might
+    have resigned first).  Returns -1.0, which turns resignation off, when
+    no higher edge qualifies.
+    """
+    hist = np.asarray(hist, dtype=np.int64)
+    if hist.shape != (65,):
+        raise ValueError(f'expected a 65-bin histogram, got shape {hist.shape}')
+    calib_games = int(calib_games)
+    if calib_games <= 0:
+        raise ValueError('no calibration games to estimate the false-positive rate from')
+    below = np.concatenate([[0], np.cumsum(hist[:64])])     # below[j]: games under edge j
+    ok = np.flatnonzero(below / calib_games <= float(max_fp_rate))
+    j = int(ok[-1]) if len(ok) else 0
+    return -1.0 + j / 64.0
+
+
 class StubEvaluator:
     """Deterministic device stub (test / bench aid; modes as in
     oracle/azalea_oracle.h): 0 uniform, 1 dyadic, 2 rough."""
@@ -93,7 +133,8 @@ class LockstepSelfPlay:
                  device=None, rank=0, world_size=1, nodes_per_game=None,
                  replay_rows=None, collect_replay=True, cuda_graph=True,
                  max_plies=300, random_play=False, streams=None, pack_leaves=None,
-                 random_reflect=False, full_search_prob=1.0, fast_simulations=None):
+                 random_reflect=False, full_search_prob=1.0, fast_simulations=None,
+                 resign_threshold=None, resign_disable_prob=0.1):
         # random_play: RandomPolicy self-play (random_policy.py:25-41) -- no
         # search, uniform move choice and uniform moves_prob at every ply;
         # how the reference fills the replay buffer before training
@@ -116,6 +157,10 @@ class LockstepSelfPlay:
         # noise whose replay row is dropped (az_engine_set_playout_cap); 0 = off
         self.fast_descents = 0 if self.random_play else playout_cap_descents(
             full_search_prob, fast_simulations, simulations, self.batch)
+        # resignation with calibration games (AlphaGo Zero): None = off (az_engine_set_resign)
+        self.resign_threshold = None if self.random_play else resign_setting(
+            resign_threshold, resign_disable_prob)
+        self.resign_disable_prob = float(resign_disable_prob)
         self.coef = float(exploration_coef)
         self.depth = int(exploration_depth)
         self.temperature = float(exploration_temperature)
@@ -154,6 +199,8 @@ class LockstepSelfPlay:
             self.eng.set_reflect(True)
         if self.fast_descents:
             self.eng.set_playout_cap(full_search_prob, self.fast_descents)
+        if self.resign_threshold is not None:
+            self.eng.set_resign(self.resign_threshold, self.resign_disable_prob)
         self.device = self.eng.device
         self.chosen = torch.zeros(self.G, 4, dtype=torch.int32,
                                   device=self.device)
@@ -254,9 +301,13 @@ class LockstepSelfPlay:
         recorded as such in the replay rows), so that a lockstep run no longer
         has every game at the same ply -- games end, restart, and reuse
         subtrees at different times, as in steady-state self-play.  Eager;
-        call it before the move graph is captured or between replays."""
+        call it before the move graph is captured or between replays.  Nobody
+        resigns on these plies: a uniform root says nothing about the
+        position."""
         eng, G = self.eng, self.G
         max_plies = int(max_plies)
+        if self.resign_threshold is not None:
+            eng.set_resign(None)
         try:
             for s in range(1, max_plies + 1):
                 g0 = -(-s * G // max_plies)         # slots with quota >= s
@@ -271,6 +322,8 @@ class LockstepSelfPlay:
                                 self.chosen)
         finally:
             eng.set_window(0, 0)
+            if self.resign_threshold is not None:
+                eng.set_resign(self.resign_threshold, self.resign_disable_prob)
 
     def capture(self):
         """Capture one move as a CUDA graph (capturing does not execute)."""
@@ -349,6 +402,9 @@ class LockstepSelfPlay:
 
     def counters(self):
         return self.eng.counter_totals()
+
+    def resign_stats(self):
+        return self.eng.resign_stats()
 
 
 def rows_to_dataframe(rows, board_size) -> ReplayDataFrame:

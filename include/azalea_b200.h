@@ -117,7 +117,15 @@ enum {
     AZ_BUF_GLOBALS = 8,     /* int64 [16]: [0] = replay append cursor (rows) */
     AZ_BUF_LEAF_ROWS = 9,   /* int32 [G]: [g0] = live leaf rows of the window starting at game g0
                                (AZ_CFG_PACK_LEAVES) */
-    AZ_BUF__COUNT = 10
+    AZ_BUF_RESIGN = 10,     /* uint32 [G][72] per-slot resignation state (az_engine_set_resign;
+                               sum the counts over games on the host): [0], [1] = f32 bits of
+                               colour 1's / 2's lowest r in the current game (+inf at its start);
+                               [2] = games that ended by resignation; [3] = calibration games that
+                               ended with a winner; [4] = of those, games whose winner's lowest r
+                               was below the threshold (false positives); [5..69] = histogram of
+                               the winner's lowest r over [3]'s games, bin min(64, max(0,
+                               floor((r + 1) * 64))) in f32; [70], [71] padding */
+    AZ_BUF__COUNT = 11
 };
 
 /* counter columns (AZ_BUF_COUNTERS); each game's warp owns its row, so the
@@ -213,6 +221,33 @@ int az_engine_set_reflect(az_engine *e, int on);
  * capturing a graph).  Off: every buffer is byte for byte what it is without
  * this call. */
 int az_engine_set_playout_cap(az_engine *e, float full_search_prob, int fast_descents);
+
+/* Resignation with calibration games (AlphaGo Zero, Silver et al. 2017,
+ * "Methods: Self-play"), off by default.  az_play_commit, after the search
+ * and before the move is drawn, computes r = max(Q_root, Q_best) for the
+ * player to move: Q_root = W/N of the root, Q_best = -W/N of the most-visited
+ * root child (lowest ordinal on ties; r = Q_root if no child has a visit), in
+ * f32 with round-to-nearest divisions.  Each game draws one coin from its
+ * Philox key (counter: 0), so the draw does not depend on windows, streams or
+ * the world size; with probability disable_prob the game is a calibration
+ * game and never resigns.  In any other game, r < threshold makes the mover
+ * resign: no move is drawn, no row is recorded for that ply and the tree is
+ * not re-rooted; the opponent is the winner, chosen_dev gets (0, -1, result,
+ * ply), and the game is finished like a won one (rows of plies 0..ply-1 are
+ * flushed with game_len = ply, AZ_CNT_GAMES counts it, AZ_CNT_PLIES does not
+ * count the resigning ply; then auto_reset).  The check comes before the
+ * max_plies draw and runs on fast plies of the playout cap as well.  A
+ * calibration game keeps each colour's lowest r and, when it ends with a
+ * winner, counts itself, a false positive if the winner's lowest r is below
+ * the threshold, and the winner's lowest r in a histogram (AZ_BUF_RESIGN).
+ * The false positives bound the rate of wrong resignations from above: the
+ * loser might have resigned first.  Draws and failed games are not counted.
+ * threshold <= -1 turns it off; disable_prob = 1 measures without resigning.
+ * AZ_E_INVALID for a NaN threshold or one above 1, or for disable_prob
+ * outside [0, 1].  Read at launch time like the window (set it before
+ * capturing a graph).  Off: every other buffer is byte for byte what it is
+ * without this call. */
+int az_engine_set_resign(az_engine *e, float threshold, float disable_prob);
 
 /* HexGame.reset + Policy.reset for the games whose mask byte is non-zero
  * (NULL = all), hex.py:47-49, policy.py:72-76, search_tree.py:59-71. */
