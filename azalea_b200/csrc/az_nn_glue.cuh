@@ -406,10 +406,11 @@ k_nn_tail(const uint16_t *__restrict__ y, long long N, int ld, int nfc2, int nn,
             const float v[2] = {__uint_as_float(w << 16), __uint_as_float(w & 0xffff0000u)};
 #pragma unroll
             for (int h = 0; h < 2; h++) {
+                // the last pair of an odd nfc2 + nn ends one column past the row: bias has
+                // only nfc2 + nn elements, so it is read for real columns only
                 const int c = 2 * c2 + h;
-                const float x = v[h] + bias[c];
-                if (c < nfc2) part = fmaf(fmaxf(x, 0.f), w3[c], part);
-                else if (c < nfc2 + nn && logits) logits[b * logits_stride + (c - nfc2)] = x;
+                if (c < nfc2) part = fmaf(fmaxf(v[h] + bias[c], 0.f), w3[c], part);
+                else if (c < nfc2 + nn && logits) logits[b * logits_stride + (c - nfc2)] = v[h] + bias[c];
             }
         }
         for (int off = 16; off; off >>= 1) part += __shfl_xor_sync(0xffffffffu, part, off);

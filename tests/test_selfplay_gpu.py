@@ -688,8 +688,10 @@ def test_tcgen05_evaluator_against_reference_network_golden():
     """The whole bf16 evaluator on our kernels (stem, tcgen05 tower, heads)
     against the outputs of the REFERENCE's HexNetwork on the same seeded
     weights and boards (tests/golden/network.npz, generated by importing
-    azalea.network): value within 0.03, log-probabilities of the legal moves
-    within 0.15 (bf16 activations through 13 layers)."""
+    azalea.network): value within 2e-3, log-probabilities of the legal moves
+    within 4e-3, about twice what a B200 measures (7.7e-4 / 1.9e-3; bf16
+    activations through 13 layers).  A dropped bias of the FC layers or the
+    stem moves these outputs by 0.013 or more."""
     import os
     from azalea_b200.network import HexNetwork
     g = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'network.npz'))
@@ -710,12 +712,12 @@ def test_tcgen05_evaluator_against_reference_network_golden():
     cells = torch.zeros(B, 128, dtype=torch.int8, device='cuda')
     cells[:, :121] = torch.from_numpy(board.reshape(B, 121).astype(np.int8)).cuda()
     value, logits = net.evaluate_cells(cells)
-    assert np.abs(value.cpu().numpy() - g['value']).max() < 0.03
+    assert np.abs(value.cpu().numpy() - g['value']).max() < 2e-3
     for i in range(B):
         k = int((moves[i] > 0).sum())
         idx = torch.from_numpy(moves[i, :k].astype(np.int64) - 1).cuda()
         logp = torch.log_softmax(logits[i, idx], 0).cpu().numpy()
-        assert np.abs(logp - g['moves_logprob'][i, :k]).max() < 0.15, i
+        assert np.abs(logp - g['moves_logprob'][i, :k]).max() < 4e-3, i
 
 
 @pytest.mark.parametrize('streams', (2, 3))
