@@ -112,6 +112,7 @@ def lib():
     L.az_engine_set_reflect.argtypes = [eng, C.c_int]
     L.az_engine_set_playout_cap.argtypes = [eng, C.c_float, C.c_int]
     L.az_engine_set_resign.argtypes = [eng, C.c_float, C.c_float]
+    L.az_engine_set_forced_playouts.argtypes = [eng, C.c_float, C.c_float]
     L.az_status.argtypes = [eng, i32p, vp]
     L.az_stub_eval.argtypes = [eng, C.c_int, vp]
     L.az_replay_collate.argtypes = [vp, C.c_int, vp, C.c_int, C.c_int, i32p, i32p,

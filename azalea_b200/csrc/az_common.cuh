@@ -63,6 +63,8 @@ struct az_engine {
     int resign_on;          // 1: resignation / calibration bookkeeping on (az_engine_set_resign)
     float resign_thresh;    // the mover resigns iff r < resign_thresh
     unsigned long long calib_thresh;    // a game is a calibration game iff its coin < calib_thresh
+    float forced_k;         // != 0: forced playouts and policy target pruning on (az_engine_set_forced_playouts)
+    float prune_coef;       // the search's c_puct, for the pruning's PUCT scores
     int cell_stride;        // bytes per leaf board row (nn rounded up to 16)
     int path_stride;        // uint32 per descent path
     int row_bytes;          // replay row
@@ -273,6 +275,27 @@ __device__ __forceinline__ bool az_calibration_game(const az_engine &e, const in
     const uint2 key = make_uint2((uint32_t)e.cfg.seed ^ (uint32_t)meta[M_GID_LO],
                                  (uint32_t)(e.cfg.seed >> 32) ^ (uint32_t)meta[M_GID_HI]);
     return (unsigned long long)az_philox(make_uint4(0u, 0u, 0u, AZ_RESIGN_DOMAIN), key).x < e.calib_thresh;
+}
+
+// The most-visited of the root's k children {N, W, P, link} at nodes[fc..], lowest ordinal on
+// ties; k when none has a visit.  N >= 0, so the float order is the bit order.
+__device__ __forceinline__ int az_most_visited(const uint4 *nodes, int fc, int k, int lane)
+{
+    uint32_t nmax = 0u;
+    for (int j = lane; j < k; j += 32) nmax = max(nmax, nodes[fc + j].x);
+    nmax = __reduce_max_sync(AZ_FULL, nmax);
+    if (nmax == 0u) return k;
+    uint32_t best = (uint32_t)k;
+    for (int j = lane; j < k; j += 32)
+        if (nodes[fc + j].x == nmax) best = min(best, (uint32_t)j);
+    return (int)__reduce_min_sync(AZ_FULL, best);
+}
+
+// Forced playouts (az_engine_set_forced_playouts): n_forced = sqrt(k * P * sum N), one rounding
+// per operation, from the child's stored prior
+__device__ __forceinline__ float az_forced_visits(float k, float prior, float sum_n)
+{
+    return __fsqrt_rn(__fmul_rn(__fmul_rn(k, prior), sum_n));
 }
 
 __device__ __forceinline__ float az_u01(uint32_t r)     // (0,1)

@@ -476,6 +476,33 @@ __device__ __forceinline__ void az_finish_game(const az_engine &e, const az_play
     if (p.auto_reset) az_game_reset(e, g, meta, lane, true);
 }
 
+// Policy target pruning: the PUCT score of a root child {N, W, P, link} as if it had n visits, with
+// k_select's operation order and zero shortcut.  Q keeps the child's real N: the paper holds the
+// utility estimate constant.
+__device__ __forceinline__ float az_prune_score(uint4 c, float sq, float coef, float n)
+{
+    const float nv = __uint_as_float(c.x), tv = __uint_as_float(c.y);
+    const float q = tv == 0.0f ? 0.0f : __fdiv_rn(-tv, fmaxf(nv, 1.0f));
+    return __fadd_rn(q, __fmul_rn(__fmul_rn(coef, __uint_as_float(c.z)), __fdiv_rn(sq, __fadd_rn(1.0f, n))));
+}
+
+// The pruned count of a visited child other than the most-visited one: the fewest visits n' that
+// still score below the most-visited child's s_best, but at least N - floor(n_forced) and at most
+// N; one left at 1 becomes 0.  The score falls with n' (every rounding is monotone), so a
+// bisection finds the same n' as a scan.
+__device__ __forceinline__ float az_pruned_visits(uint4 c, float sq, float sum_n, float s_best,
+                                                  float coef, float k)
+{
+    const float nv = __uint_as_float(c.x);
+    const float d = floorf(az_forced_visits(k, __uint_as_float(c.z), sum_n));
+    int lo = d >= nv ? 0 : (int)nv - (int)d, hi = (int)nv;
+    while (lo < hi) {
+        const int mid = (lo + hi) >> 1;
+        if (az_prune_score(c, sq, coef, (float)mid) < s_best) hi = mid; else lo = mid + 1;
+    }
+    return lo == 1 ? 0.0f : (float)lo;
+}
+
 __global__ void __launch_bounds__(AZ_WARPS_PER_CTA * 32)
 k_play_commit(az_engine e, az_play_params p, int32_t *chosen)
 {
@@ -515,21 +542,11 @@ k_play_commit(az_engine e, az_play_params p, int32_t *chosen)
     // r = max(Q_root, Q_best) for the player to move.  A node's W is from the view of the
     // player to move there, so Q_best = -W/N of the most-visited child (lowest ordinal on ties).
     if (e.resign_on) {
-        uint32_t nmax = 0u;                 // N >= 0: the float order is the bit order
-        for (int s = 0; s < nslots; s++) {
-            const int j = lane + 32 * s;
-            if (j < k) nmax = max(nmax, nodes[fc + j].x);
-        }
-        nmax = __reduce_max_sync(AZ_FULL, nmax);
+        const int best = az_most_visited(nodes, fc, k, lane);
         const uint4 root = nodes[0];
         float r = __fdiv_rn(__uint_as_float(root.y), __uint_as_float(root.x));
-        if (nmax != 0u) {
-            uint32_t best = (uint32_t)k;
-            for (int s = 0; s < nslots; s++) {
-                const int j = lane + 32 * s;
-                if (j < k && nodes[fc + j].x == nmax) best = min(best, (uint32_t)j);
-            }
-            const uint4 c = nodes[fc + __reduce_min_sync(AZ_FULL, best)];
+        if (best < k) {
+            const uint4 c = nodes[fc + best];
             r = fmaxf(r, -__fdiv_rn(__uint_as_float(c.y), __uint_as_float(c.x)));
         }
         const int color = meta[M_COLOR];
@@ -661,8 +678,33 @@ k_play_commit(az_engine e, az_play_params p, int32_t *chosen)
             if (t < e.cell_stride) cells[t] = (int8_t)(((xs >> lane) & 1u) + 2u * ((os >> lane) & 1u));
         }
         float *vis = reinterpret_cast<float *>(row + sizeof(az_row_header) + e.cell_stride);
-        for (int j = lane; j < e.nn; j += 32)
-            vis[j] = j < k ? __uint_as_float(nodes[fc + j].x) : 0.0f;
+        if (e.forced_k != 0.0f && !fast) {
+            // policy target pruning (Wu 2019, section 3.2): the row gets the visits PUCT would
+            // have given without forced playouts; the move above was drawn from the raw ones
+            const int best = az_most_visited(nodes, fc, k, lane);
+            int ni = 0;
+            for (int j = lane; j < k; j += 32) ni += (int)__uint_as_float(nodes[fc + j].x);
+            const float sum_n = (float)__reduce_add_sync(AZ_FULL, ni);
+            const float sq = __fsqrt_rn(sum_n);
+            float s_best = 0.0f;
+            if (best < k) {
+                const uint4 c = nodes[fc + best];
+                s_best = az_prune_score(c, sq, e.prune_coef, __uint_as_float(c.x));
+            }
+            for (int j = lane; j < e.nn; j += 32) {
+                float v = 0.0f;
+                if (j < k) {
+                    const uint4 c = nodes[fc + j];
+                    v = __uint_as_float(c.x);
+                    if (j != best && v > 0.0f)
+                        v = az_pruned_visits(c, sq, sum_n, s_best, e.prune_coef, e.forced_k);
+                }
+                vis[j] = v;
+            }
+        } else {
+            for (int j = lane; j < e.nn; j += 32)
+                vis[j] = j < k ? __uint_as_float(nodes[fc + j].x) : 0.0f;
+        }
     }
     __syncwarp();
 
@@ -1128,6 +1170,15 @@ int az_engine_set_resign(az_engine *e, float threshold, float disable_prob)
     e->resign_thresh = e->resign_on ? threshold : 0.0f;
     // coin < p * 2^32 for an integer coin is coin < ceil(p * 2^32); exact in double
     e->calib_thresh = e->resign_on ? (unsigned long long)ceil((double)disable_prob * 4294967296.0) : 0ull;
+    return AZ_OK;
+}
+
+int az_engine_set_forced_playouts(az_engine *e, float k, float exploration_coef)
+{
+    if (!e || !(k >= 0.0f) || !isfinite(k) || !(exploration_coef >= 0.0f) || !isfinite(exploration_coef))
+        return AZ_E_INVALID;
+    e->forced_k = k;
+    e->prune_coef = k != 0.0f ? exploration_coef : 0.0f;
     return AZ_OK;
 }
 

@@ -324,6 +324,10 @@ k_select(az_engine e, az_select_args a)
             if (mix)
                 az_dirichlet_noise<MAXS>(lane, k, (float)a.noise_alpha, (uint32_t)(sim0 + b),
                                          (uint32_t)ply, key, noise);
+            // forced playouts (az_engine_set_forced_playouts): at the root of a full ply a child
+            // with 0 < N < sqrt(k P sum N) scores +inf; warp-uniform, like mix
+            const bool force = e.forced_k != 0.0f &&
+                               (NOISE ? mix : depth == 0 && az_full_search(e, meta));
             uint32_t bestkey = 0;
             int bestj = 0x7fffffff;
             // sum N == 0 (first descent into a freshly expanded node): every
@@ -356,6 +360,10 @@ k_select(az_engine e, az_select_args a)
                     float q = __fdiv_rn(tv_zero ? 1.0f : -tv, fmaxf(nv, 1.0f));
                     q = tv_zero ? 0.0f : q;
                     score = __fadd_rn(q, __fmul_rn(cp, gap));
+                    // (an unvisited child is never forced: the other branch needs no test)
+                    if (force && nv > 0.0f &&
+                        nv < az_forced_visits(e.forced_k, __uint_as_float(rec[s].z), (float)sum_n))
+                        score = INFINITY;
                 } else {
                     score = __fmul_rn(cp, sq);
                 }

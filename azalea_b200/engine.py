@@ -251,6 +251,16 @@ class Engine:
         t = -1.0 if threshold is None else float(threshold)
         check(self.lib.az_engine_set_resign(self._h, t, float(disable_prob)))
 
+    def set_forced_playouts(self, k=0.0, exploration_coef=0.5):
+        """Forced playouts and policy target pruning (Wu 2019, section 3.2;
+        az_engine_set_forced_playouts): on full plies a visited root child
+        with fewer than sqrt(k * P * sum N) visits is descended into first,
+        and the replay row's visits are pruned back to what PUCT with
+        ``exploration_coef`` would have given; the move is still drawn from
+        the raw visits.  ``k=0`` is off.  Read at launch time: set it before
+        capturing a graph."""
+        check(self.lib.az_engine_set_forced_playouts(self._h, float(k), float(exploration_coef)))
+
     def resign_stats(self):
         """Resignation counts summed over the slots (one D2H copy):
         ``resigned_games``, ``calibration_games`` (calibration games that

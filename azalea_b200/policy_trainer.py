@@ -34,7 +34,12 @@ Deviations from the reference, all on purpose:
   (default 0.1) turn on resignation (AlphaGo Zero) in the self-play refills:
   the player to move resigns when its root value is below the threshold,
   except in calibration games, which never resign and measure how often the
-  eventual winner would have; the refill metrics report both (rank 0's games).
+  eventual winner would have; the refill metrics report both (rank 0's games);
+* ``forced_playouts_k`` (default 0.0, off; the paper uses 2) turns on forced
+  playouts and policy target pruning (Wu 2019, section 3.2) in the self-play
+  refills: at the root of a full search a visited child with fewer than
+  sqrt(k * P * sum N) visits is searched again, and the recorded policy
+  targets lose the visits that PUCT would not have given on its own.
 """
 import logging
 import os
@@ -209,11 +214,13 @@ def train(policy, config, rundir, *,
     num_games = int(config.get('num_selfplay_games', 1024))
 
     # playout cap randomization: a self-play setting, not part of the policy (not checkpointed)
-    # resignation (AlphaGo Zero) likewise: a data-generation setting, not checkpointed
+    # resignation (AlphaGo Zero) and forced playouts (Wu 2019) likewise: data-generation
+    # settings, not checkpointed
     cap = dict(full_search_prob=float(config.get('full_search_prob', 1.0)),
                fast_simulations=config.get('fast_simulations'),
                resign_threshold=config.get('resign_threshold'),
-               resign_disable_prob=float(config.get('resign_disable_prob', 0.1)))
+               resign_disable_prob=float(config.get('resign_disable_prob', 0.1)),
+               forced_playouts_k=float(config.get('forced_playouts_k', 0.0)))
 
     game_class = _game_class(config['game'])
     game_factory = partial(game_class, board_size=config['board_size'])

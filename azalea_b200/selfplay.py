@@ -18,6 +18,8 @@ Philox stream is keyed by its global id, so results do not depend on the
 world size.  The only exchange is the replay gather to rank 0.
 """
 
+import math
+
 import numpy as np
 import torch
 
@@ -93,6 +95,20 @@ def resign_setting(threshold, disable_prob):
     return None if t <= -1.0 else t
 
 
+def forced_playouts_setting(k, exploration_coef):
+    """Validated forced-playouts constant ``k`` (0.0 = off).
+
+    Raises ``ValueError`` for a negative or non-finite ``k`` or
+    ``exploration_coef`` (the coefficient the pruning scores with).
+    """
+    k, coef = float(k), float(exploration_coef)
+    if not (k >= 0.0 and math.isfinite(k)):
+        raise ValueError(f'forced_playouts_k must be a finite number >= 0, got {k!r}')
+    if not (coef >= 0.0 and math.isfinite(coef)):
+        raise ValueError(f'exploration_coef must be a finite number >= 0, got {coef!r}')
+    return k
+
+
 def resign_threshold_for(hist, calib_games, max_fp_rate):
     """The highest resignation threshold whose estimated false-positive
     rate is at most ``max_fp_rate``, from ``Engine.resign_stats()``.
@@ -134,7 +150,7 @@ class LockstepSelfPlay:
                  replay_rows=None, collect_replay=True, cuda_graph=True,
                  max_plies=300, random_play=False, streams=None, pack_leaves=None,
                  random_reflect=False, full_search_prob=1.0, fast_simulations=None,
-                 resign_threshold=None, resign_disable_prob=0.1):
+                 resign_threshold=None, resign_disable_prob=0.1, forced_playouts_k=0.0):
         # random_play: RandomPolicy self-play (random_policy.py:25-41) -- no
         # search, uniform move choice and uniform moves_prob at every ply;
         # how the reference fills the replay buffer before training
@@ -161,6 +177,10 @@ class LockstepSelfPlay:
         self.resign_threshold = None if self.random_play else resign_setting(
             resign_threshold, resign_disable_prob)
         self.resign_disable_prob = float(resign_disable_prob)
+        # forced playouts and policy target pruning (Wu 2019, section 3.2): 0.0 = off
+        # (az_engine_set_forced_playouts)
+        self.forced_playouts_k = 0.0 if self.random_play else forced_playouts_setting(
+            forced_playouts_k, exploration_coef)
         self.coef = float(exploration_coef)
         self.depth = int(exploration_depth)
         self.temperature = float(exploration_temperature)
@@ -201,6 +221,8 @@ class LockstepSelfPlay:
             self.eng.set_playout_cap(full_search_prob, self.fast_descents)
         if self.resign_threshold is not None:
             self.eng.set_resign(self.resign_threshold, self.resign_disable_prob)
+        if self.forced_playouts_k:
+            self.eng.set_forced_playouts(self.forced_playouts_k, self.coef)
         self.device = self.eng.device
         self.chosen = torch.zeros(self.G, 4, dtype=torch.int32,
                                   device=self.device)
@@ -303,11 +325,14 @@ class LockstepSelfPlay:
         subtrees at different times, as in steady-state self-play.  Eager;
         call it before the move graph is captured or between replays.  Nobody
         resigns on these plies: a uniform root says nothing about the
-        position."""
+        position, and their rows are not pruned: every child of a uniform
+        root has one visit, which pruning would take away."""
         eng, G = self.eng, self.G
         max_plies = int(max_plies)
         if self.resign_threshold is not None:
             eng.set_resign(None)
+        if self.forced_playouts_k:
+            eng.set_forced_playouts(0.0)
         try:
             for s in range(1, max_plies + 1):
                 g0 = -(-s * G // max_plies)         # slots with quota >= s
@@ -324,6 +349,8 @@ class LockstepSelfPlay:
             eng.set_window(0, 0)
             if self.resign_threshold is not None:
                 eng.set_resign(self.resign_threshold, self.resign_disable_prob)
+            if self.forced_playouts_k:
+                eng.set_forced_playouts(self.forced_playouts_k, self.coef)
 
     def capture(self):
         """Capture one move as a CUDA graph (capturing does not execute)."""

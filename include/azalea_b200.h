@@ -249,6 +249,28 @@ int az_engine_set_playout_cap(az_engine *e, float full_search_prob, int fast_des
  * without this call. */
 int az_engine_set_resign(az_engine *e, float threshold, float disable_prob);
 
+/* Forced playouts and policy target pruning (Wu 2019, "Accelerating
+ * Self-Play Learning in Go", section 3.2), off by default.  Forcing: on full
+ * plies (every ply unless the playout cap is on), az_mcts_select gives a root
+ * child with 0 < N < n_forced = sqrt(k * P * sum N) the score +inf, so the
+ * lowest such ordinal is descended into; sum N is the children's visit sum
+ * including the batch's virtual losses, and P is the child's stored prior, not
+ * the noised one (the noise is drawn per simulation), in f32 with one rounding
+ * per operation.  Root mode and fast plies never force.  Pruning: on full
+ * plies az_play_commit, after the move has been drawn from the raw visits,
+ * writes pruned visits into the ply's replay row: with c* the most-visited
+ * child (lowest ordinal on ties) and score(c, n) = Q_c + (exploration_coef *
+ * P_c) * (sqrt(sum N) / (1 + n)) in az_mcts_select's operation order (Q_c
+ * from the child's real N), every other visited child keeps the fewest n that
+ * still score below score(c*, N*), but at least N - floor(n_forced) and at
+ * most N, and one left at 1 visit gets 0.  The tree, the move, chosen_dev,
+ * resignation and every counter see the raw visits.  k == 0 turns it off;
+ * AZ_E_INVALID for a negative or non-finite k or exploration_coef, which
+ * should be the coefficient az_mcts_select is launched with.  Read at launch
+ * time like the window (set it before capturing a graph).  Off: every buffer
+ * is byte for byte what it is without this call. */
+int az_engine_set_forced_playouts(az_engine *e, float k, float exploration_coef);
+
 /* HexGame.reset + Policy.reset for the games whose mask byte is non-zero
  * (NULL = all), hex.py:47-49, policy.py:72-76, search_tree.py:59-71. */
 int az_games_reset(az_engine *e, const uint8_t *mask_dev, void *stream);
