@@ -1,13 +1,22 @@
-/* Forced playouts at the root (Wu 2019, "Accelerating Self-Play Learning in
- * Go", section 3.2; az_engine_set_forced_playouts) for the CPU oracle.  TEST
- * INFRASTRUCTURE ONLY.
+/* The two root rules of the engine's search for the CPU oracle: forced
+ * playouts (Wu 2019, "Accelerating Self-Play Learning in Go", section 3.2;
+ * az_engine_set_forced_playouts) and Dirichlet root noise (mcts.py:126-131).
+ * TEST INFRASTRUCTURE ONLY.
  *
- * omcts_select_batch_forced is omcts_select_batch (azalea_oracle.c,
- * mcts.py:46-76) with one rule added at the root: with forced_k != 0 a root
- * child with 0 < N < sqrtf((forced_k * P) * sum N) scores +inf, so np.argmax
- * takes the lowest such ordinal.  P is the stored prior; N and sum N include
- * the batch's virtual losses.  float32, one rounding per operation.  With
- * forced_k = 0 both entry points are bit for bit the oracle's own (tested).
+ * select_batch below is omcts_select_batch (azalea_oracle.c, mcts.py:46-76)
+ * with both rules added at the root:
+ *  - root noise: with noise != NULL and noise_scale != 0, descent i of the
+ *    call scores the root's children with P'[j] = (float)((1 - eps) * (double)
+ *    P[j] + eps * (double)noise[i][j]), mixed in double (k_select), where the
+ *    noise array is [batch][k_root].  The noise vectors are given, not drawn:
+ *    the device's own draws (Engine.noise_sample) make the search comparable
+ *    bit for bit;
+ *  - forced playouts: with forced_k != 0 a root child with 0 < N <
+ *    sqrtf((forced_k * P) * sum N) scores +inf, so np.argmax takes the lowest
+ *    such ordinal.  P is the stored prior, not the noised one; N and sum N
+ *    include the batch's virtual losses.
+ * float32 otherwise, one rounding per operation.  With forced_k = 0 and no
+ * noise every entry point is bit for bit the oracle's own (tested).
  * Everything else goes through the oracle's exported functions: this file is
  * linked against libazalea_oracle.so and works on its trees. */
 #include "azalea_oracle.h"
@@ -44,14 +53,32 @@ static void leaf_state(const ohex *g, oleaves *out, int slot)
     }
 }
 
-int omcts_select_batch_forced(otree *t, const ohex *game, int batch_size,
-                              float coef, float forced_k, oleaves *out)
+/* How the root noise is mixed into the prior: OMIX_F64 is the engine's rule.
+ * The float32 variants exist only so that a test can ask whether a search
+ * would notice a kernel that mixed in float32. */
+enum { OMIX_F64 = 0, OMIX_F32 = 1, OMIX_F32_FMA = 2 };
+
+static float mix_prior(float p, float eta, double eps, int mix)
+{
+    if (mix == OMIX_F32)
+        return (1.0f - (float)eps) * p + (float)eps * eta;
+    if (mix == OMIX_F32_FMA)
+        return fmaf((float)eps, eta, (1.0f - (float)eps) * p);
+    return (float)((1.0 - eps) * (double)p + eps * (double)eta);
+}
+
+static int select_batch(otree *t, const ohex *game, int batch_size, float coef,
+                        float forced_k, double noise_scale, const float *noise,
+                        int mix, oleaves *out)
 {
     int32_t leaf_nodes[OMAX_BATCH];
     static __thread ohex leaf_games[OMAX_BATCH];
-    float nv[19 * 19], ntv[19 * 19], pr[19 * 19], score[19 * 19];
-    if (batch_size > OMAX_BATCH || t->num_children[t->root_id] <= 0)
+    float nv[19 * 19], ntv[19 * 19], pr[19 * 19], pm[19 * 19], score[19 * 19];
+    const int32_t k_root = t->num_children[t->root_id];
+    if (batch_size > OMAX_BATCH || k_root <= 0)
         return -1;
+    if (noise_scale == 0.0)
+        noise = NULL;
     out->sum_children = 0;
     out->sum_depth = 0;
     for (int i = 0; i < batch_size; i++) {
@@ -66,7 +93,14 @@ int omcts_select_batch_forced(otree *t, const ohex *game, int batch_size,
                 ntv[j] = -t->total_value[fc + j];
                 pr[j] = t->prior_prob[fc + j];
             }
-            omcts_score_actions(nv, ntv, pr, k, coef, score);
+            if (noise && node == t->root_id) {
+                const float *eta = noise + (size_t)i * k_root;
+                for (int j = 0; j < k; j++)
+                    pm[j] = mix_prior(pr[j], eta[j], noise_scale, mix);
+                omcts_score_actions(nv, ntv, pm, k, coef, score);
+            } else {
+                omcts_score_actions(nv, ntv, pr, k, coef, score);
+            }
             if (forced_k != 0.0f && node == t->root_id) {
                 double s = 0;           /* sum of small integers: exact */
                 for (int j = 0; j < k; j++)
@@ -109,6 +143,20 @@ int omcts_select_batch_forced(otree *t, const ohex *game, int batch_size,
     return out->count;
 }
 
+int omcts_select_batch_forced(otree *t, const ohex *game, int batch_size,
+                              float coef, float forced_k, oleaves *out)
+{
+    return select_batch(t, game, batch_size, coef, forced_k, 0.0, NULL, OMIX_F64, out);
+}
+
+/* Both root rules; noise is [batch_size][k_root] (may be NULL). */
+int omcts_select_batch_noise(otree *t, const ohex *game, int batch_size,
+                             float coef, float forced_k, double noise_scale,
+                             const float *noise, int mix, oleaves *out)
+{
+    return select_batch(t, game, batch_size, coef, forced_k, noise_scale, noise, mix, out);
+}
+
 static void eval_stub(const oleaves *lv, int n, int mode, float *value,
                       float *prior, int stride)
 {
@@ -122,12 +170,14 @@ static void eval_stub(const oleaves *lv, int n, int mode, float *value,
     }
 }
 
-/* omcts_sample_paths_stub (mcts.py:258-293) with the forced select.
- * Returns -1 on SearchTreeFull. */
-int omcts_sample_paths_stub_forced(otree *t, const ohex *game,
-                                   int num_simulations, int batch_size,
-                                   float coef, float forced_k, int stub_mode,
-                                   float *search_value)
+/* omcts_sample_paths_stub (mcts.py:258-293) with both root rules: the
+ * call's b-th select uses noise rows b * batch_size .. b * batch_size +
+ * batch_size - 1 of noise[num_batches * batch_size][k_root].  Returns -1 on
+ * SearchTreeFull. */
+static int sample_paths_stub(otree *t, const ohex *game, int num_simulations,
+                             int batch_size, float coef, float forced_k,
+                             double noise_scale, const float *noise, int mix,
+                             int stub_mode, float *search_value)
 {
     int num_batches = num_simulations / batch_size + 1;
     int stride = 19 * 19;
@@ -150,7 +200,8 @@ int omcts_sample_paths_stub_forced(otree *t, const ohex *game,
     }
     for (int b = 0; b < num_batches; b++) {
         float sv;
-        rc = omcts_select_batch_forced(t, game, batch_size, coef, forced_k, lv);
+        const float *rows = noise ? noise + (size_t)b * batch_size * t->num_children[t->root_id] : NULL;
+        rc = select_batch(t, game, batch_size, coef, forced_k, noise_scale, rows, mix, lv);
         if (rc < 0)
             goto done;
         eval_stub(lv, game->n, stub_mode, value, prior, stride);
@@ -166,4 +217,23 @@ done:
     free(lv);
     free(prior);
     return rc;
+}
+
+int omcts_sample_paths_stub_forced(otree *t, const ohex *game,
+                                   int num_simulations, int batch_size,
+                                   float coef, float forced_k, int stub_mode,
+                                   float *search_value)
+{
+    return sample_paths_stub(t, game, num_simulations, batch_size, coef, forced_k, 0.0, NULL,
+                             OMIX_F64, stub_mode, search_value);
+}
+
+int omcts_sample_paths_stub_noise(otree *t, const ohex *game,
+                                  int num_simulations, int batch_size,
+                                  float coef, float forced_k, double noise_scale,
+                                  const float *noise, int mix, int stub_mode,
+                                  float *search_value)
+{
+    return sample_paths_stub(t, game, num_simulations, batch_size, coef, forced_k, noise_scale,
+                             noise, mix, stub_mode, search_value);
 }

@@ -8,36 +8,16 @@ import torch
 
 import oracle
 from oracle import forced, stubs
+from oracle.philox import full_ply, game_ids, philox, philox_key
 from oracle.pruning import prune_visits
 
 gpu = pytest.mark.gpu
-M32 = 0xFFFFFFFF
-FULL_SEARCH_DOMAIN = 0xCA9F5EA7
 MOVE_DOMAIN = 0xC0111700
-
-
-def philox(c, k):
-    """Philox4x32-10 as az_philox (az_common.cuh)."""
-    c, k = list(c), list(k)
-    for _ in range(10):
-        p0, p1 = 0xD2511F53 * c[0], 0xCD9E8D57 * c[2]
-        c = [((p1 >> 32) ^ c[1] ^ k[0]) & M32, p1 & M32, ((p0 >> 32) ^ c[3] ^ k[1]) & M32, p0 & M32]
-        k = [(k[0] + 0x9E3779B9) & M32, (k[1] + 0xBB67AE85) & M32]
-    return c
-
-
-def _key(seed, game_id):
-    return ((seed ^ game_id) & M32, ((seed >> 32) ^ (game_id >> 32)) & M32)
-
-
-def full_ply(seed, game_id, ply, p):
-    thresh = np.ceil(np.float64(np.float32(p)) * 2.0 ** 32)
-    return philox((ply, 0, 0, FULL_SEARCH_DOMAIN), _key(seed, game_id))[0] < thresh
 
 
 def move_at_temperature_1(v, seed, game_id, ply):
     """k_play_commit's inverse CDF over integer weights: exact in any order."""
-    x = philox((0, 0, ply, MOVE_DOMAIN), _key(seed, game_id))[0]
+    x = philox((0, 0, ply, MOVE_DOMAIN), philox_key(seed, game_id))[0]
     w = v.astype(np.float64)
     tot = w.sum()
     target = tot * ((x + 0.5) * (1.0 / 4294967296.0))
@@ -49,11 +29,6 @@ def move_at_temperature_1(v, seed, game_id, ply):
 
 def bits(a):
     return np.ascontiguousarray(a, dtype=np.float32).tobytes()
-
-
-def game_ids(eng):
-    meta = eng.meta.cpu().numpy().astype(np.int64)
-    return (meta[:, 10] & M32) | (meta[:, 11] << 32), meta[:, 4].copy()
 
 
 def stub_selfplay(moves, G=64, n=5, seed=3, graph=False, streams=None, **kw):

@@ -8,28 +8,10 @@ import torch
 
 import oracle
 from oracle import stubs
+from oracle.philox import full_ply, game_ids
 
 gpu = pytest.mark.gpu
 AZ_PRIOR_LOGITS = 1
-M32 = 0xFFFFFFFF
-FULL_SEARCH_DOMAIN = 0xCA9F5EA7
-
-
-def philox(c, k):
-    """Philox4x32-10 as az_philox (az_common.cuh)."""
-    c, k = list(c), list(k)
-    for _ in range(10):
-        p0, p1 = 0xD2511F53 * c[0], 0xCD9E8D57 * c[2]
-        c = [((p1 >> 32) ^ c[1] ^ k[0]) & M32, p1 & M32, ((p0 >> 32) ^ c[3] ^ k[1]) & M32, p0 & M32]
-        k = [(k[0] + 0x9E3779B9) & M32, (k[1] + 0xBB67AE85) & M32]
-    return c
-
-
-def full_ply(seed, game_id, ply, p):
-    """The full-search coin of (seed, global game id, ply)."""
-    key = ((seed ^ game_id) & M32, ((seed >> 32) ^ (game_id >> 32)) & M32)
-    return philox((ply, 0, 0, FULL_SEARCH_DOMAIN), key)[0] < np.ceil(np.float64(np.float32(p)) * 2.0 ** 32)
-
 
 def bits(a):
     return np.ascontiguousarray(a, dtype=np.float32).tobytes()
@@ -46,11 +28,6 @@ def random_positions(G, n, rng):
         boards[g, tiles[1::2]] = 2
         colors[g] = 1 if p % 2 == 0 else 2
     return boards, colors
-
-
-def game_ids(eng):
-    meta = eng.meta.cpu().numpy().astype(np.int64)
-    return (meta[:, 10] & M32) | (meta[:, 11] << 32), meta[:, 4].copy()
 
 
 def stub_selfplay(moves, G=64, n=5, seed=3, graph=False, **kw):

@@ -8,38 +8,15 @@ import torch
 
 import oracle
 from oracle import stubs
+from oracle.philox import M32, full_ply, philox, philox_key, threshold
 
 gpu = pytest.mark.gpu
-M32 = 0xFFFFFFFF
 RESIGN_DOMAIN = 0x2E51C0A1
-FULL_SEARCH_DOMAIN = 0xCA9F5EA7
-
-
-def philox(c, k):
-    """Philox4x32-10 as az_philox (az_common.cuh)."""
-    c, k = list(c), list(k)
-    for _ in range(10):
-        p0, p1 = 0xD2511F53 * c[0], 0xCD9E8D57 * c[2]
-        c = [((p1 >> 32) ^ c[1] ^ k[0]) & M32, p1 & M32, ((p0 >> 32) ^ c[3] ^ k[1]) & M32, p0 & M32]
-        k = [(k[0] + 0x9E3779B9) & M32, (k[1] + 0xBB67AE85) & M32]
-    return c
-
-
-def _key(seed, game_id):
-    return ((seed ^ game_id) & M32, ((seed >> 32) ^ (game_id >> 32)) & M32)
-
-
-def _thresh(p):
-    return np.ceil(np.float64(np.float32(p)) * 2.0 ** 32)
 
 
 def calibration_game(seed, game_id, p):
     """The calibration coin of (seed, global game id)."""
-    return philox((0, 0, 0, RESIGN_DOMAIN), _key(seed, game_id))[0] < _thresh(p)
-
-
-def full_ply(seed, game_id, ply, p):
-    return philox((ply, 0, 0, FULL_SEARCH_DOMAIN), _key(seed, game_id))[0] < _thresh(p)
+    return philox((0, 0, 0, RESIGN_DOMAIN), philox_key(seed, game_id))[0] < threshold(p)
 
 
 def resign_value(v, w, k, root_nw):
