@@ -11,6 +11,7 @@ reference (tests/golden/make_golden.py, tests/test_oracle_golden.py).
 import ctypes as C
 import os
 import subprocess
+import zlib
 
 import numpy as np
 
@@ -19,6 +20,13 @@ _LIB_PATH = os.path.join(_HERE, 'build', 'libazalea_oracle.so')
 
 MAXT = 19 * 19
 OMAX_BATCH = 64
+# the board sizes of tests/golden/hex_rules.npz
+HEX_SIZES = (2, 3, 4, 5, 7, 9, 11, 13, 19)
+
+
+def crc(a):
+    """The checksum tests/golden/hex_rules.npz records legal-move lists by."""
+    return zlib.crc32(np.ascontiguousarray(a, dtype=np.int32).tobytes())
 
 
 class OHex(C.Structure):

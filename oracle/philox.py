@@ -8,6 +8,8 @@ import numpy as np
 
 M32 = 0xFFFFFFFF
 FULL_SEARCH_DOMAIN = 0xCA9F5EA7
+RESIGN_DOMAIN = 0x2E51C0A1
+MOVE_DOMAIN = 0xC0111700
 
 
 def philox(c, k):
@@ -33,6 +35,23 @@ def threshold(p):
 def full_ply(seed, game_id, ply, p):
     """The playout cap's full-search coin of (seed, global game id, ply)."""
     return philox((ply, 0, 0, FULL_SEARCH_DOMAIN), philox_key(seed, game_id))[0] < threshold(p)
+
+
+def calibration_game(seed, game_id, p):
+    """The resignation calibration coin of (seed, global game id)."""
+    return philox((0, 0, 0, RESIGN_DOMAIN), philox_key(seed, game_id))[0] < threshold(p)
+
+
+def move_at_temperature_1(v, seed, game_id, ply):
+    """k_play_commit's inverse CDF over integer weights: exact in any order."""
+    x = philox((0, 0, ply, MOVE_DOMAIN), philox_key(seed, game_id))[0]
+    w = v.astype(np.float64)
+    tot = w.sum()
+    target = tot * ((x + 0.5) * (1.0 / 4294967296.0))
+    hit = np.flatnonzero((w > 0) & (np.cumsum(w) > target))
+    if len(hit):
+        return int(hit[0])
+    return int(np.flatnonzero(w > 0)[-1])
 
 
 def game_ids(eng):

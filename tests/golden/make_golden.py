@@ -13,7 +13,6 @@ script.  Nothing here is used at test time except the files it wrote.
 """
 import os
 import sys
-import zlib
 
 import numpy as np
 
@@ -31,13 +30,9 @@ import azalea as az  # noqa: E402
 from azalea import mcts, search_tree  # noqa: E402
 from azalea.game import hex as refhex  # noqa: E402
 from azalea.game.hex import HexGame  # noqa: E402
-from oracle import stubs  # noqa: E402
+from oracle import crc, stubs  # noqa: E402
 
 _REAL_EVALUATE_BATCH = mcts.evaluate_batch
-
-
-def crc(a):
-    return zlib.crc32(np.ascontiguousarray(a, dtype=np.int32).tobytes())
 
 
 # ------------------------------------------------------------------ hex ----

@@ -5,6 +5,7 @@ import pytest
 import torch
 
 import oracle
+from oracle.lockstep import bits
 
 pytestmark = pytest.mark.gpu
 
@@ -93,10 +94,6 @@ def search_policy(sims, batch, coef, mode, sampling=False):
     p.exploration_noise_alpha, p.exploration_noise_scale = 0.03, 0.25
     p.settings['move_sampling'] = sampling
     return p
-
-
-def bits(a):
-    return np.ascontiguousarray(a, dtype=np.float32).tobytes()
 
 
 def test_lockstep_seats_match_oracle_trees():

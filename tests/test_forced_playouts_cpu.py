@@ -45,7 +45,6 @@ def test_random_play_ignores_forced_playouts():
 def test_abi_surface():
     from azalea_b200 import _cabi
     assert 'az_engine_set_forced_playouts' in _cabi.declared_symbols()
-    assert len(_cabi.COUNTER_NAMES) == 16
 
 
 # --------------------------------------------------------- the forced rule --

@@ -8,40 +8,13 @@ import torch
 
 import oracle
 from oracle import forced, stubs
-from oracle.philox import full_ply, game_ids, philox, philox_key
+from oracle.lockstep import (assert_root_matches, assert_same_games, assert_streams_and_graphs_agree,
+                             bits, check_replay_buffer, network, selfplay_fingerprint, selfplay_player,
+                             stub_search, stub_selfplay, train_config)
+from oracle.philox import full_ply, game_ids, move_at_temperature_1
 from oracle.pruning import prune_visits
 
 gpu = pytest.mark.gpu
-MOVE_DOMAIN = 0xC0111700
-
-
-def move_at_temperature_1(v, seed, game_id, ply):
-    """k_play_commit's inverse CDF over integer weights: exact in any order."""
-    x = philox((0, 0, ply, MOVE_DOMAIN), philox_key(seed, game_id))[0]
-    w = v.astype(np.float64)
-    tot = w.sum()
-    target = tot * ((x + 0.5) * (1.0 / 4294967296.0))
-    hit = np.flatnonzero((w > 0) & (np.cumsum(w) > target))
-    if len(hit):
-        return int(hit[0])
-    return int(np.flatnonzero(w > 0)[-1])
-
-
-def bits(a):
-    return np.ascontiguousarray(a, dtype=np.float32).tobytes()
-
-
-def stub_selfplay(moves, G=64, n=5, seed=3, graph=False, streams=None, **kw):
-    from azalea_b200 import LockstepSelfPlay, StubEvaluator
-    sp = LockstepSelfPlay(StubEvaluator(stubs.ROUGH), num_games=G, board_size=n, simulations=30,
-                          search_batch_size=4, seed=seed, cuda_graph=graph, exploration_depth=4,
-                          streams=streams, **kw)
-    chosen = []
-    for _ in range(moves):
-        sp.step_move()
-        chosen.append(sp.chosen.cpu().numpy().copy())
-    assert (sp.eng.status().cpu().numpy() == 0).all()
-    return sp, np.stack(chosen)
 
 
 def rows_by_game(rows, n):
@@ -64,12 +37,7 @@ def test_forced_playouts_off_is_byte_identical(n):
                               search_batch_size=4, seed=3, cuda_graph=False)
         if off is not None:
             sp.eng.set_forced_playouts(*off)
-        chosen = []
-        for _ in range(30):
-            sp.step_move()
-            chosen.append(sp.chosen.cpu().numpy().copy())
-        out.append((np.stack(chosen).tobytes(), sp.harvest().tobytes(),
-                    sp.eng.counters.cpu().numpy().tobytes(), sp.eng.meta.cpu().numpy().tobytes()))
+        out.append(selfplay_fingerprint(sp, 30))
     assert len(out[0][1]) > 0
     assert all(o == out[0] for o in out[1:])
 
@@ -100,14 +68,8 @@ def test_forcing_matches_the_oracle(n, G, plies, cap):
         if done.all():
             break
         gid, ply = game_ids(eng)
-        eng.select_root()
-        eng.stub_eval(mode)
-        eng.expand_root()
-        for _ in range(num_batches):
-            eng.select(batch, coef)
-            eng.stub_eval(mode)
-            eng.expand_backup()
-        v, w, p, k, rnw, nodes = (x.cpu().numpy() for x in eng.root_stats())
+        stub_search(eng, mode, batch, coef, num_batches)
+        stats = [x.cpu().numpy() for x in eng.root_stats()]
         eng.play_commit(0.0, 0, False, False, False, chosen)
         ch = chosen.cpu().numpy()
         for g in np.flatnonzero(~done):
@@ -115,14 +77,7 @@ def test_forcing_matches_the_oracle(n, G, plies, cap):
             g_sims = sims if full else fast_sims
             forced.sample_paths_stub(trees[g], games[g], g_sims, batch, coef, mode, fk if full else 0.0)
             plain[g].sample_paths_stub(games[g], g_sims, batch, coef, mode)
-            ov, ow, op = trees[g].root_stats()
-            kg = int(k[g])
-            where = (g, int(ply[g]), full)
-            assert bits(v[g, :kg]) == bits(ov), where
-            assert bits(w[g, :kg]) == bits(ow), where
-            assert bits(p[g, :kg]) == bits(op), where
-            assert bits(rnw[g]) == bits(trees[g].root_node()), where
-            assert int(nodes[g]) == trees[g].num_nodes, where
+            ov = assert_root_matches(stats, g, trees[g], (g, int(ply[g]), full))
             if full:
                 full_plies += 1
                 differ += bits(plain[g].root_stats()[0]) != bits(ov)
@@ -159,13 +114,7 @@ def test_pruned_rows_match_numpy(noise):
     moves_checked = 0
     for _ in range(60):
         gid, ply = game_ids(eng)
-        eng.select_root()
-        eng.stub_eval(mode)
-        eng.expand_root()
-        for _ in range(num_batches):
-            eng.select(batch, coef, 0.25 if noise else 0.0, 0.03)
-            eng.stub_eval(mode)
-            eng.expand_backup()
+        stub_search(eng, mode, batch, coef, num_batches, 0.25 if noise else 0.0, 0.03)
         v, w, p, k, _, _ = (x.cpu().numpy() for x in eng.root_stats())
         eng.play_commit(1.0, depth, True, True, True, chosen)
         ch = chosen.cpu().numpy()
@@ -243,22 +192,11 @@ def test_forced_playouts_invariance():
     kw = dict(forced_playouts_k=2.0, full_search_prob=0.5, fast_simulations=5)
 
     def play(streams, graph, **more):
-        sp, chosen = stub_selfplay(40, streams=streams, graph=graph, **kw, **more)
+        sp, _, _, chosen = stub_selfplay(40, streams=streams, graph=graph, **kw, **more)
         return chosen, sp.harvest(), sp.counters()
-    c0, r0, n0 = play(1, False)
+    r0 = assert_streams_and_graphs_agree(play)[1]
     assert len(r0) > 0
-    for streams, graph in ((2, False), (2, True), (1, True)):
-        c1, r1, n1 = play(streams, graph)
-        assert np.array_equal(c0, c1) and r0.tobytes() == r1.tobytes() and n0 == n1
-    parts = [play(1, False, G=32, rank=r, world_size=2) for r in range(2)]
-    _, _, whole = rows_by_game(r0, 5)
-    seen = 0
-    for part in parts:
-        _, _, index = rows_by_game(part[1], 5)
-        for key, i in index.items():
-            assert r0[whole[key]].tobytes() == part[1][i].tobytes()
-            seen += 1
-    assert seen == len(whole) > 0
+    assert_same_games(r0, [play(1, False, G=32, rank=r, world_size=2)[1] for r in range(2)])
 
 
 @gpu
@@ -266,15 +204,8 @@ def test_forced_playouts_with_the_network():
     """6x64 network in the loop, packed leaves, two streams, a CUDA graph,
     preroll: rows go through rows_to_dataframe, DeviceReplayBuffer and
     Player.read, and every engine status stays 0."""
-    import azalea_b200 as az
     from azalea_b200 import LockstepSelfPlay
-    from azalea_b200.network import HexNetwork
-    from azalea_b200.parallel_player import Player
-    from azalea_b200.replay_device import DeviceReplayBuffer
-    from azalea_b200.selfplay import rows_to_dataframe
-    torch.manual_seed(0)
-    net = HexNetwork(5, 6, 64).eval().cuda()
-    net.prepare_inference(torch.bfloat16)
+    net = network(6)
     sp = LockstepSelfPlay(net, num_games=128, board_size=5, simulations=40, search_batch_size=8,
                           seed=5, streams=2, cuda_graph=True, forced_playouts_k=2.0)
     assert sp.pack_leaves and sp.streams == 2
@@ -285,20 +216,9 @@ def test_forced_playouts_with_the_network():
     assert (sp.eng.status().cpu().numpy() == 0).all()
     rows = sp.harvest()
     assert len(rows) > 0
-    df = rows_to_dataframe(rows, 5)
-    assert len(df) == len(rows)
-    buf = DeviceReplayBuffer(len(rows) + 7, 5)
-    buf.put(torch.from_numpy(rows).cuda())
-    batch = buf.sample(64, generator=torch.Generator(device='cuda').manual_seed(4))
-    assert np.allclose(batch['moves_prob'].sum(1).cpu().numpy(), 1.0, atol=1e-5)
+    check_replay_buffer(rows)
 
-    pol = az.Policy()
-    pol.net = net
-    pol.simulations, pol.search_batch_size, pol.exploration_coef = 40, 8, 0.5
-    pol.exploration_depth, pol.exploration_temperature = 4, 1.0
-    pol.exploration_noise_alpha, pol.exploration_noise_scale = 0.03, 0.25
-    agent = az.AzaleaAgent(lambda: az.HexGame(5), policy=pol)
-    player = Player(None, [agent], num_games=64, seed=3, forced_playouts_k=2.0)
+    player = selfplay_player(net, 40, 8, forced_playouts_k=2.0)
     assert player.sp.forced_playouts_k == 2.0
     examples, metrics = player.read(200)
     assert len(examples) >= 200
@@ -318,14 +238,7 @@ def test_train_with_forced_playouts(tmp_path, monkeypatch):
             super().__init__(*a, **kw)
             made.append(self)
     monkeypatch.setattr(policy_trainer, 'Player', Recording)
-    config = dict(seed=3, device='cuda', game='hex', network='HexNetwork', board_size=5,
-                  num_blocks=1, base_chans=64, simulations=10, search_batch_size=5,
-                  exploration_coef=0.5, exploration_temperature=1.0, exploration_depth=15,
-                  exploration_noise_alpha=0.03, exploration_noise_scale=0.25,
-                  replaybuf_size=256, replaybuf_oversampling=1, batch_size=128, lr_initial=0.01,
-                  lr_decay_steps=100, lr_decay=0.5, momentum=0.9, l2_regularization=1e-4,
-                  total_steps=4, log_interval=0, model_checkpoint_interval=0,
-                  num_selfplay_games=32, forced_playouts_k=2)
+    config = train_config(forced_playouts_k=2)
     policy = az.Policy()
     policy.initialize(config)
     buf = policy_trainer.initialize_replay_buffer(None, lambda: az.HexGame(5), 256, num_games=32,

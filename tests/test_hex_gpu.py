@@ -1,20 +1,13 @@
 """GPU parity: Hex rules in the CUDA engine vs the reference's golden vectors
 and vs the C oracle.  Everything goes through the C ABI (Engine)."""
-import zlib
-
 import numpy as np
 import pytest
 import torch
 
 import oracle
+from oracle import HEX_SIZES, crc
 
 pytestmark = pytest.mark.gpu
-
-HEX_SIZES = (2, 3, 4, 5, 7, 9, 11, 13, 19)
-
-
-def crc(a):
-    return zlib.crc32(np.ascontiguousarray(a, dtype=np.int32).tobytes())
 
 
 def make_engine(G, n, **kw):

@@ -8,12 +8,9 @@ import torch
 import oracle
 from oracle import dirichlet_stats as ds
 from oracle import stubs
+from oracle.lockstep import assert_root_matches, bits, stub_search
 
 pytestmark = pytest.mark.gpu
-
-
-def bits(a):
-    return np.ascontiguousarray(a, dtype=np.float32).tobytes()
 
 
 class GpuTree:
@@ -183,31 +180,16 @@ def test_lockstep_games_vs_oracle(n, G, sims, batch, coef, mode, plies):
     trees = [oracle.Tree(max_nodes=3_000_000) for _ in range(G)]
     alive = np.ones(G, dtype=bool)
     for ply in range(plies):
-        eng.select_root()
-        eng.stub_eval(mode)
-        eng.expand_root()
-        for _ in range(sims // batch + 1):
-            eng.select(batch, coef)
-            eng.stub_eval(mode)
-            eng.expand_backup()
-        v, w, p, k, rnw, nodes = (x.cpu().numpy() for x in eng.root_stats())
+        stub_search(eng, mode, batch, coef, sims // batch + 1)
+        stats = [x.cpu().numpy() for x in eng.root_stats()]
         assert (eng.status().cpu().numpy()[alive] == 0).all()
         move_ids = -np.ones(G, dtype=np.int32)
         moves = np.zeros(G, dtype=np.int32)
         for gi in np.flatnonzero(alive):
             trees[gi].sample_paths_stub(games[gi], sims, batch, coef, mode)
-            ov, ow, op = trees[gi].root_stats()
-            kk = len(ov)
-            where = (ply, gi)
-            assert k[gi] == kk, where
-            assert bits(v[gi, :kk]) == bits(ov), where
-            assert bits(w[gi, :kk]) == bits(ow), where
-            assert bits(p[gi, :kk]) == bits(op), where
-            rn, rw = trees[gi].root_node()
-            assert bits(rnw[gi]) == bits([rn, rw]), where
-            assert nodes[gi] == trees[gi].num_nodes, where
+            ov = assert_root_matches(stats, gi, trees[gi], (ply, gi))
             order = np.argsort(-ov, kind='stable')
-            mid = int(order[(gi + ply) % min(kk, 3)])
+            mid = int(order[(gi + ply) % min(len(ov), 3)])
             move_ids[gi] = mid
             moves[gi] = games[gi].legal_moves()[mid]
             trees[gi].move(mid)
@@ -247,9 +229,7 @@ def test_search_tree_full_is_raised():
 def test_pool_overflow_is_flagged_not_corrupting():
     from azalea_b200 import Engine, _cabi
     eng = Engine(4, 11, max_batch=10, nodes_per_game=2000)
-    eng.select_root(); eng.stub_eval(0); eng.expand_root()
-    for _ in range(40):
-        eng.select(10, 0.5); eng.stub_eval(0); eng.expand_backup()
+    stub_search(eng, 0, 10, 0.5, 40)
     st = eng.status().cpu().numpy()
     assert (st == _cabi.AZ_ST_POOL_FULL).all()
     v, _, _, k, _, _ = eng.root_stats()
@@ -265,9 +245,7 @@ def test_soft_pool_full_skips_expansions_and_keeps_the_game():
     resumes.  Whole games finish with games_failed == 0."""
     from azalea_b200 import Engine, LockstepSelfPlay, StubEvaluator
     eng = Engine(4, 11, max_batch=10, nodes_per_game=2000, soft_pool_full=True)
-    eng.select_root(); eng.stub_eval(2); eng.expand_root()
-    for _ in range(40):
-        eng.select(10, 0.5); eng.stub_eval(2); eng.expand_backup()
+    stub_search(eng, 2, 10, 0.5, 40)
     assert (eng.status().cpu().numpy() == 0).all()
     cnt = eng.counter_totals()
     assert cnt['pool_skipped_expansions'] > 0
@@ -316,10 +294,7 @@ def test_dirichlet_noise_statistics():
     from azalea_b200 import Engine
     G = 64
     eng = Engine(G, 11, max_batch=10, seed=5)
-    eng.select_root(); eng.stub_eval(0); eng.expand_root()
-    for _ in range(30):
-        eng.select(10, 2.0, noise_scale=0.25, noise_alpha=0.03)
-        eng.stub_eval(0); eng.expand_backup()
+    stub_search(eng, 0, 10, 2.0, 30, eps=0.25, alpha=0.03)
     v = eng.root_stats()[0].cpu().numpy()
     # duplicate leaves inside a batch are backed up once (mcts.py:75)
     assert (v.sum(1) <= 300).all() and (v.sum(1) >= 280).all()
@@ -375,9 +350,7 @@ def test_deep_search_19x19_vs_oracle():
     games = [oracle.Hex(n) for _ in range(G)]
     trees = [oracle.Tree(max_nodes=8_000_000) for _ in range(G)]
     for ply in range(3):
-        eng.select_root(); eng.stub_eval(mode); eng.expand_root()
-        for _ in range(sims // batch + 1):
-            eng.select(batch, coef); eng.stub_eval(mode); eng.expand_backup()
+        stub_search(eng, mode, batch, coef, sims // batch + 1)
         v, w, p, k, rnw, nodes = (x.cpu().numpy() for x in eng.root_stats())
         assert (eng.status().cpu().numpy() == 0).all()
         move_ids = np.zeros(G, dtype=np.int32)

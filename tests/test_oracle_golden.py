@@ -1,18 +1,10 @@
 """Pin the C oracle against fixtures generated from the Python reference
 (tests/golden/make_golden.py).  CPU only."""
-import zlib
-
 import numpy as np
 import pytest
 
 import oracle
-from oracle import stubs
-
-HEX_SIZES = (2, 3, 4, 5, 7, 9, 11, 13, 19)
-
-
-def crc(a):
-    return zlib.crc32(np.ascontiguousarray(a, dtype=np.int32).tobytes())
+from oracle import HEX_SIZES, crc, stubs
 
 
 @pytest.mark.parametrize('n', HEX_SIZES)

@@ -72,10 +72,11 @@ def make_rows(games, n=3):
 
 
 class FakeSelfPlay:
-    """One harvest of canned rows; counters as the engine would report."""
+    """Canned harvests; counters and resignation counts as the engine would
+    report them, advancing by one step's worth per move."""
 
-    def __init__(self, rows, fast):
-        self.rows, self.fast, self.moves = rows, fast, 0
+    def __init__(self, rows, fast=0, resign=None):
+        self.rows, self.fast, self.resign, self.moves = rows, fast, resign or {}, 0
         outer = self
 
         class Eng:
@@ -90,8 +91,10 @@ class FakeSelfPlay:
         return self.rows
 
     def counters(self):
-        return {'fast_plies': self.fast if self.moves else 0, 'games_failed': 0,
-                'pool_skipped_expansions': 0}
+        return {'fast_plies': self.fast * self.moves, 'games_failed': 0, 'pool_skipped_expansions': 0}
+
+    def resign_stats(self):
+        return {k: v * self.moves for k, v in self.resign.items()}
 
 
 def test_player_read_counts_games_by_id():

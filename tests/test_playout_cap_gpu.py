@@ -7,50 +7,14 @@ import pytest
 import torch
 
 import oracle
+from azalea_b200._cabi import AZ_PRIOR_LOGITS
 from oracle import stubs
+from oracle.lockstep import (assert_root_matches, assert_same_games, assert_streams_and_graphs_agree,
+                             check_replay_buffer, network, random_positions, selfplay_fingerprint,
+                             selfplay_player, stub_search, stub_selfplay, train_config)
 from oracle.philox import full_ply, game_ids
 
 gpu = pytest.mark.gpu
-AZ_PRIOR_LOGITS = 1
-
-def bits(a):
-    return np.ascontiguousarray(a, dtype=np.float32).tobytes()
-
-
-def random_positions(G, n, rng):
-    """Mid-game positions that cannot be won yet (X has fewer than n stones)."""
-    boards = np.zeros((G, n * n), np.int8)
-    colors = np.zeros(G, np.int32)
-    for g in range(G):
-        p = rng.randint(1, 2 * (n - 1) + 1)
-        tiles = rng.permutation(n * n)[:p]
-        boards[g, tiles[0::2]] = 1
-        boards[g, tiles[1::2]] = 2
-        colors[g] = 1 if p % 2 == 0 else 2
-    return boards, colors
-
-
-def stub_selfplay(moves, G=64, n=5, seed=3, graph=False, **kw):
-    """Stub self-play, recording per move and slot the game id, the ply and
-    the descents of the move (simulations counter delta), and the games that
-    finished with their length and result."""
-    from azalea_b200 import LockstepSelfPlay, StubEvaluator
-    sp = LockstepSelfPlay(StubEvaluator(stubs.ROUGH), num_games=G, board_size=n, simulations=30,
-                          search_batch_size=4, seed=seed, cuda_graph=graph, exploration_depth=4, **kw)
-    plies, finished, chosen = {}, {}, []
-    for _ in range(moves):
-        gid, ply = game_ids(sp.eng)
-        sims0 = sp.eng.counters[:, 0].cpu().numpy().copy()
-        sp.step_move()
-        desc = sp.eng.counters[:, 0].cpu().numpy() - sims0
-        ch = sp.chosen.cpu().numpy().copy()
-        chosen.append(ch)
-        for g in range(G):
-            plies[(int(gid[g]), int(ply[g]))] = int(desc[g])
-            if ch[g, 2] != 0:
-                finished[int(gid[g])] = (int(ch[g, 3]), int(ch[g, 2]))
-    assert (sp.eng.status().cpu().numpy() == 0).all()
-    return sp, plies, finished, np.stack(chosen)
 
 
 # ------------------------------------------------------------------ tests --
@@ -65,12 +29,7 @@ def test_cap_off_is_byte_identical(n):
     for kw in ({}, dict(full_search_prob=1.0)):
         sp = LockstepSelfPlay(StubEvaluator(stubs.ROUGH), num_games=64, board_size=n, simulations=20,
                               search_batch_size=4, seed=3, cuda_graph=False, **kw)
-        chosen = []
-        for _ in range(30):
-            sp.step_move()
-            chosen.append(sp.chosen.cpu().numpy().copy())
-        out.append((np.stack(chosen).tobytes(), sp.harvest().tobytes(),
-                    sp.eng.counters.cpu().numpy().tobytes(), sp.eng.meta.cpu().numpy().tobytes()))
+        out.append(selfplay_fingerprint(sp, 30))
     assert len(out[0][1]) > 0
     assert out[0] == out[1]
 
@@ -100,15 +59,9 @@ def test_fast_and_full_plies_match_the_oracle():
         gid, ply = game_ids(eng)
         sims0 = eng.counters[:, 0].cpu().numpy().copy()
         fast0 = int(eng.counters[:, 15].sum())
-        eng.select_root()
-        eng.stub_eval(mode)
-        eng.expand_root()
-        for _ in range(num_batches):
-            eng.select(batch, coef)
-            eng.stub_eval(mode)
-            eng.expand_backup()
+        stub_search(eng, mode, batch, coef, num_batches)
         desc = eng.counters[:, 0].cpu().numpy() - sims0
-        v, w, p, k, rnw, nodes = (x.cpu().numpy() for x in eng.root_stats())
+        stats = [x.cpu().numpy() for x in eng.root_stats()]
         eng.play_commit(0.0, 0, False, False, False, chosen)
         ch = chosen.cpu().numpy()
         fast_now = 0
@@ -118,14 +71,8 @@ def test_fast_and_full_plies_match_the_oracle():
             counts[int(desc[g])] += 1
             fast_now += not full
             trees[g].sample_paths_stub(games[g], sims if full else fast_sims, batch, coef, mode)
-            ov, ow, op = trees[g].root_stats()
-            kg = int(k[g])
             where = (g, int(ply[g]))
-            assert bits(v[g, :kg]) == bits(ov), where
-            assert bits(w[g, :kg]) == bits(ow), where
-            assert bits(p[g, :kg]) == bits(op), where
-            assert bits(rnw[g]) == bits(trees[g].root_node()), where
-            assert int(nodes[g]) == trees[g].num_nodes, where
+            ov = assert_root_matches(stats, g, trees[g], where)
             mid = int(ch[g, 1])
             assert ov[mid] == ov.max(), where
             trees[g].move(mid)
@@ -154,13 +101,7 @@ def test_fast_plies_draw_no_noise():
             eng = Engine(G, n, max_batch=B, seed=seed, nodes_per_game=65536)
             eng.set_playout_cap(p, 3 * B)
             eng.hex_set_state(boards, colors)
-            eng.select_root()
-            eng.stub_eval(stubs.ROUGH)
-            eng.expand_root()
-            for _ in range(3):
-                eng.select(B, 0.5, eps, 0.03)
-                eng.stub_eval(stubs.ROUGH)
-                eng.expand_backup()
+            stub_search(eng, stubs.ROUGH, B, 0.5, 3, eps, 0.03)
             assert int(eng.counters[:, 0].sum()) == G * 3 * B
             stats.append([x.cpu().numpy() for x in eng.root_stats()])
         same = all(np.array_equal(a, b) for a, b in zip(*stats))
@@ -176,8 +117,6 @@ def test_replay_holds_exactly_the_full_plies():
     through rows_to_dataframe and DeviceReplayBuffer, and Player.read counts
     games and moves right when a game's first or last ply left no row."""
     from azalea_b200.engine import decode_replay_rows
-    from azalea_b200.replay_device import DeviceReplayBuffer
-    from azalea_b200.selfplay import rows_to_dataframe
     sp, plies, finished, _ = stub_selfplay(60, full_search_prob=0.5, fast_simulations=5)
     full_d, fast_d = 32, 8
     assert set(plies.values()) <= {0, fast_d, full_d}
@@ -190,41 +129,24 @@ def test_replay_holds_exactly_the_full_plies():
         if gid in finished and ply < finished[gid][0]:
             assert d == (full_d if full_ply(3, gid, ply, 0.5) else fast_d)
     fast_finished = sum(1 for (gid, ply), d in plies.items() if gid in finished and d == fast_d)
-    assert len(h) + fast_finished == sum(length for length, _ in finished.values())
+    assert len(h) + fast_finished == sum(f[0] for f in finished.values())
     assert sp.counters()['replay_rows'] == len(h)
     for i in range(len(h)):
-        length, result = finished[int(h['game_id'][i])]
+        length, result, _ = finished[int(h['game_id'][i])]
         assert h['game_len'][i] == length and h['result'][i] == result
         rw = np.float32(result - 2)
         assert h['reward'][i] == (-rw if h['ply'][i] % 2 else rw)
         assert h['reserved'][i] == 0
     # games whose first / last ply was fast are in the sample
     first = {gid for gid in finished if (gid, 0) not in got}
-    last = {gid for gid, (length, _) in finished.items() if (gid, length - 1) not in got}
+    last = {gid for gid, (length, _, _) in finished.items() if (gid, length - 1) not in got}
     assert first and last
-    df = rows_to_dataframe(rows, 5)
-    assert len(df) == len(h)
-    buf = DeviceReplayBuffer(len(h) + 7, 5)
-    buf.put(torch.from_numpy(rows).cuda())
-    gen = torch.Generator(device='cuda').manual_seed(4)
-    batch = buf.sample(64, generator=gen)
-    idx = torch.randint(0, len(buf), (64,), device='cuda',
-                        generator=torch.Generator(device='cuda').manual_seed(4)).cpu().numpy()
-    assert np.array_equal(batch['reward'].cpu().numpy(), h['reward'][idx])
-    assert np.array_equal(batch['color'].cpu().numpy(), h['color'][idx])
-    assert np.allclose(batch['moves_prob'].sum(1).cpu().numpy(), 1.0, atol=1e-5)
+    check_replay_buffer(rows)
 
     # Player.read: games by id, lengths from game_len
-    import azalea_b200 as az
-    from azalea_b200.parallel_player import Player
-    pol = az.Policy()
-    pol.net = az.StubEvaluator(stubs.ROUGH)
-    pol.simulations, pol.search_batch_size, pol.exploration_coef = 30, 4, 0.5
-    pol.exploration_depth, pol.exploration_temperature = 4, 1.0
-    pol.exploration_noise_alpha, pol.exploration_noise_scale = 0.03, 0.25
-    agent = az.AzaleaAgent(lambda: az.HexGame(5), policy=pol)
-    player = Player(None, [agent], num_games=64, seed=3, cuda_graph=False,
-                    full_search_prob=0.5, fast_simulations=5)
+    from azalea_b200 import StubEvaluator
+    player = selfplay_player(StubEvaluator(stubs.ROUGH), 30, 4, cuda_graph=False,
+                             full_search_prob=0.5, fast_simulations=5)
     assert player.sp.fast_descents == fast_d
     seen = []
     harvest = player.sp.harvest
@@ -247,11 +169,7 @@ def test_cap_selfplay_invariance():
     eager vs graphed give the same moves and replay bytes; with the stub,
     2 ranks x 32 games play the games 1 rank x 64 plays."""
     from azalea_b200 import LockstepSelfPlay
-    from azalea_b200.engine import decode_replay_rows
-    from azalea_b200.network import HexNetwork
-    torch.manual_seed(0)
-    net = HexNetwork(5, 2, 64).eval().cuda()
-    net.prepare_inference(torch.bfloat16)
+    net = network(2)
 
     def play(streams, graph):
         sp = LockstepSelfPlay(net, num_games=64, board_size=5, simulations=40, search_batch_size=8,
@@ -264,29 +182,13 @@ def test_cap_selfplay_invariance():
             chosen.append(sp.chosen.cpu().numpy().copy())
         assert (sp.eng.status().cpu().numpy() == 0).all()
         return np.stack(chosen), sp.harvest(), sp.counters()
-    c0, r0, n0 = play(1, False)
+    _, r0, n0 = assert_streams_and_graphs_agree(play)
     assert len(r0) > 0 and 0 < n0['fast_plies'] < n0['plies']
-    for streams, graph in ((2, False), (2, True), (1, True)):
-        c1, r1, n1 = play(streams, graph)
-        assert np.array_equal(c0, c1) and r0.tobytes() == r1.tobytes() and n0 == n1
 
     whole = stub_selfplay(40, full_search_prob=0.5, fast_simulations=5)[0].harvest()
     parts = [stub_selfplay(40, G=32, rank=r, world_size=2, full_search_prob=0.5,
                            fast_simulations=5)[0].harvest() for r in range(2)]
-    hw = decode_replay_rows(whole, 5)[0]
-    by_id = {}
-    for i, gid in enumerate(hw['game_id']):
-        by_id.setdefault(int(gid), []).append(i)
-    seen = 0
-    for part in parts:
-        hp = decode_replay_rows(part, 5)[0]
-        games = {}
-        for i, gid in enumerate(hp['game_id']):
-            games.setdefault(int(gid), []).append(i)
-        for gid, idx in games.items():
-            assert whole[by_id[gid]].tobytes() == part[idx].tobytes()
-            seen += 1
-    assert seen == len(by_id) > 0
+    assert_same_games(whole, parts)
 
 
 @gpu
@@ -334,14 +236,7 @@ def test_train_with_playout_cap(tmp_path):
     import azalea_b200 as az
     from azalea_b200 import policy_trainer
     from azalea_b200.engine import decode_replay_rows
-    config = dict(seed=3, device='cuda', game='hex', network='HexNetwork', board_size=5,
-                  num_blocks=1, base_chans=64, simulations=10, search_batch_size=5,
-                  exploration_coef=0.5, exploration_temperature=1.0, exploration_depth=15,
-                  exploration_noise_alpha=0.03, exploration_noise_scale=0.25,
-                  replaybuf_size=256, replaybuf_oversampling=1, batch_size=128, lr_initial=0.01,
-                  lr_decay_steps=100, lr_decay=0.5, momentum=0.9, l2_regularization=1e-4,
-                  total_steps=4, log_interval=0, model_checkpoint_interval=0,
-                  num_selfplay_games=32, full_search_prob=0.5, fast_simulations=2)
+    config = train_config(full_search_prob=0.5, fast_simulations=2)
     policy = az.Policy()
     policy.initialize(config)
     buf = policy_trainer.initialize_replay_buffer(None, lambda: az.HexGame(5), 256, num_games=32,

@@ -7,10 +7,12 @@ import pytest
 import torch
 
 import oracle
+from azalea_b200._cabi import AZ_PRIOR_LOGITS
 from oracle import stubs
+from oracle.lockstep import (assert_same_games, assert_streams_and_graphs_agree, network, random_positions,
+                             train_config)
 
 gpu = pytest.mark.gpu
-AZ_PRIOR_LOGITS = 1
 
 
 def flip_tile(t, n):
@@ -68,19 +70,6 @@ def test_host_rotation_helper():
 
 
 # ------------------------------------------------------------------- GPU --
-
-def random_positions(G, n, rng):
-    """Mid-game positions that cannot be won yet (X has fewer than n stones)."""
-    boards = np.zeros((G, n * n), np.int8)
-    colors = np.zeros(G, np.int32)
-    for g in range(G):
-        p = rng.randint(1, 2 * (n - 1) + 1)
-        tiles = rng.permutation(n * n)[:p]
-        boards[g, tiles[0::2]] = 1
-        boards[g, tiles[1::2]] = 2
-        colors[g] = 1 if p % 2 == 0 else 2
-    return boards, colors
-
 
 def leaf_rows(eng, root):
     """{(g, b): (network row bytes, leaf_info)} of the rows the evaluator reads."""
@@ -286,39 +275,15 @@ def test_reflect_selfplay_invariance_with_network():
     """Reflect on, random-init HexNetwork: the coins follow the game's Philox
     stream, so one vs two streams and eager vs graphed are bit-identical, and
     2 ranks x 32 games play the games 1 rank x 64 plays."""
-    from azalea_b200.engine import decode_replay_rows
-    from azalea_b200.network import HexNetwork
-    torch.manual_seed(0)
-    net = HexNetwork(5, 2, 64).eval().cuda()
-    net.prepare_inference(torch.bfloat16)
-    c0, r0, n0 = play(net, True, 1, False)
+    net = network(2)
+    _, r0, n0 = assert_streams_and_graphs_agree(lambda streams, graph: play(net, True, streams, graph))
     assert n0['reflected_rows'] > 0
-    for streams, graph in ((2, False), (2, True), (1, True)):
-        c1, r1, n1 = play(net, True, streams, graph)
-        assert np.array_equal(c0, c1) and r0.tobytes() == r1.tobytes() and n0 == n1
     # and the orientation matters for a real network
     _, r_off, _ = play(net, False, 1, False)
     assert r_off.tobytes() != r0.tobytes()
     whole = play(net, True, 1, False, G=64, moves=25)[1]
     parts = [play(net, True, 1, False, G=32, moves=25, rank=r, world_size=2)[1] for r in range(2)]
-    hw, _, vw = decode_replay_rows(whole, 5)
-    first = {}
-    for i, gid in enumerate(hw['game_id']):
-        if gid < 64:
-            first.setdefault(int(gid), []).append(i)
-    seen = 0
-    for part in parts:
-        hp, _, vp = decode_replay_rows(part, 5)
-        games = {}
-        for i, gid in enumerate(hp['game_id']):
-            if gid < 64:
-                games.setdefault(int(gid), []).append(i)
-        for gid, idx in games.items():
-            ref = first[gid]
-            assert (hw['move'][ref] == hp['move'][idx]).all()
-            assert vw[ref].tobytes() == vp[idx].tobytes()
-            seen += 1
-    assert seen == len(first) > 0
+    assert_same_games(whole, parts)
 
 
 class RecordingHostNet:
@@ -462,14 +427,7 @@ def test_train_with_reflect_and_checkpoint_key(tmp_path):
     hex11-20180712-3362.policy.pth) loads with it off."""
     import azalea_b200 as az
     from azalea_b200 import policy_trainer
-    config = dict(seed=3, device='cuda', game='hex', network='HexNetwork', board_size=5,
-                  num_blocks=1, base_chans=64, simulations=10, search_batch_size=5,
-                  exploration_coef=0.5, exploration_temperature=1.0, exploration_depth=15,
-                  exploration_noise_alpha=0.03, exploration_noise_scale=0.25,
-                  replaybuf_size=256, replaybuf_oversampling=1, batch_size=128, lr_initial=0.01,
-                  lr_decay_steps=100, lr_decay=0.5, momentum=0.9, l2_regularization=1e-4,
-                  total_steps=4, log_interval=0, model_checkpoint_interval=0,
-                  num_selfplay_games=32, random_reflect=True)
+    config = train_config(random_reflect=True)
     policy = az.Policy()
     policy.initialize(config)
     assert policy.random_reflect

@@ -46,7 +46,6 @@ def test_abi_surface():
     assert 'az_engine_set_resign' in _cabi.declared_symbols()
     assert _cabi.AZ_BUF_RESIGN == 10
     assert _cabi.AZ_RS_HIST + _cabi.AZ_RS_BINS <= 72
-    assert len(_cabi.COUNTER_NAMES) == 16
 
 
 def test_resign_threshold_for():
@@ -74,46 +73,20 @@ def test_resign_threshold_for():
         resign_threshold_for(np.zeros(65), 0, 0.05)
 
 
-class FakeSelfPlay:
-    """Canned harvests; counters and resignation counts as the engine would
-    report them, advancing by one step's worth per move."""
-
-    def __init__(self, rows, step):
-        self.rows, self.step, self.moves = rows, step, 0
-        outer = self
-
-        class Eng:
-            def replay_count(self):
-                return len(outer.rows) if outer.moves else 0
-        self.eng = Eng()
-
-    def step_move(self):
-        self.moves += 1
-
-    def harvest(self):
-        return self.rows
-
-    def counters(self):
-        return {'fast_plies': 0, 'games_failed': 0, 'pool_skipped_expansions': 0}
-
-    def resign_stats(self):
-        return {k: v * self.moves for k, v in self.step.items()}
-
-
 def test_player_read_reports_resignation(caplog):
     from azalea_b200.parallel_player import Player
-    from test_playout_cap_cpu import make_rows
+    from test_playout_cap_cpu import FakeSelfPlay, make_rows
     rows = make_rows({5: (3, [0, 1, 2]), 7: (2, [0, 1])})
     player = Player.__new__(Player)
     player.board_size = 3
     player.resign = True
-    player.sp = FakeSelfPlay(rows, dict(resigned_games=4, calibration_games=20, false_positives=1))
+    player.sp = FakeSelfPlay(rows, resign=dict(resigned_games=4, calibration_games=20, false_positives=1))
     with caplog.at_level(logging.WARNING):
         _, metrics = player.read(1)
     assert metrics['resigned_games'] == 4
     assert metrics['resign_calibration_games'] == 20 and metrics['resign_false_positives'] == 1
     assert 'calibration games' not in caplog.text          # 5 %: not above the limit
-    player.sp = FakeSelfPlay(rows, dict(resigned_games=4, calibration_games=20, false_positives=2))
+    player.sp = FakeSelfPlay(rows, resign=dict(resigned_games=4, calibration_games=20, false_positives=2))
     with caplog.at_level(logging.WARNING):
         _, metrics = player.read(1)
     assert metrics['resign_false_positives'] == 2

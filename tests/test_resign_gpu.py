@@ -8,15 +8,12 @@ import torch
 
 import oracle
 from oracle import stubs
-from oracle.philox import M32, full_ply, philox, philox_key, threshold
+from oracle.lockstep import (assert_root_matches, assert_same_games, assert_streams_and_graphs_agree,
+                             bits, check_replay_buffer, network, selfplay_fingerprint, selfplay_player,
+                             stub_search, stub_selfplay, train_config)
+from oracle.philox import calibration_game, full_ply, game_ids
 
 gpu = pytest.mark.gpu
-RESIGN_DOMAIN = 0x2E51C0A1
-
-
-def calibration_game(seed, game_id, p):
-    """The calibration coin of (seed, global game id)."""
-    return philox((0, 0, 0, RESIGN_DOMAIN), philox_key(seed, game_id))[0] < threshold(p)
 
 
 def resign_value(v, w, k, root_nw):
@@ -31,37 +28,6 @@ def resign_value(v, w, k, root_nw):
 
 def hist_bin(m):
     return min(64, max(0, int(np.floor((np.float32(m) + np.float32(1)) * np.float32(64)))))
-
-
-def bits(a):
-    return np.ascontiguousarray(a, dtype=np.float32).tobytes()
-
-
-def game_ids(eng):
-    meta = eng.meta.cpu().numpy().astype(np.int64)
-    return (meta[:, 10] & M32) | (meta[:, 11] << 32), meta[:, 4].copy(), meta[:, 2].copy()
-
-
-def stub_selfplay(moves, G=64, n=5, seed=3, graph=False, streams=None, **kw):
-    """Stub self-play recording per move and slot the game id and ply, the
-    plies that were fast (playout cap), and the finished games with their
-    length, result and whether they ended by resignation."""
-    from azalea_b200 import LockstepSelfPlay, StubEvaluator
-    sp = LockstepSelfPlay(StubEvaluator(stubs.ROUGH), num_games=G, board_size=n, simulations=30,
-                          search_batch_size=4, seed=seed, cuda_graph=graph, exploration_depth=4,
-                          streams=streams, **kw)
-    finished, chosen = {}, []
-    for _ in range(moves):
-        gid, ply, _ = game_ids(sp.eng)
-        sp.step_move()
-        ch = sp.chosen.cpu().numpy().copy()
-        chosen.append(ch)
-        for g in range(G):
-            if ch[g, 2] > 0:
-                finished[int(gid[g])] = (int(ch[g, 3]), int(ch[g, 2]), bool(ch[g, 1] == -1))
-                assert ch[g, 3] == ply[g] + (ch[g, 1] != -1)
-    assert (sp.eng.status().cpu().numpy() == 0).all()
-    return sp, finished, np.stack(chosen)
 
 
 # A deterministic stub's values sit close to 0 at these search sizes (the search averages
@@ -83,12 +49,7 @@ def test_resign_off_is_byte_identical(n):
                               search_batch_size=4, seed=3, cuda_graph=False)
         if off is not None:
             sp.eng.set_resign(*off)
-        chosen = []
-        for _ in range(30):
-            sp.step_move()
-            chosen.append(sp.chosen.cpu().numpy().copy())
-        out.append((np.stack(chosen).tobytes(), sp.harvest().tobytes(),
-                    sp.eng.counters.cpu().numpy().tobytes(), sp.eng.meta.cpu().numpy().tobytes()))
+        out.append(selfplay_fingerprint(sp, 30))
         rs = sp.resign_stats()
         assert rs['resigned_games'] == rs['calibration_games'] == 0
     assert len(out[0][1]) > 0
@@ -123,28 +84,20 @@ def test_resign_decisions_match_the_oracle():
     for _ in range(n * n):
         if done.all():
             break
-        gid, ply, color = game_ids(eng)
+        gid, ply = game_ids(eng)
+        color = eng.meta[:, 2].cpu().numpy()          # the colour to move
         assert (gid == gid0).all()
-        eng.select_root()
-        eng.stub_eval(mode)
-        eng.expand_root()
-        for _ in range(num_batches):
-            eng.select(batch, coef)
-            eng.stub_eval(mode)
-            eng.expand_backup()
-        v, w, p, k, rnw, nodes = (x.cpu().numpy() for x in eng.root_stats())
+        stub_search(eng, mode, batch, coef, num_batches)
+        stats = [x.cpu().numpy() for x in eng.root_stats()]
+        v, w, _, k, rnw, _ = stats
         eng.play_commit(0.0, 0, False, False, False, chosen)
         ch = chosen.cpu().numpy()
         _, _, result, hply = (x.cpu().numpy() for x in eng.hex_state())
         for g in np.flatnonzero(~done):
             where = (g, int(ply[g]))
             trees[g].sample_paths_stub(games[g], sims, batch, coef, mode)
-            ov, ow, op = trees[g].root_stats()
-            kg = int(k[g])
-            assert bits(v[g, :kg]) == bits(ov), where
-            assert bits(w[g, :kg]) == bits(ow), where
-            assert bits(rnw[g]) == bits(trees[g].root_node()), where
-            r = resign_value(v[g], w[g], kg, rnw[g])
+            assert_root_matches(stats, g, trees[g], where)
+            r = resign_value(v[g], w[g], int(k[g]), rnw[g])
             c = int(color[g])
             if calib[g]:
                 mins[g, c - 1] = min(mins[g, c - 1], r)
@@ -198,13 +151,7 @@ def test_resign_value_sign_on_a_known_position():
     board[0, [1, 2]] = 2
     eng = Engine(G, n, max_batch=B, seed=1, nodes_per_game=4096)
     eng.hex_set_state(board, np.array([1], np.int32))
-    eng.select_root()
-    eng.stub_eval(stubs.UNIFORM)
-    eng.expand_root()
-    for _ in range(20):
-        eng.select(B, 0.5)
-        eng.stub_eval(stubs.UNIFORM)
-        eng.expand_backup()
+    stub_search(eng, stubs.UNIFORM, B, 0.5, 20)
     v, w, _, k, rnw, _ = (x.cpu().numpy() for x in eng.root_stats())
     kg = int(k[0])
     assert rnw[0, 1] / rnw[0, 0] > 0.3
@@ -220,13 +167,12 @@ def test_replay_of_resigned_games(cap):
     ply-parity rewards and reserved 0; natural endings are unchanged.  The
     rows go through rows_to_dataframe and DeviceReplayBuffer, and
     Player.read reports the resignation counts of its call."""
+    from azalea_b200 import StubEvaluator
     from azalea_b200.engine import decode_replay_rows
-    from azalea_b200.replay_device import DeviceReplayBuffer
-    from azalea_b200.selfplay import rows_to_dataframe
     capkw = dict(full_search_prob=0.5, fast_simulations=5) if cap else {}
     # 40 moves of 64 games record at most 2560 rows: the replay output (2 * 64 * 25 rows) holds
     # every finished game's rows until the one harvest below
-    sp, finished, _ = stub_selfplay(40, resign_threshold=STUB_THRESHOLD, resign_disable_prob=0.2, **capkw)
+    sp, _, finished, _ = stub_selfplay(40, resign_threshold=STUB_THRESHOLD, resign_disable_prob=0.2, **capkw)
     assert sp.counters()['replay_dropped'] == 0
     rows = sp.harvest()
     h, _, _ = decode_replay_rows(rows, 5)
@@ -249,26 +195,10 @@ def test_replay_of_resigned_games(cap):
     assert set(by_game) <= set(finished)
     assert len(h) == cnt['replay_rows']
     assert cnt['games'] == len(finished)
-    df = rows_to_dataframe(rows, 5)
-    assert len(df) == len(h)
-    buf = DeviceReplayBuffer(len(h) + 7, 5)
-    buf.put(torch.from_numpy(rows).cuda())
-    batch = buf.sample(64, generator=torch.Generator(device='cuda').manual_seed(4))
-    idx = torch.randint(0, len(buf), (64,), device='cuda',
-                        generator=torch.Generator(device='cuda').manual_seed(4)).cpu().numpy()
-    assert np.array_equal(batch['reward'].cpu().numpy(), h['reward'][idx])
-    assert np.allclose(batch['moves_prob'].sum(1).cpu().numpy(), 1.0, atol=1e-5)
+    check_replay_buffer(rows)
 
-    import azalea_b200 as az
-    from azalea_b200.parallel_player import Player
-    pol = az.Policy()
-    pol.net = az.StubEvaluator(stubs.ROUGH)
-    pol.simulations, pol.search_batch_size, pol.exploration_coef = 30, 4, 0.5
-    pol.exploration_depth, pol.exploration_temperature = 4, 1.0
-    pol.exploration_noise_alpha, pol.exploration_noise_scale = 0.03, 0.25
-    agent = az.AzaleaAgent(lambda: az.HexGame(5), policy=pol)
-    player = Player(None, [agent], num_games=64, seed=3, cuda_graph=False,
-                    resign_threshold=STUB_THRESHOLD, resign_disable_prob=0.2, **capkw)
+    player = selfplay_player(StubEvaluator(stubs.ROUGH), 30, 4, cuda_graph=False,
+                             resign_threshold=STUB_THRESHOLD, resign_disable_prob=0.2, **capkw)
     assert player.resign
     for read in (player.read, player.read_device):
         rs0 = player.sp.resign_stats()
@@ -284,14 +214,14 @@ def test_resign_edge_settings():
     """disable_prob = 1 resigns nothing: the games are those of the setting
     off, and every game that ended is a calibration game with its winner's
     lowest r in the histogram.  disable_prob = 0 has no calibration game."""
-    _, _, c_off = stub_selfplay(50)
-    sp, finished, c_all = stub_selfplay(50, resign_threshold=STUB_THRESHOLD, resign_disable_prob=1.0)
+    c_off = stub_selfplay(50)[3]
+    sp, _, finished, c_all = stub_selfplay(50, resign_threshold=STUB_THRESHOLD, resign_disable_prob=1.0)
     assert np.array_equal(c_off, c_all)
     rs = sp.resign_stats()
     assert rs['resigned_games'] == 0 and not any(f[2] for f in finished.values())
     assert rs['calibration_games'] == sp.counters()['games'] == rs['histogram'].sum() > 0
     assert rs['false_positives'] <= rs['calibration_games']
-    sp, finished, _ = stub_selfplay(50, resign_threshold=STUB_THRESHOLD, resign_disable_prob=0.0)
+    sp, _, finished, _ = stub_selfplay(50, resign_threshold=STUB_THRESHOLD, resign_disable_prob=0.0)
     rs = sp.resign_stats()
     assert rs['calibration_games'] == rs['false_positives'] == rs['histogram'].sum() == 0
     assert rs['resigned_games'] == sum(f[2] for f in finished.values()) > 0
@@ -301,36 +231,19 @@ def test_resign_edge_settings():
 def test_resign_invariance():
     """Streams 1 and 2, eager and graphed, and 2 ranks x 32 games against
     1 rank x 64 leave the games and the resignation state unchanged."""
-    from azalea_b200.engine import decode_replay_rows
     kw = dict(resign_threshold=STUB_THRESHOLD, resign_disable_prob=0.3, full_search_prob=0.5,
               fast_simulations=5)
 
     def play(streams, graph, **more):
-        sp, finished, chosen = stub_selfplay(40, streams=streams, graph=graph, **kw, **more)
-        return sp, chosen, sp.harvest(), sp.counters(), sp.eng.resign.cpu().numpy()
-    sp0, c0, r0, n0, s0 = play(1, False)
-    assert len(r0) > 0 and sp0.resign_stats()['resigned_games'] > 0
-    for streams, graph in ((2, False), (2, True), (1, True)):
-        _, c1, r1, n1, s1 = play(streams, graph)
-        assert np.array_equal(c0, c1) and r0.tobytes() == r1.tobytes() and n0 == n1
-        assert np.array_equal(s0, s1)
+        sp, _, _, chosen = stub_selfplay(40, streams=streams, graph=graph, **kw, **more)
+        return (chosen, sp.harvest(), sp.counters(), sp.eng.resign.cpu().numpy(),
+                sp.resign_stats()['resigned_games'])
+    _, r0, _, s0, resigned = assert_streams_and_graphs_agree(play)
+    assert len(r0) > 0 and resigned > 0
     parts = [play(1, False, G=32, rank=r, world_size=2) for r in range(2)]
     # slot s of the 64-game run plays the games of rank s // 32's slot s % 32
-    assert np.array_equal(np.concatenate([p[4] for p in parts]), s0)
-    hw = decode_replay_rows(r0, 5)[0]
-    by_id = {}
-    for i, gid in enumerate(hw['game_id']):
-        by_id.setdefault(int(gid), []).append(i)
-    seen = 0
-    for part in parts:
-        hp = decode_replay_rows(part[2], 5)[0]
-        games = {}
-        for i, gid in enumerate(hp['game_id']):
-            games.setdefault(int(gid), []).append(i)
-        for gid, idx in games.items():
-            assert r0[by_id[gid]].tobytes() == part[2][idx].tobytes()
-            seen += 1
-    assert seen == len(by_id) > 0
+    assert np.array_equal(np.concatenate([p[3] for p in parts]), s0)
+    assert_same_games(r0, [p[1] for p in parts])
 
 
 @gpu
@@ -339,11 +252,8 @@ def test_resign_with_the_network():
     a measure-only run picks a threshold with resign_threshold_for, and a run
     with it resigns games and keeps every engine status at 0."""
     from azalea_b200 import LockstepSelfPlay
-    from azalea_b200.network import HexNetwork
     from azalea_b200.selfplay import resign_threshold_for
-    torch.manual_seed(0)
-    net = HexNetwork(5, 6, 64).eval().cuda()
-    net.prepare_inference(torch.bfloat16)
+    net = network(6)
 
     def play(threshold, disable):
         sp = LockstepSelfPlay(net, num_games=128, board_size=5, simulations=40, search_batch_size=8,
@@ -379,14 +289,7 @@ def test_train_with_resign(tmp_path, monkeypatch):
             super().__init__(*a, **kw)
             made.append(self)
     monkeypatch.setattr(policy_trainer, 'Player', Recording)
-    config = dict(seed=3, device='cuda', game='hex', network='HexNetwork', board_size=5,
-                  num_blocks=1, base_chans=64, simulations=10, search_batch_size=5,
-                  exploration_coef=0.5, exploration_temperature=1.0, exploration_depth=15,
-                  exploration_noise_alpha=0.03, exploration_noise_scale=0.25,
-                  replaybuf_size=256, replaybuf_oversampling=1, batch_size=128, lr_initial=0.01,
-                  lr_decay_steps=100, lr_decay=0.5, momentum=0.9, l2_regularization=1e-4,
-                  total_steps=4, log_interval=0, model_checkpoint_interval=0,
-                  num_selfplay_games=32, resign_threshold=-0.2, resign_disable_prob=0.3)
+    config = train_config(resign_threshold=-0.2, resign_disable_prob=0.3)
     policy = az.Policy()
     policy.initialize(config)
     buf = policy_trainer.initialize_replay_buffer(None, lambda: az.HexGame(5), 256, num_games=32,

@@ -14,14 +14,11 @@ import torch
 
 import oracle
 from oracle import forced, stubs
+from oracle.lockstep import assert_root_matches, bits
 from oracle.philox import full_ply, game_ids
 
 gpu = pytest.mark.gpu
 M_SIM = 8
-
-
-def bits(a):
-    return np.ascontiguousarray(a, dtype=np.float32).tobytes()
 
 
 # n, G, sims, batch, c, eps, alpha, plies (None: to the end), extra settings
@@ -142,7 +139,8 @@ def test_noised_search_matches_the_oracle(name):
                     _repack(eng, g0, cnt)
                 eng.expand_backup()
         eng.set_window(0, 0)
-        v, w, p, kk, rnw, nodes = (x.cpu().numpy() for x in eng.root_stats())
+        stats = [x.cpu().numpy() for x in eng.root_stats()]
+        v, w, p, kk, _, _ = stats
         eng.play_commit(0.0, 0, False, False, False, chosen)
         ch = chosen.cpu().numpy()
         if it == 0:
@@ -159,16 +157,14 @@ def test_noised_search_matches_the_oracle(name):
         for g in live:
             assert int(kk[g]) == k, (g, int(kk[g]), k)
             g_sims = sims if full[g] else cap[1]
-            got = (bits(v[g, :k]), bits(w[g, :k]), bits(p[g, :k]), (float(rnw[g, 0]), float(rnw[g, 1])),
-                   int(nodes[g]))
-            want = _oracle_search(trees[g], games[g], g_sims, batch, coef, mode, fk if full[g] else 0.0,
-                                  eps if full[g] else 0.0, noise.get(g))
-            assert got == want, (name, g, int(ply[g]), full[g])
+            forced.sample_paths_stub_noise(trees[g], games[g], g_sims, batch, coef, mode, fk if full[g] else 0.0,
+                                           eps if full[g] else 0.0, noise.get(g))
+            ov = assert_root_matches(stats, g, trees[g], (name, g, int(ply[g]), full[g]))
             ref = _oracle_search(plain[g], games[g], g_sims, batch, coef, mode, fk if full[g] else 0.0, 0.0, None)
             compared += 1
             if full[g]:
                 noised += 1
-                differ += ref[0] != got[0]
+                differ += ref[0] != bits(ov)
             else:
                 fast += 1           # (compared above with an oracle search without noise)
             mid = int(ch[g, 1])
